@@ -16,6 +16,8 @@ end-of-frame combine; per-GPU work is fixed as N grows ("weak").
           and `cornell_box` / `cornell_smoke` (scenes 7 and 8, 600x600, --cornell-spp in total)
   --impl reference : the reference's own CPU implementation of the path (the C++ f64 oracle — the
           Rust reference cannot be built here), all host threads, on a bounded sample of the frame
+  --dump-outputs DIR : (GPU arm) what the last timed step computed, as .npy files: the same arguments give the same
+          samples on every run, so two builds can be compared output for output
 """
 import argparse
 import ctypes as C
@@ -57,6 +59,10 @@ def parse():
     ap.add_argument("--big-scene", type=int, default=2_000_000, help="spheres of the out-of-cache closest-hit leg at N=1 (0: skip)")
     ap.add_argument("--final-spp", type=int, default=10000, help="total spp of the final_10k frame (the reference default)")
     ap.add_argument("--cornell-spp", type=int, default=8000, help="total spp of the Cornell frames (reference default 200: too short to time)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed on rank 0 to DIR/<name>.npy (float32): `accum`, the (H, W, 4) "
+                         "fp32 accumulator after the combine, and `frame`, the (H, W, 4) RGBA8 frame; past 64 MB in all, the same "
+                         "seeded sample of pixels from both, with their flat indices in `pixel_index`")
     return ap.parse_args()
 
 
@@ -366,6 +372,10 @@ class Frame:
         class _Arr:
             __cuda_array_interface__ = {"shape": (h, w, 4), "typestr": "|u1", "data": (self.rgba_p.value, False), "version": 2}
         self.d_rgba = torch.as_tensor(_Arr(), device=dev)
+
+        class _Acc:
+            __cuda_array_interface__ = {"shape": (h, w, 4), "typestr": "<f4", "data": (self.accum.value, False), "version": 2}
+        self.d_accum = torch.as_tensor(_Acc(), device=dev)
         self.rgba_host = torch.empty((h, w, 4), dtype=torch.uint8).pin_memory()
         self.combine = "local" if world == 1 else combine
         self.all_acc = self.root_rgba = self.peers = self.comm = None
@@ -534,6 +544,8 @@ def run_ours(args):
     launches = ctx.kernel_launches() - launches0
     prof = ctx.profile_read(reset=True)
     ctx.set_profiling(False)
+    # the last timed step's outputs, before the legs below reuse the frame's buffers
+    outputs = {"accum": frame.d_accum.cpu().numpy(), "frame": frame.d_rgba.cpu().numpy()} if args.dump_outputs and rank == 0 else None
     kern_ms = [a.elapsed_time(b) for a, b in kev]
     rays_rank = int(ray_counter.item())
     samples_total = n_px * args.spp * world * args.steps
@@ -694,11 +706,33 @@ def run_ours(args):
                 line["big_scene"] = {"unavailable": str(e)}
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline(args)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
     if rank == 0:
         emit(line)
+
+
+DUMP_LIMIT = 64 * 10 ** 6  # bytes of .npy data in all
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each (H, W, C) array as out_dir/<name>.npy in float32. Past DUMP_LIMIT bytes in all, every array keeps the
+    same fixed, seeded sample of pixels, whose flat indices go to pixel_index.npy (float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    h, w = next(iter(arrays.values())).shape[:2]
+    per_px = sum(4 * a.shape[2] for a in arrays.values())
+    if h * w * per_px > DUMP_LIMIT:
+        k = (DUMP_LIMIT - 4096) // (per_px + 8)  # (room for the index and the .npy headers)
+        idx = np.sort(np.random.default_rng(0).choice(h * w, k, replace=False))
+        np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
+        arrays = {name: a.reshape(h * w, -1)[idx] for name, a in arrays.items()}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float32))
+    sys.stderr.write(f"outputs of the last timed step: {', '.join(sorted(arrays))} -> {out_dir}\n")
 
 
 _REAL_STDOUT = None

@@ -276,6 +276,32 @@ def test_bench_arms_print_the_same_config():
         assert bench.scene_defaults(number) == R.scene_defaults(number)  # bench.py's copy of the scene table
 
 
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: float32 copies of the arrays, whole while they fit the size limit; past it, one seeded
+    sample of pixels, the same on every run and in every array, with its indices."""
+    import bench
+    rng = np.random.default_rng(3)
+    accum = rng.random((50, 40, 4), dtype=np.float32)
+    frame = rng.integers(0, 256, (50, 40, 4), dtype=np.uint8)
+    bench.dump_outputs(str(tmp_path / "whole"), {"accum": accum, "frame": frame})
+    assert sorted(os.listdir(tmp_path / "whole")) == ["accum.npy", "frame.npy"]
+    assert np.array_equal(np.load(tmp_path / "whole" / "accum.npy"), accum)
+    got = np.load(tmp_path / "whole" / "frame.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, frame)
+    h, w = 2000, 1500  # 2 x 48 MB as float32: over the limit
+    accum = rng.random((h, w, 4), dtype=np.float32)
+    frame = rng.integers(0, 256, (h, w, 4), dtype=np.uint8)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"accum": accum, "frame": frame})
+        assert sum(os.path.getsize(tmp_path / run / f) for f in os.listdir(tmp_path / run)) <= bench.DUMP_LIMIT
+    idx = np.load(tmp_path / "a" / "pixel_index.npy")
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "pixel_index.npy"))
+    idx = idx.astype(np.int64)
+    assert idx.shape[0] > 0.9 * bench.DUMP_LIMIT / (2 * 16 + 8) and (np.diff(idx) > 0).all() and idx[-1] < h * w
+    assert np.array_equal(np.load(tmp_path / "a" / "accum.npy"), accum.reshape(-1, 4)[idx])
+    assert np.array_equal(np.load(tmp_path / "a" / "frame.npy"), frame.reshape(-1, 4)[idx])
+
+
 # ---------------------------------------------------------------------------
 # struct layouts: C header (gcc offsetof) == ctypes (abi.py) == Rust #[repr(C)] (ffi.rs), field by field
 # ---------------------------------------------------------------------------
