@@ -245,8 +245,9 @@ void* rtx_ctx_stream(rtx_ctx* ctx);
 /* Which builder makes the BVH over the world in rtx_scene_create (replaces BvhTree::new, hittable.rs:260-321; the
  * tree's topology is not part of the contract, only the closest-hit answers): 0 = host, binned SAH (default, the
  * better trees), 1 = device, Morton-code LBVH, 2 = device, PLOC (locally-ordered agglomerative clustering along the Morton
- * curve: merges decided by box surface areas) — the device builders are for scenes large enough that the host build is
- * the bottleneck. */
+ * curve: merges decided by box surface areas), 3 = device, top-down binned SAH (the host builder's policy: trees of
+ * host quality) — the device builders are for scenes large enough that the host build is the bottleneck. Other kinds
+ * are refused. */
 int rtx_ctx_set_bvh_builder(rtx_ctx* ctx, int kind);
 /* number of CUDA kernels this context has launched so far (bookkeeping for benchmarks) */
 int rtx_ctx_kernel_launches(rtx_ctx* ctx, unsigned long long* out);

@@ -20,6 +20,7 @@
 #include "flatten.hpp"
 #include "kernels.cuh"
 #include "lbvh.cuh"
+#include "sah_build.cuh"
 #include "shade2.cuh"
 #include "trace2.cuh"
 #include "trace3.cuh"
@@ -112,7 +113,8 @@ struct rtx_ctx {
     cudaEvent_t fork_event = nullptr;
     unsigned long long wf_iterations = 0;  // (shade, trace) iterations launched on partition 0
     unsigned long long launches = 0;  // kernels launched by this context (rtx_ctx_kernel_launches)
-    int bvh_builder = 0;              // 0: host binned SAH (default), 1: device LBVH, 2: device PLOC (rtx_ctx_set_bvh_builder, RTX_BVH=lbvh|ploc)
+    int bvh_builder = 0;              // 0: host binned SAH (default), 1: device LBVH, 2: device PLOC, 3: device binned SAH
+                                      // (rtx_ctx_set_bvh_builder, RTX_BVH=lbvh|ploc|sah_device)
     int ploc_radius = 16;             // neighbours searched on each side by the PLOC builder (RTX_PLOC_RADIUS, 1..32)
     int last_build_passes = 0;        // passes the last PLOC build took (RTX_DEBUG_BUILD=1 prints it)
     uint8_t* h_stage = nullptr;       // pinned staging buffer of rtx_scene_create (every H2D copy leaves from here)
@@ -252,7 +254,8 @@ int rtx_ctx_create(int device, void* stream, rtx_ctx** out) {
     { int g = 8; while (g * 2 <= c->order_groups && g < (1 << 15)) g *= 2; c->order_groups = g; }
     cudaDeviceGetAttribute(&c->smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
     if (const char* m = std::getenv("RTX_MODE")) c->mode = std::strcmp(m, "mega") == 0 ? 0 : 1;
-    if (const char* m = std::getenv("RTX_BVH")) c->bvh_builder = std::strcmp(m, "lbvh") == 0 ? 1 : (std::strcmp(m, "ploc") == 0 ? 2 : 0);
+    if (const char* m = std::getenv("RTX_BVH"))
+        c->bvh_builder = std::strcmp(m, "lbvh") == 0 ? 1 : (std::strcmp(m, "ploc") == 0 ? 2 : (std::strcmp(m, "sah_device") == 0 ? 3 : 0));
     c->ploc_radius = env_int("RTX_PLOC_RADIUS", c->ploc_radius);
     // the traversal stack lives in local memory: prefer L1 over shared for it
     cudaFuncSetCacheConfig(rtx::render_kernel<false>, cudaFuncCachePreferL1);
@@ -362,7 +365,7 @@ int rtx_ctx_measure_l2_read(rtx_ctx* c, unsigned long long bytes, int repeats, d
     return RTX_OK;
 }
 int rtx_ctx_set_bvh_builder(rtx_ctx* c, int kind) {
-    if (!c || kind < 0 || kind > 2) return fail(RTX_ERR_INVALID, "bad argument");
+    if (!c || kind < 0 || kind > 3) return fail(RTX_ERR_INVALID, "bad argument");
     c->bvh_builder = kind;
     return RTX_OK;
 }
@@ -381,9 +384,11 @@ int rtx_scene_create(rtx_ctx* c, const rtx_scene_desc* desc, rtx_scene** out) {
     rtx::FlatScene fs;
     std::string err;
     if (!rtx::flatten_scene(*desc, fs, err, c->bvh_builder >= 1, c->wf_wide != 0)) return fail(RTX_ERR_INVALID, "scene description: " + err);
-    // nodes the device builder will add behind the host-built ones (medium boundaries), and its box upload
+    // nodes the device builder may add behind the host-built ones (medium boundaries), and its box upload: a binary
+    // tree over n items has at most n - 1 inner nodes (the binned-SAH builder's leaves of several items make fewer)
     const size_t host_nodes = fs.nodes.size();
     const size_t lbvh_nodes = fs.world_deferred ? (size_t)fs.world_count - 1 : 0;
+    size_t built_nodes = lbvh_nodes;
     rtx_scene* s = new (std::nothrow) rtx_scene();
     if (!s) return fail(RTX_ERR_NOMEM, "out of host memory");
     s->device = c->device;
@@ -523,7 +528,18 @@ int rtx_scene_create(rtx_ctx* c, const rtx_scene_desc* desc, rtx_scene** out) {
             }
         for (int a = 0; a < 3; ++a) ext[a] -= lo[a];
         int depth = 0;
-        if (c->bvh_builder == 2) {
+        if (c->bvh_builder == 3) {
+            rtx::SahBuildStats st;
+            e = rtx::sah_build(c->stream, fs.world_count, (const float*)(base + off_boxes), fs.world_first_record,
+                               (rtx::Record*)(base + off_records) + fs.world_first_record, (int32_t)host_nodes,
+                               (rtx::BvhNode*)(base + off_nodes) + host_nodes, rtx::BvhPolicy::from_env(), rtx::kTraversalStack - 2, &st);
+            if (e != cudaSuccess) return bail(cuda_fail(e, "sah_build"));
+            c->launches += st.launches;
+            depth = st.depth;
+            built_nodes = (size_t)st.nodes;
+            if (std::getenv("RTX_DEBUG_BUILD"))
+                std::fprintf(stderr, "[rtx] SAH (device): %d primitives, %d levels, depth %d, %d nodes\n", fs.world_count, st.levels, depth, st.nodes);
+        } else if (c->bvh_builder == 2) {
             int passes = 0;
             e = rtx::ploc_build(c->stream, fs.world_count, (const float*)(base + off_boxes), lo, ext, fs.world_first_record, (int32_t)host_nodes,
                                 (rtx::BvhNode*)(base + off_nodes) + host_nodes, &depth, c->ploc_radius, &passes);
@@ -541,7 +557,7 @@ int rtx_scene_create(rtx_ctx* c, const rtx_scene_desc* desc, rtx_scene** out) {
             return bail(fail(RTX_ERR_UNSUPPORTED, "device-built BVH deeper than the traversal stack: use the host builder"));
         fs.world_root = (int32_t)host_nodes;
         fs.world_first_node = (int32_t)host_nodes;
-        fs.world_node_count = (int32_t)lbvh_nodes;
+        fs.world_node_count = (int32_t)built_nodes;
         fs.world_depth = depth;
     }
     s->view.nodes = (const rtx::BvhNode*)(base + off_nodes);
@@ -557,7 +573,7 @@ int rtx_scene_create(rtx_ctx* c, const rtx_scene_desc* desc, rtx_scene** out) {
     s->view.wide_root = fs.world_deferred ? -1 : fs.wide_root;
     s->view.n_media = fs.n_media;
     s->camera = fs.camera;
-    s->n_nodes = (int32_t)(host_nodes + lbvh_nodes);
+    s->n_nodes = (int32_t)(host_nodes + built_nodes);
     s->n_records = (int32_t)fs.records.size();
     s->n_xforms = (int32_t)fs.xforms.size();
     s->world_first_node = fs.world_first_node;

@@ -39,6 +39,13 @@ double Aabb::half_area() const {
     return dx * dy + dy * dz + dz * dx;
 }
 
+BvhPolicy BvhPolicy::from_env() {
+    BvhPolicy p;
+    if (const char* v = std::getenv("RTX_BVH_LEAF")) p.max_leaf = std::min(kBvhMaxLeafLimit, std::max(1, std::atoi(v)));
+    if (const char* v = std::getenv("RTX_BVH_CPRIM")) p.cost_prim = std::max(0.1, std::atof(v));
+    return p;
+}
+
 namespace {
 
 struct Item {
@@ -65,12 +72,8 @@ struct BvhBuilder {
     std::vector<BvhNode>& nodes;
     std::vector<Record>& records;
     std::vector<Item>& items;
-    static constexpr int kBins = 16;
-    static constexpr int kMaxLeafLimit = 4;
-    static constexpr double kCostTraverse = 1.0;  // one 64-byte node fetch + two fp32 slab tests
-    // tunables (RTX_BVH_LEAF, RTX_BVH_CPRIM override for experiments)
-    int kMaxLeaf = 4;
-    double kCostPrim = 2.0;  // one 96-byte record + an f64 intersection, in units of kCostTraverse
+    static constexpr int kBins = kBvhBins;
+    const BvhPolicy pol = BvhPolicy::from_env();
 
     struct Tmp {
         Aabb box;
@@ -87,10 +90,7 @@ struct BvhBuilder {
     };
     std::vector<Prim> prims;
 
-    BvhBuilder(std::vector<BvhNode>& n, std::vector<Record>& r, std::vector<Item>& it) : nodes(n), records(r), items(it) {
-        if (const char* v = std::getenv("RTX_BVH_LEAF")) kMaxLeaf = std::min(kMaxLeafLimit, std::max(1, std::atoi(v)));
-        if (const char* v = std::getenv("RTX_BVH_CPRIM")) kCostPrim = std::max(0.1, std::atof(v));
-    }
+    BvhBuilder(std::vector<BvhNode>& n, std::vector<Record>& r, std::vector<Item>& it) : nodes(n), records(r), items(it) {}
 
     int build_range(int lo, int hi) {
         Tmp t;
@@ -162,10 +162,10 @@ struct BvhBuilder {
         if (any_solo) {
             make_leaf = false;  // the traversal switches space on these: one per leaf
         } else if (best_axis < 0) {
-            make_leaf = n <= kMaxLeaf;  // all centroids coincide
-        } else if (n <= kMaxLeaf) {
-            double split_cost = kCostTraverse + (area > 0 ? best_cost / area : 0.0) * kCostPrim;
-            make_leaf = n * kCostPrim <= split_cost;
+            make_leaf = n <= pol.max_leaf;  // all centroids coincide
+        } else if (n <= pol.max_leaf) {
+            double split_cost = pol.cost_traverse + (area > 0 ? best_cost / area : 0.0) * pol.cost_prim;
+            make_leaf = n * pol.cost_prim <= split_cost;
         }
         if (make_leaf) return self;
 
@@ -851,7 +851,7 @@ struct Checker {
             } else {
                 int32_t v = ~ref;
                 int first = v >> 4, count = v & 15;
-                if (count > BvhBuilder::kMaxLeafLimit && count != 0) return fail("leaf larger than the maximum");
+                if (count > kBvhMaxLeafLimit && count != 0) return fail("leaf larger than the maximum");
                 if (first < 0 || first + count > (int)fs.records.size()) return fail("leaf range out of bounds");
                 for (int i = 0; i < count; ++i) {
                     const Record& r = fs.records[(size_t)(first + i)];

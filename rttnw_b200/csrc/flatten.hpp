@@ -46,6 +46,16 @@ struct FlatScene {
     CameraView camera;
 };
 
+// The binned-SAH policy, one definition for the host builder (flatten.cpp) and the device builder (sah_build.cuh).
+constexpr int kBvhBins = 16;         // bins per axis (a node of n < 16 primitives gets max(2, n))
+constexpr int kBvhMaxLeafLimit = 4;  // largest leaf either builder makes
+struct BvhPolicy {
+    int max_leaf = 4;            // RTX_BVH_LEAF (1 .. kBvhMaxLeafLimit) overrides, for experiments
+    double cost_traverse = 1.0;  // one 64-byte node fetch + two fp32 slab tests
+    double cost_prim = 2.0;      // one 96-byte record + an f64 intersection, in units of cost_traverse; RTX_BVH_CPRIM overrides
+    static BvhPolicy from_env();
+};
+
 // Returns false and fills `err` on malformed input.
 // defer_world_bvh: leave the BVH over the world to the device builder when the world has at least two items.
 // wide_copy: append the 4-wide copy of the (host-built) world BVH to the node array and set wide_root.

@@ -97,8 +97,10 @@ class Context:
         abi.check(self.lib.rtx_ctx_sync(self.h))
 
     def set_bvh_builder(self, kind: str) -> None:
-        """'sah' (host, default), 'lbvh' or 'ploc' (device) for the scenes created from now on."""
-        abi.check(self.lib.rtx_ctx_set_bvh_builder(self.h, {"sah": 0, "lbvh": 1, "ploc": 2}[kind]))
+        """Which builder makes the world BVH of the scenes created from now on: 'sah' (host binned SAH, the
+        default), 'lbvh' or 'ploc' (device, faster builds of slower trees), or 'sah_device' (device binned SAH:
+        the host builder's policy, trees of host quality)."""
+        abi.check(self.lib.rtx_ctx_set_bvh_builder(self.h, {"sah": 0, "lbvh": 1, "ploc": 2, "sah_device": 3}[kind]))
 
     def set_profiling(self, on: bool) -> None:
         abi.check(self.lib.rtx_ctx_set_profiling(self.h, 1 if on else 0))

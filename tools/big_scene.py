@@ -1,4 +1,4 @@
-"""Scratch: build time (host SAH vs device LBVH vs device PLOC) and trace throughput on a large random scene."""
+"""Scratch: build time (host SAH vs device LBVH, PLOC and binned SAH) and trace throughput on a large random scene."""
 import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -22,7 +22,8 @@ rays["t_min"], rays["t_max"], rays["xi"] = 0.001, np.finfo(np.float64).max, 0.5
 d_rays = torch.from_numpy(rays.view(np.uint8).reshape(-1)).cuda()
 d_hits = torch.empty(m * 88, dtype=torch.uint8, device="cuda")
 res = {}
-kinds = ("sah", "lbvh", "ploc", "sah", "lbvh", "ploc") if n <= 500_000 else ("lbvh", "ploc", "lbvh", "ploc")
+device = ("lbvh", "ploc", "sah_device")
+kinds = ((("sah",) if n <= 1_000_000 else ()) + device) * 2
 for kind in kinds:
     ctx.set_bvh_builder(kind)
     torch.cuda.synchronize(); t0 = time.perf_counter()
@@ -35,7 +36,7 @@ for kind in kinds:
     h = d_hits.cpu().numpy().view(abi.HIT_DTYPE)
     res[kind] = h.copy()
     st = sc.trace_stats(d_rays, m)
-    print(f"{kind:5s}: scene create {1e3 * (t1 - t0):8.1f} ms ({sc.info()['bvh_nodes']} nodes), trace {m} rays {ms:.2f} ms = {m / ms / 1e6:.2f} Grays/s, hits {np.mean(h['prim_id'] >= 0):.3f}, "
+    print(f"{kind:10s}: scene create {1e3 * (t1 - t0):8.1f} ms ({sc.info()['bvh_nodes']} nodes), trace {m} rays {ms:.2f} ms = {m / ms / 1e6:.2f} Grays/s, hits {np.mean(h['prim_id'] >= 0):.3f}, "
           f"{st['node_visits']:.1f} node visits and {st['sphere_tests']:.2f} sphere tests per ray", flush=True)
     sc.close()
 for k in res:
