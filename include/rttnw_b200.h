@@ -314,6 +314,40 @@ int rtx_render_counted(rtx_ctx* ctx, const rtx_scene* scene, const rtx_render_pa
  * synchronous) or device (asynchronous). */
 int rtx_tonemap_rgba8(rtx_ctx* ctx, const float* d_accum, int32_t width, int32_t height,
                       uint8_t* out, int out_on_device);
+/* Adaptive sampling. The reference gives every pixel the same number of samples (the fixed per-pixel fold of
+ * src/main.rs:211); here each 8x4 tile of pixels stops once its noise estimate is below a threshold. Every pixel ends
+ * with the samples [spp_begin, spp_begin + n) of the uniform render (a prefix of its sample sequence), n shared by the
+ * pixels of a tile: round 0 renders min_spp samples for every tile, each later round min(step_spp, max_spp - n) more
+ * for the tiles still sampling. d_aux (width*height float4, like d_accum) receives only the samples with an odd
+ * global index, so aux.w == n / 2. The pixel error compares the two halves' means I = accum.rgb / accum.w and
+ * A = aux.rgb / aux.w, with the sqrt gamma of main.rs:217-225 in the denominator:
+ *     e = (|I_r - A_r| + |I_g - A_g| + |I_b - A_b|) / (1e-4 + sqrt(I_r + I_g + I_b)),
+ * a tile's error is the largest e of its pixels inside the frame (a pixel with no samples in either buffer counts 0),
+ * and after each round a tile whose error is below the threshold stops for good, as does every tile at max_spp. */
+typedef struct rtx_adaptive_params {
+    double threshold; /* >= 0, finite; 0 = every pixel gets max_spp (params->spp_count) */
+    int32_t min_spp;  /* even, >= 2, <= max_spp */
+    int32_t step_spp; /* even, >= 2 */
+} rtx_adaptive_params; /* 16 bytes */
+
+typedef struct rtx_adaptive_stats {
+    int64_t path_samples;    /* sum of n over the pixels of the frame */
+    int32_t rounds;          /* render rounds */
+    int32_t tiles;           /* 8x4 tiles of the frame */
+    int32_t tiles_converged; /* stopped below the threshold before max_spp */
+    int32_t tiles_at_max;    /* stopped at max_spp (tiles_converged + tiles_at_max == tiles) */
+} rtx_adaptive_stats; /* 24 bytes */
+
+/* params->spp_count is max_spp (even, <= 2^24); params->spp_begin is even. Zeroes d_accum and d_aux, then renders.
+ * Synchronous: joins any queued asynchronous job first (like rtx_render_counted). stats may be NULL. Needs the
+ * default wavefront driver: RTX_MODE=mega, RTX_SHADE=1 and RTX_ORDER=1 give RTX_ERR_UNSUPPORTED. */
+int rtx_render_adaptive(rtx_ctx* ctx, const rtx_scene* scene, const rtx_render_params* params,
+                        const rtx_adaptive_params* adaptive, float* d_accum, float* d_aux,
+                        rtx_adaptive_stats* stats);
+/* Per-tile error of any (accum, aux) pair: tiles_y x tiles_x floats, row 0 = top tiles. Asynchronous.
+ * This is the same error rtx_render_adaptive decides on, so a user can show a noise map. */
+int rtx_adaptive_error(rtx_ctx* ctx, const float* d_accum, const float* d_aux, int32_t width, int32_t height,
+                       float* d_tile_error);
 /* Rank-0 side of the multi-GPU combine: sums n_peers device accumulators
  * (peer-mapped pointers, read over NVLink) into d_accum and tonemaps in the
  * same kernel. d_rgba8 is a device buffer. Asynchronous. DESTRUCTIVE: d_accum

@@ -91,8 +91,18 @@ class SceneDefaults(C.Structure):
                 ("max_depth", C.c_int32), ("name", C.c_char_p)]
 
 
+class AdaptiveParams(C.Structure):
+    _fields_ = [("threshold", C.c_double), ("min_spp", C.c_int32), ("step_spp", C.c_int32)]
+
+
+class AdaptiveStats(C.Structure):
+    _fields_ = [("path_samples", C.c_int64), ("rounds", C.c_int32), ("tiles", C.c_int32),
+                ("tiles_converged", C.c_int32), ("tiles_at_max", C.c_int32)]
+
+
 assert C.sizeof(Node) == 96 and C.sizeof(Material) == 40 and C.sizeof(Texture) == 48
 assert C.sizeof(Ray) == 80 and C.sizeof(Hit) == 88 and C.sizeof(RenderParams) == 32
+assert C.sizeof(AdaptiveParams) == 16 and C.sizeof(AdaptiveStats) == 24
 
 # numpy views of the two bulk records (same memory layout as the C structs)
 RAY_DTYPE = [("origin", "<f8", 3), ("direction", "<f8", 3), ("time", "<f8"), ("t_min", "<f8"),
@@ -126,6 +136,9 @@ SIGNATURES = {
     "rtx_trace_rays_stats": (C.c_int, [_P, _P, C.c_int64, _P, C.POINTER(TraceStats)]),
     "rtx_render": (C.c_int, [_P, _P, C.POINTER(RenderParams), _P, _P]),
     "rtx_render_counted": (C.c_int, [_P, _P, C.POINTER(RenderParams), _P, C.POINTER(TraceStats)]),
+    "rtx_render_adaptive": (C.c_int, [_P, _P, C.POINTER(RenderParams), C.POINTER(AdaptiveParams), _P, _P,
+                                      C.POINTER(AdaptiveStats)]),
+    "rtx_adaptive_error": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, _P]),
     "rtx_tonemap_rgba8": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P, C.c_int]),
     "rtx_reduce_tonemap_peers": (C.c_int, [_P, _P, C.POINTER(_P), C.c_int32, C.c_int32, C.c_int32, _P]),
     "rtx_reduce_tonemap_slice": (C.c_int, [_P, C.POINTER(_P), C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P]),

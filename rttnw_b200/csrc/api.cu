@@ -3,11 +3,13 @@
 #include <cuda_runtime.h>
 #include <dlfcn.h>
 
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <algorithm>
+#include <chrono>
 #include <condition_variable>
 #include <deque>
 #include <functional>
@@ -18,6 +20,7 @@
 
 #include "../../include/rttnw_b200.h"
 #include "flatten.hpp"
+#include "adaptive.cuh"
 #include "kernels.cuh"
 #include "lbvh.cuh"
 #include "sah_build.cuh"
@@ -741,9 +744,13 @@ static int wf_prepare(rtx_ctx* c, int64_t slots) {
 // submitting once a batch ended with no ray in flight and no sample left (the batch queued behind it
 // then runs over empty slots). The call returns when everything has been submitted AND that check
 // has come back, i.e. it may block the calling thread for most of the render.
+// With tile_list (adaptive sampling), only the n_list tiles of that list of dispenser order indices are rendered, and
+// the samples with an odd global index also go to d_aux.
 static int render_wavefront(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, float* d_accum,
-                            unsigned long long* d_ray_count, bool counted) {
-    const int64_t n_tiles = (int64_t)((p->width + rtx::kTileW - 1) / rtx::kTileW) * ((p->height + rtx::kTileH - 1) / rtx::kTileH);
+                            unsigned long long* d_ray_count, bool counted, const uint32_t* tile_list = nullptr,
+                            int64_t n_list = 0, float* d_aux = nullptr) {
+    const bool adaptive = tile_list != nullptr;
+    const int64_t n_tiles = adaptive ? n_list : (int64_t)((p->width + rtx::kTileW - 1) / rtx::kTileW) * ((p->height + rtx::kTileH - 1) / rtx::kTileH);
     const unsigned long long total = (unsigned long long)n_tiles * 32ull * (unsigned long long)p->spp_count;
     // pool size: the configured maximum, but a small job (few pool refills) is all ramp-up and drain with a pool
     // that large: keep at least ~24 refills, down to 256 Ki slots
@@ -767,6 +774,8 @@ static int render_wavefront(rtx_ctx* c, const rtx_scene* s, const rtx_render_par
     a.n_slots = (int32_t)slots;
     a.total_items = total;
     a.next_item = c->d_next_item;
+    a.adaptive.tile_list = tile_list;  // (ray ordering, the other user of this space, fills it per partition below)
+    a.adaptive.aux = reinterpret_cast<float4*>(d_aux);
     {   // carve the SoA arrays out of the pool allocation (8-byte arrays first)
         uint8_t* base = (uint8_t*)c->d_pool;
         size_t n = (size_t)slots;
@@ -960,7 +969,10 @@ static int render_wavefront(rtx_ctx* c, const rtx_scene* s, const rtx_render_par
                 }
                 prof_now = q == 0 && c->profiling && (iteration++ % kProfStride) == 0;
                 CU(prof_mark());
-                if (c->shade_form >= 2) {
+                if (adaptive) {  // (rtx_render_adaptive refuses the first shade form and ray ordering)
+                    if (c->perlin_smem && s->n_perlins == 1) rtx::wf_shade2_kernel<false, true, false, true><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, nullptr);
+                    else rtx::wf_shade2_kernel<false, false, false, true><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, nullptr);
+                } else if (c->shade_form >= 2) {
                     if (counted && !ordered) rtx::wf_shade2_kernel<true><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, c->d_counters);
                     else if (ordered) {
                         if (counted) rtx::wf_shade2_kernel<true, false, true><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, c->d_counters);
@@ -1134,6 +1146,134 @@ int rtx_render_counted(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* 
     out->rect_tests = (double)h.rect_tests / dn;
     out->instance_enters = (double)h.instance_enters / dn;
     out->medium_tests = (double)h.medium_tests / dn;
+    return RTX_OK;
+}
+
+// ---- adaptive sampling (adaptive.cuh) ----------------------------------------
+int rtx_render_adaptive(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, const rtx_adaptive_params* ap,
+                        float* d_accum, float* d_aux, rtx_adaptive_stats* stats) {
+    if (!c || !s || !p || !ap || !d_accum || !d_aux) return fail(RTX_ERR_INVALID, "NULL argument");
+    if (p->width <= 0 || p->height <= 0 || p->max_depth < 0 || p->spp_begin < 0 || (p->spp_begin & 1))
+        return fail(RTX_ERR_INVALID, "bad render parameters (spp_begin must be even)");
+    if ((int64_t)p->width * p->height > 0x7fffffff) return fail(RTX_ERR_INVALID, "image too large");
+    const int max_spp = p->spp_count;
+    if (max_spp < 2 || (max_spp & 1) || max_spp > (1 << 24)) return fail(RTX_ERR_INVALID, "spp_count (max_spp) must be even, in [2, 2^24]");
+    if (ap->min_spp < 2 || (ap->min_spp & 1) || ap->min_spp > max_spp) return fail(RTX_ERR_INVALID, "min_spp must be even, in [2, max_spp]");
+    if (ap->step_spp < 2 || (ap->step_spp & 1)) return fail(RTX_ERR_INVALID, "step_spp must be even and >= 2");
+    if (!(ap->threshold >= 0.0) || !std::isfinite(ap->threshold)) return fail(RTX_ERR_INVALID, "threshold must be finite and >= 0");
+    if (c->mode != 1 || c->shade_form < 2 || c->order_form != 0)
+        return fail(RTX_ERR_UNSUPPORTED, "adaptive sampling needs the wavefront driver with the default shade form and no ray ordering");
+    JOIN(c);
+    CU(cudaSetDevice(c->device));
+    const int w = p->width, h = p->height;
+    const int tiles_x = (w + rtx::kTileW - 1) / rtx::kTileW, tiles_y = (h + rtx::kTileH - 1) / rtx::kTileH;
+    const int n_tiles = tiles_x * tiles_y;
+    const float inv_per_block_row = 1.0f / (float)(tiles_x * rtx::kBlockH);
+    // scratch: tile errors, flags, their scan, the list, the round's read-back, cub's temporary storage
+    size_t scan_bytes = 0;
+    CU(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, n_tiles, c->stream));
+    const size_t words = ((size_t)n_tiles + 63) / 64 * 64 * 4;
+    const size_t o_round = 4 * words, o_cub = o_round + 256;
+    uint8_t* block = nullptr;
+    CU(cudaMalloc(&block, o_cub + scan_bytes));
+    float* d_err = (float*)block;
+    uint32_t* d_flag = (uint32_t*)(block + words);
+    uint32_t* d_pos = (uint32_t*)(block + 2 * words);
+    uint32_t* d_list = (uint32_t*)(block + 3 * words);
+    rtx::AdaptiveRound* d_round = (rtx::AdaptiveRound*)(block + o_round);
+    float4* acc = reinterpret_cast<float4*>(d_accum);
+    float4* aux = reinterpret_cast<float4*>(d_aux);
+    rtx::AdaptiveRound cur{};
+    rtx_adaptive_stats st{};
+    st.tiles = n_tiles;
+    // the tiles that keep sampling after the errors in `err` (all of them for nullptr): list + read-back
+    auto select_tiles = [&](const float* err) -> int {
+        const unsigned grid = (unsigned)((n_tiles + 255) / 256);
+        CU(cudaMemsetAsync(d_round, 0, sizeof(rtx::AdaptiveRound), c->stream));
+        rtx::adaptive_flag_kernel<<<grid, 256, 0, c->stream>>>(err, ap->threshold, tiles_x, tiles_y, inv_per_block_row, d_flag);
+        size_t cb = scan_bytes;
+        CU(cub::DeviceScan::ExclusiveSum(block + o_cub, cb, d_flag, d_pos, n_tiles, c->stream));
+        rtx::adaptive_scatter_kernel<<<grid, 256, 0, c->stream>>>(d_flag, d_pos, w, h, tiles_x, tiles_y, inv_per_block_row, d_list, d_round);
+        c->launches += 4;  // (cub's scan counts as two)
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(&cur, d_round, sizeof(cur), cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        return RTX_OK;
+    };
+    // RTX_DEBUG_ADAPTIVE=1: one stderr line per round (the render is then synchronised before the decision, to time it)
+    const bool debug = std::getenv("RTX_DEBUG_ADAPTIVE") != nullptr;
+    auto ms_since = [](std::chrono::steady_clock::time_point t) {
+        return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t).count();
+    };
+    auto run = [&]() -> int {
+        CU(cudaMemsetAsync(d_accum, 0, (size_t)w * h * 16, c->stream));
+        CU(cudaMemsetAsync(d_aux, 0, (size_t)w * h * 16, c->stream));
+        int rc = select_tiles(nullptr);
+        if (rc != RTX_OK) return rc;
+        int n = 0, spp = ap->min_spp;
+        for (;;) {
+            const auto t_round = std::chrono::steady_clock::now();
+            double render_ms = 0.0;
+            if (p->max_depth == 0) {  // color(.., depth = 0) is black (main.rs:27-29): only the sample counts move
+                rtx::adaptive_black_kernel<<<(unsigned)((cur.tiles * 32 + 127) / 128), 128, 0, c->stream>>>(
+                    d_list, (int)cur.tiles, w, h, tiles_x, tiles_y, inv_per_block_row, p->spp_begin + n, spp, acc, aux);
+                c->launches += 1;
+                CU(cudaGetLastError());
+            } else {
+                rtx_render_params rp = *p;
+                rp.spp_begin = p->spp_begin + n;
+                rp.spp_count = spp;
+                rc = render_wavefront(c, s, &rp, d_accum, nullptr, false, d_list, (int64_t)cur.tiles, d_aux);
+                if (rc != RTX_OK) return rc;
+            }
+            if (debug) {
+                CU(cudaStreamSynchronize(c->stream));
+                render_ms = ms_since(t_round);
+            }
+            n += spp;
+            ++st.rounds;
+            st.path_samples += (int64_t)cur.pixels * spp;
+            const unsigned long long before = cur.tiles;
+            if (n == max_spp) {
+                st.tiles_at_max = (int32_t)cur.tiles;
+                if (debug) std::fprintf(stderr, "[rtx] adaptive round %d: %llu tiles x %d spp (n = %d), %llu path samples, render %.3f ms\n",
+                                        st.rounds - 1, before, spp, n, cur.pixels * (unsigned long long)spp, render_ms);
+                break;
+            }
+            rtx::adaptive_error_kernel<<<(unsigned)(((int64_t)n_tiles * 32 + rtx::kAdaptiveBlock - 1) / rtx::kAdaptiveBlock),
+                                         rtx::kAdaptiveBlock, 0, c->stream>>>(acc, aux, w, h, tiles_x, n_tiles, d_err);
+            c->launches += 1;
+            CU(cudaGetLastError());
+            const unsigned long long pixels = cur.pixels;
+            rc = select_tiles(d_err);
+            if (rc != RTX_OK) return rc;
+            if (debug) std::fprintf(stderr, "[rtx] adaptive round %d: %llu tiles x %d spp (n = %d), %llu path samples, render %.3f ms, decision %.3f ms\n",
+                                    st.rounds - 1, before, spp, n, pixels * (unsigned long long)spp, render_ms, ms_since(t_round) - render_ms);
+            st.tiles_converged += (int32_t)(before - cur.tiles);
+            if (cur.tiles == 0) break;
+            spp = std::min(ap->step_spp, max_spp - n);
+        }
+        CU(cudaStreamSynchronize(c->stream));
+        return RTX_OK;
+    };
+    const int rc = run();
+    cudaStreamSynchronize(c->stream);  // (nothing may still use the scratch block when it is freed)
+    cudaFree(block);
+    if (rc == RTX_OK && stats) *stats = st;
+    return rc;
+}
+
+int rtx_adaptive_error(rtx_ctx* c, const float* d_accum, const float* d_aux, int32_t width, int32_t height, float* d_tile_error) {
+    if (!c || !d_accum || !d_aux || !d_tile_error || width <= 0 || height <= 0) return fail(RTX_ERR_INVALID, "bad argument");
+    if ((int64_t)width * height > 0x7fffffff) return fail(RTX_ERR_INVALID, "image too large");
+    JOIN(c);
+    CU(cudaSetDevice(c->device));
+    const int tiles_x = (width + rtx::kTileW - 1) / rtx::kTileW, tiles_y = (height + rtx::kTileH - 1) / rtx::kTileH;
+    const int64_t n_tiles = (int64_t)tiles_x * tiles_y;
+    rtx::adaptive_error_kernel<<<(unsigned)((n_tiles * 32 + rtx::kAdaptiveBlock - 1) / rtx::kAdaptiveBlock), rtx::kAdaptiveBlock, 0, c->stream>>>(
+        reinterpret_cast<const float4*>(d_accum), reinterpret_cast<const float4*>(d_aux), width, height, tiles_x, (int)n_tiles, d_tile_error);
+    c->launches += 1;
+    CU(cudaGetLastError());
     return RTX_OK;
 }
 

@@ -3,6 +3,11 @@
 // CWD and reads assets/earth.png relative to it. Optional flags default to the reference values:
 //   --spp N  --width W  --height H  --seed S  --scene-seed S  --gpus N  --out PATH  --chunk N
 //   --checkpoint PATH [--checkpoint-every K]  --resume PATH  --stop-after-chunks N
+//   --adaptive THRESHOLD [--min-spp N] [--step N]
+// --adaptive (one GPU; rtx_render_adaptive): every 8x4 tile stops sampling once its noise estimate is below THRESHOLD,
+// with --spp as the most samples a pixel gets; --min-spp defaults to spp / 64 (at least 2, even), --step to --min-spp.
+// It prints the samples spent and the tiles that converged. Not with --gpus > 1, --checkpoint or --resume: several GPUs
+// would have to decide on their combined buffer every round.
 // Checkpoint / resume (the reference keeps pixels in RAM until the final save_buffer, main.rs:202-231, so a
 // killed 10k-spp render loses everything): after every K chunks each GPU writes its fp32 accumulator and the
 // next sample index it would render to PATH.<gpu>; --resume reloads them (same scene, size, spp, seed, gpus)
@@ -128,6 +133,8 @@ int main(int argc, char** argv) {
     unsigned long long seed = 1, scene_seed = 0;
     bool have_scene_seed = false;
     std::string out = "image.png";
+    double adaptive = -1.0;  // --adaptive THRESHOLD (< 0: uniform sampling)
+    int min_spp = -1, step_spp = -1;
     int worker_rank = -1, shm_fd = -1;  // --worker R --shm-fd FD --device-list L: a worker process of a multi-GPU render (internal)
     std::string device_list = std::getenv("CUDA_VISIBLE_DEVICES") ? std::getenv("CUDA_VISIBLE_DEVICES") : "";
     for (int i = 1; i < argc; ++i) {
@@ -148,6 +155,14 @@ int main(int argc, char** argv) {
         else if (a == "--checkpoint-every") ckpt_every = std::atoi(next("--checkpoint-every"));
         else if (a == "--resume") resume_path = next("--resume");
         else if (a == "--stop-after-chunks") stop_after = std::atoi(next("--stop-after-chunks"));
+        else if (a == "--adaptive") {
+            const char* v = next("--adaptive");
+            char* end = nullptr;
+            adaptive = std::strtod(v, &end);
+            if (*end != 0 || !(adaptive >= 0.0)) { std::fprintf(stderr, "--adaptive needs a threshold >= 0\n"); return 1; }
+        }
+        else if (a == "--min-spp") min_spp = std::atoi(next("--min-spp"));
+        else if (a == "--step") step_spp = std::atoi(next("--step"));
         else if (a == "--worker") worker_rank = std::atoi(next("--worker"));
         else if (a == "--shm-fd") shm_fd = std::atoi(next("--shm-fd"));
         else if (a == "--device-list") device_list = next("--device-list");
@@ -159,6 +174,11 @@ int main(int argc, char** argv) {
         } else { usage(argv[0]); std::fprintf(stderr, "Error: There was an error\n"); return 1; }
     }
     if (scene < 0) { usage(argv[0]); std::fprintf(stderr, "Error: There was an error\n"); return 1; }
+    if (adaptive >= 0.0 && (gpus > 1 || !ckpt_path.empty() || !resume_path.empty())) {
+        std::fprintf(stderr, "--adaptive renders on one GPU without checkpoints: it cannot be combined with --gpus > 1, "
+                             "--checkpoint or --resume\n");
+        return 1;
+    }
     if (worker_rank < 0) std::printf("Scene number: %d\n", scene);
     auto t0 = std::chrono::steady_clock::now();
     rtx_scene_defaults def;
@@ -175,6 +195,36 @@ int main(int argc, char** argv) {
     if (!have_scene_seed) scene_seed = 0x5254544E57ull + (unsigned long long)scene;
     rtx_scene_desc* desc = nullptr;
     RTX(rtx_builtin_scene(scene, scene_seed, nullptr, &desc));
+
+    if (adaptive >= 0.0) {
+        if (min_spp < 0) min_spp = std::max(2, (spp / 64 + 1) / 2 * 2);
+        if (step_spp < 0) step_spp = min_spp;
+        rtx_ctx* ctx = nullptr;
+        rtx_scene* sc = nullptr;
+        float *accum = nullptr, *aux = nullptr;
+        const size_t bytes = (size_t)width * height * 4 * sizeof(float);
+        RTX(rtx_ctx_create(0, nullptr, &ctx));
+        RTX(rtx_scene_create(ctx, desc, &sc));
+        RTX(rtx_malloc(ctx, bytes, (void**)&accum));
+        RTX(rtx_malloc(ctx, bytes, (void**)&aux));
+        rtx_render_params p{width, height, 0, spp, def.max_depth, 0, seed};
+        rtx_adaptive_params ap{adaptive, min_spp, step_spp};
+        rtx_adaptive_stats st{};
+        RTX(rtx_render_adaptive(ctx, sc, &p, &ap, accum, aux, &st));
+        std::vector<uint8_t> rgba((size_t)width * height * 4);
+        RTX(rtx_tonemap_rgba8(ctx, accum, width, height, rgba.data(), 0));
+        RTX(rtx_png_write_rgba8(out.c_str(), width, height, rgba.data()));
+        std::printf("Adaptive sampling: %lld path samples (%.1f per pixel, at most %d), %d rounds, %d of %d tiles converged, %d at %d spp\n",
+                    (long long)st.path_samples, (double)st.path_samples / ((double)width * height), spp, st.rounds,
+                    st.tiles_converged, st.tiles, st.tiles_at_max, spp);
+        rtx_free(ctx, accum);
+        rtx_free(ctx, aux);
+        rtx_scene_destroy(sc);
+        rtx_ctx_destroy(ctx);
+        rtx_scene_desc_free(desc);
+        std::printf("%.6fs\n", std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count());
+        return 0;
+    }
 
     const bool verbose = std::getenv("RTTNW_VERBOSE") != nullptr;
     auto lap = [&](const char* what) {

@@ -1225,6 +1225,11 @@ struct PathPool {
 };
 constexpr int kPoolBytesPerSlot = 8 * 8 + 8 * 4;
 
+struct AdaptiveArgs {
+    const uint32_t* tile_list;  // dispenser tile k renders tile_of_order(tile_list[k], ...)
+    float4* aux;                // receives the samples with an odd global index a second time
+};
+
 struct WfArgs {
     SceneView sc;
     CameraView cam;
@@ -1236,7 +1241,13 @@ struct WfArgs {
     int32_t n_slots;
     unsigned long long total_items;   // tiles * 32 * spp_count
     unsigned long long* next_item;    // global dispenser of path samples
-    OrderArgs order;                  // ray ordering for the trace pass (order.cuh); unused unless the kernel is built with kOrder
+    // Last, what one specialisation of the shade kernel needs, never both: ray ordering for the trace pass (order.cuh,
+    // kOrder) or adaptive sampling (adaptive.cuh, kAdaptive). Sharing the space keeps the size of WfArgs, so the kernel
+    // parameters behind it, and the code of every other shade kernel, stay where they were.
+    union {
+        OrderArgs order;
+        AdaptiveArgs adaptive;
+    };
 };
 
 constexpr int kWfBlock = 128;   // trace kernel CTA; the pool size is a multiple of it

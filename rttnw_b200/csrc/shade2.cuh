@@ -69,7 +69,9 @@ __device__ __forceinline__ void media_after(const SceneView& sc, const RayD& ray
 
 // kPerlinShared (RTX_PERLIN_SMEM=1, scenes with exactly one Perlin table): the 4.75 KB table — 256 gradients and the three
 // byte permutations (noise.rs:5-29) — is staged in shared memory by every CTA and NoiseTexture::value reads it there.
-template <bool kCount, bool kPerlinShared = false, bool kOrder = false>
+// kAdaptive (rtx_render_adaptive, adaptive.cuh): the dispenser's tiles are the entries of a.adaptive.tile_list, and a
+// finished path with an odd sample index is also added to a.adaptive.aux.
+template <bool kCount, bool kPerlinShared = false, bool kOrder = false, bool kAdaptive = false>
 __global__ void __launch_bounds__(kShadeBlock, WF_SHADE_MINB*(128 / kShadeBlock)) wf_shade2_kernel(WfArgs a, float4* __restrict__ accum, unsigned int* active_out,
                                                                                                    Counters* counters) {
     const unsigned FULL = 0xffffffffu;
@@ -113,6 +115,8 @@ __global__ void __launch_bounds__(kShadeBlock, WF_SHADE_MINB*(128 / kShadeBlock)
         apply_albedo(pc, al);
         if (ended) {
             atomicAdd(accum + smp.pixel, make_float4(pc.rad_r, pc.rad_g, pc.rad_b, 1.0f));  // one path sample done
+            if constexpr (kAdaptive)
+                if (smp.sample & 1u) atomicAdd(a.adaptive.aux + smp.pixel, make_float4(pc.rad_r, pc.rad_g, pc.rad_b, 1.0f));
             bounce = -1;
             a.pool.bounce[i] = -1;
         } else {
@@ -134,7 +138,7 @@ __global__ void __launch_bounds__(kShadeBlock, WF_SHADE_MINB*(128 / kShadeBlock)
                 const unsigned int tile = (unsigned int)(group / (unsigned long long)a.spp_count);
                 const unsigned int smp_i = (unsigned int)(group - (unsigned long long)tile * (unsigned long long)a.spp_count);
                 int tx, ty;
-                tile_of_order(tile, a.tiles_x, a.tiles_y, a.inv_per_block_row, tx, ty);
+                tile_of_order(kAdaptive ? __ldg(a.adaptive.tile_list + tile) : tile, a.tiles_x, a.tiles_y, a.inv_per_block_row, tx, ty);
                 const int pi = (int)(item & 31ull);
                 const int px = tx * kTileW + (pi & (kTileW - 1));
                 const int row = ty * kTileH + (pi / kTileW);  // row 0 = top

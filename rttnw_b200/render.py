@@ -200,6 +200,30 @@ class DeviceScene:
         abi.check(self.lib.rtx_render_counted(self.ctx.h, self.h, C.byref(p), accum.data_ptr(), C.byref(st)))
         return {k: getattr(st, k) for k, _ in abi.TraceStats._fields_}
 
+    def render_adaptive(self, accum, aux, threshold: float, min_spp: int, step_spp: int, max_spp: int, seed: int = 1,
+                        max_depth: int = 50, spp_begin: int = 0) -> dict:
+        """Adaptive sampling (rtx_render_adaptive): zeroes accum and aux (H, W, 4) fp32, then renders min_spp samples per
+        pixel and step_spp more per round to every 8x4 tile whose noise estimate is still >= threshold, up to max_spp.
+        Each pixel ends with the samples [spp_begin, spp_begin + n) of the uniform render; aux holds the odd ones.
+        Synchronous; returns the stats."""
+        h, w, _ = accum.shape
+        assert accum.is_contiguous() and aux.is_contiguous() and aux.shape == accum.shape
+        p = abi.RenderParams(w, h, spp_begin, max_spp, max_depth, 0, seed)
+        ap = abi.AdaptiveParams(threshold, min_spp, step_spp)
+        st = abi.AdaptiveStats()
+        abi.check(self.lib.rtx_render_adaptive(self.ctx.h, self.h, C.byref(p), C.byref(ap), accum.data_ptr(),
+                                               aux.data_ptr(), C.byref(st)))
+        return {k: getattr(st, k) for k, _ in abi.AdaptiveStats._fields_}
+
+    def adaptive_error(self, accum, aux):
+        """The per-tile error rtx_render_adaptive decides on, for any (accum, aux) pair: (tiles_y, tiles_x) fp32 on the
+        device, row 0 = top tiles."""
+        h, w, _ = accum.shape
+        t = self.ctx.torch
+        out = t.empty(((h + 3) // 4, (w + 7) // 8), dtype=t.float32, device=accum.device)
+        abi.check(self.lib.rtx_adaptive_error(self.ctx.h, accum.data_ptr(), aux.data_ptr(), w, h, out.data_ptr()))
+        return out
+
     def tonemap(self, accum) -> np.ndarray:
         h, w, _ = accum.shape
         out = np.zeros((h, w, 4), dtype=np.uint8)
@@ -217,9 +241,12 @@ def shard_spp(total_spp: int, rank: int, world_size: int) -> tuple:
 
 def render(scene_number: int, width: Optional[int] = None, height: Optional[int] = None,
            samples: Optional[int] = None, seed: int = 1, device: int = 0, out_path: Optional[str] = None,
-           scene_seed: Optional[int] = None) -> np.ndarray:
+           scene_seed: Optional[int] = None, noise_threshold: Optional[float] = None,
+           min_samples: Optional[int] = None) -> np.ndarray:
     """`render(width, aspect, samples, scene)` of src/main.rs:58 on one GPU; returns RGBA8 (H, W, 4)
-    and, like the reference, writes it as a PNG when `out_path` is given ("image.png" there)."""
+    and, like the reference, writes it as a PNG when `out_path` is given ("image.png" there).
+    With `noise_threshold`, adaptive sampling (DeviceScene.render_adaptive): `samples` is the most a pixel gets,
+    `min_samples` the least (default samples / 64, at least 2, even), each later round adds min_samples."""
     d = scene_defaults(scene_number)
     width, height = width or d["width"], height or d["height"]
     samples = samples or d["samples"]
@@ -227,7 +254,13 @@ def render(scene_number: int, width: Optional[int] = None, height: Optional[int]
     desc = BuiltinDesc(scene_number, scene_seed)
     scene = DeviceScene(ctx, desc)
     accum = scene.new_accum(width, height)
-    scene.render_into(accum, 0, samples, seed=seed, max_depth=d["max_depth"])
+    if noise_threshold is None:
+        scene.render_into(accum, 0, samples, seed=seed, max_depth=d["max_depth"])
+    else:
+        if min_samples is None:
+            min_samples = max(2, (samples // 64 + 1) // 2 * 2)
+        scene.render_adaptive(accum, scene.new_accum(width, height), noise_threshold, min_samples, min_samples, samples,
+                              seed=seed, max_depth=d["max_depth"])
     rgba = scene.tonemap(accum)
     if out_path:
         png_write_rgba8(out_path, rgba)

@@ -150,6 +150,24 @@ pub struct rtx_trace_stats {
     pub instance_enters: f64,
     pub medium_tests: f64,
 }
+/// Adaptive sampling settings (`rtx_render_adaptive`); `rtx_render_params.spp_count` is the largest spp.
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct rtx_adaptive_params {
+    pub threshold: f64,
+    pub min_spp: i32,
+    pub step_spp: i32,
+}
+/// What an adaptive render spent (`rtx_render_adaptive`).
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct rtx_adaptive_stats {
+    pub path_samples: i64,
+    pub rounds: i32,
+    pub tiles: i32,
+    pub tiles_converged: i32,
+    pub tiles_at_max: i32,
+}
 /// The scene table of src/main.rs:66-183 and the defaults of :255.
 #[repr(C)]
 #[derive(Clone, Copy)]
@@ -188,6 +206,8 @@ extern "C" {
     pub fn rtx_trace_rays_stats(ctx: *mut rtx_ctx, scene: *const rtx_scene, n: i64, d_rays: *const rtx_ray, out: *mut rtx_trace_stats) -> c_int;
     pub fn rtx_render(ctx: *mut rtx_ctx, scene: *const rtx_scene, params: *const rtx_render_params, d_accum: *mut f32, d_ray_count: *mut u64) -> c_int;
     pub fn rtx_render_counted(ctx: *mut rtx_ctx, scene: *const rtx_scene, params: *const rtx_render_params, d_accum: *mut f32, out: *mut rtx_trace_stats) -> c_int;
+    pub fn rtx_render_adaptive(ctx: *mut rtx_ctx, scene: *const rtx_scene, params: *const rtx_render_params, adaptive: *const rtx_adaptive_params, d_accum: *mut f32, d_aux: *mut f32, stats: *mut rtx_adaptive_stats) -> c_int;
+    pub fn rtx_adaptive_error(ctx: *mut rtx_ctx, d_accum: *const f32, d_aux: *const f32, width: i32, height: i32, d_tile_error: *mut f32) -> c_int;
     pub fn rtx_tonemap_rgba8(ctx: *mut rtx_ctx, d_accum: *const f32, width: i32, height: i32, out: *mut u8, out_on_device: c_int) -> c_int;
     pub fn rtx_reduce_tonemap_peers(ctx: *mut rtx_ctx, d_accum: *mut f32, d_peer_accums: *const *const f32, n_peers: i32, width: i32, height: i32, d_rgba8: *mut u8) -> c_int;
     pub fn rtx_reduce_tonemap_slice(ctx: *mut rtx_ctx, d_accums: *const *const f32, n_ranks: i32, rank: i32, width: i32, height: i32, d_rgba8_root: *mut u8) -> c_int;

@@ -183,6 +183,37 @@ impl Gpu {
         }
         Ok(pixels)
     }
+
+    /// `render_desc` with adaptive sampling (`rtx_render_adaptive`): every 8x4 tile stops once its noise estimate is
+    /// below `adaptive.threshold`, after at least `adaptive.min_spp` and at most `max_spp` samples per pixel.
+    pub fn render_adaptive_desc(&self, desc: *const ffi::rtx_scene_desc, width: u32, height: u32, max_spp: usize,
+                                adaptive: ffi::rtx_adaptive_params, seed: u64) -> Result<(Vec<u8>, ffi::rtx_adaptive_stats), RtxError> {
+        let bytes = width as usize * height as usize * 16;
+        let mut pixels = vec![0u8; width as usize * height as usize * 4];
+        let mut stats = ffi::rtx_adaptive_stats::default();
+        unsafe {
+            let mut scene = ptr::null_mut();
+            check(ffi::rtx_scene_create(self.ctx, desc, &mut scene))?;
+            let mut accum: *mut c_void = ptr::null_mut();
+            let mut aux: *mut c_void = ptr::null_mut();
+            let result = (|| {
+                check(ffi::rtx_malloc(self.ctx, bytes, &mut accum))?;
+                check(ffi::rtx_malloc(self.ctx, bytes, &mut aux))?;
+                let params = ffi::rtx_render_params { width: width as i32, height: height as i32, spp_begin: 0,
+                                                      spp_count: max_spp as i32, max_depth: 50, _pad: 0, seed };
+                check(ffi::rtx_render_adaptive(self.ctx, scene, &params, &adaptive, accum as *mut f32, aux as *mut f32, &mut stats))?;
+                check(ffi::rtx_tonemap_rgba8(self.ctx, accum as *const f32, width as i32, height as i32, pixels.as_mut_ptr(), 0))
+            })();
+            for p in [accum, aux] {
+                if !p.is_null() {
+                    ffi::rtx_free(self.ctx, p);
+                }
+            }
+            ffi::rtx_scene_destroy(scene);
+            result?;
+        }
+        Ok((pixels, stats))
+    }
 }
 
 impl Drop for Gpu {
