@@ -348,6 +348,27 @@ int rtx_render_adaptive(rtx_ctx* ctx, const rtx_scene* scene, const rtx_render_p
  * This is the same error rtx_render_adaptive decides on, so a user can show a noise map. */
 int rtx_adaptive_error(rtx_ctx* ctx, const float* d_accum, const float* d_aux, int32_t width, int32_t height,
                        float* d_tile_error);
+/* Feature buffers ("AOVs") of the first vertex of every path, for denoisers and compositors. For every pixel and every
+ * global sample index s in [spp_begin, spp_begin + spp_count), take the path rtx_render follows for (pixel, s) with the
+ * same seed: the same camera ray (jitter, lens, shutter time) and the same bounce-0 draws, each ConstantMedium's
+ * free-flight draw included. Its first vertex is the closest of the surface hit and any medium scatter point in front
+ * of it, exactly as the render's bounce 0 decides. Per sample the call adds (layouts width*height, row 0 = top, like
+ * d_accum):
+ *   d_albedo  float4 {sum r, sum g, sum b, n}: Lambertian / Isotropic: the texture value at the vertex; Metal: its
+ *             albedo, whether or not the scatter is absorbed; Dielectric: (1, 1, 1), the reference's attenuation;
+ *             DiffuseLight: its emitted texture value clamped to [0, 1]; a miss: the background clamped to [0, 1].
+ *   d_normal  float4 {sum nx, sum ny, sum nz, n}: the hit record's normal as the render uses it (front-face oriented,
+ *             hittable.rs:30-44); 0 for a medium vertex (whose normal is arbitrary in the reference) and for a miss.
+ *   d_depth   float2 {sum dist, hits}: dist = t * |d|, the distance from the ray's origin on the lens to the vertex;
+ *             only samples that have a vertex add, and `hits` counts them.
+ * The call ADDS into the buffers, so chunked calls compose; a buffer pointer may be NULL (not wanted), all three NULL
+ * is RTX_ERR_INVALID. params is validated like rtx_render's; max_depth must be >= 1 and does not matter otherwise.
+ * Asynchronous on the ctx stream; joins any queued asynchronous job first. Deterministic: each pixel sums its samples
+ * in ascending order in registers and adds the sums once (one thread per pixel, no atomics), so a call's result is
+ * bit-identical from run to run. The samples are keyed like the beauty's: a pass over [0, k) describes the same
+ * paths as the first k samples of a render. */
+int rtx_render_aov(rtx_ctx* ctx, const rtx_scene* scene, const rtx_render_params* params, float* d_albedo,
+                   float* d_normal, float* d_depth);
 /* Rank-0 side of the multi-GPU combine: sums n_peers device accumulators
  * (peer-mapped pointers, read over NVLink) into d_accum and tonemaps in the
  * same kernel. d_rgba8 is a device buffer. Asynchronous. DESTRUCTIVE: d_accum
@@ -421,6 +442,10 @@ int rtx_flatten_check(const rtx_scene_desc* desc, int32_t* n_bvh_nodes, int32_t*
  * RGBA8, RGBA8 encode (image::save_buffer, src/main.rs:231). */
 int rtx_png_read_rgba8(const char* path, int32_t* width, int32_t* height, uint8_t** rgba_out);
 int rtx_png_write_rgba8(const char* path, int32_t width, int32_t height, const uint8_t* rgba);
+/* PFM (portable float map) writer for linear images: channels 3 ("PF") or 1 ("Pf"), anything else is
+ * RTX_ERR_INVALID. `data` is host memory, width*height*channels floats, row 0 = top; the file stores the rows
+ * bottom-up as little-endian floats (scale -1.0). */
+int rtx_pfm_write(const char* path, int32_t width, int32_t height, int32_t channels, const float* data);
 int rtx_buffer_free(void* p);
 
 #ifdef __cplusplus

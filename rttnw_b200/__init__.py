@@ -6,5 +6,5 @@
 """
 from . import abi, scene  # noqa: F401
 from .abi import RtxError  # noqa: F401
-from .render import (BuiltinDesc, Context, DeviceScene, flatten_check, png_read_rgba8, png_write_rgba8,  # noqa: F401
-                     render, scene_defaults, shard_spp)
+from .render import (BuiltinDesc, Context, DeviceScene, flatten_check, pfm_write, png_read_rgba8,  # noqa: F401
+                     png_write_rgba8, render, scene_defaults, shard_spp)

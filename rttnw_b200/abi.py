@@ -139,6 +139,7 @@ SIGNATURES = {
     "rtx_render_adaptive": (C.c_int, [_P, _P, C.POINTER(RenderParams), C.POINTER(AdaptiveParams), _P, _P,
                                       C.POINTER(AdaptiveStats)]),
     "rtx_adaptive_error": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, _P]),
+    "rtx_render_aov": (C.c_int, [_P, _P, C.POINTER(RenderParams), _P, _P, _P]),
     "rtx_tonemap_rgba8": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P, C.c_int]),
     "rtx_reduce_tonemap_peers": (C.c_int, [_P, _P, C.POINTER(_P), C.c_int32, C.c_int32, C.c_int32, _P]),
     "rtx_reduce_tonemap_slice": (C.c_int, [_P, C.POINTER(_P), C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P]),
@@ -163,6 +164,7 @@ SIGNATURES = {
     "rtx_png_read_rgba8": (C.c_int, [C.c_char_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                      C.POINTER(C.POINTER(C.c_uint8))]),
     "rtx_png_write_rgba8": (C.c_int, [C.c_char_p, C.c_int32, C.c_int32, _P]),
+    "rtx_pfm_write": (C.c_int, [C.c_char_p, C.c_int32, C.c_int32, C.c_int32, _P]),
     "rtx_buffer_free": (C.c_int, [_P]),
 }
 

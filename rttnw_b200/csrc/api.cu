@@ -21,6 +21,7 @@
 #include "../../include/rttnw_b200.h"
 #include "flatten.hpp"
 #include "adaptive.cuh"
+#include "aov.cuh"
 #include "kernels.cuh"
 #include "lbvh.cuh"
 #include "sah_build.cuh"
@@ -1277,6 +1278,36 @@ int rtx_adaptive_error(rtx_ctx* c, const float* d_accum, const float* d_aux, int
     return RTX_OK;
 }
 
+// ---- feature buffers (aov.cuh) -------------------------------------------------
+int rtx_render_aov(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, float* d_albedo, float* d_normal,
+                   float* d_depth) {
+    if (!c || !s || !p) return fail(RTX_ERR_INVALID, "NULL argument");
+    if (!d_albedo && !d_normal && !d_depth) return fail(RTX_ERR_INVALID, "no feature buffer given");
+    if (p->width <= 0 || p->height <= 0 || p->spp_count < 0 || p->spp_begin < 0 || p->max_depth < 1)
+        return fail(RTX_ERR_INVALID, "bad render parameters (the feature pass needs max_depth >= 1)");
+    if ((int64_t)p->width * p->height > 0x7fffffff) return fail(RTX_ERR_INVALID, "image too large");
+    if (p->spp_count > (1 << 24)) return fail(RTX_ERR_INVALID, "more than 2^24 samples per pixel in one call (the fp32 sample count of the buffers)");
+    JOIN(c);
+    if (p->spp_count == 0) return RTX_OK;
+    CU(cudaSetDevice(c->device));
+    rtx::AovArgs a;
+    a.sc = s->view;
+    a.cam = s->camera;
+    a.width = p->width; a.height = p->height;
+    a.spp_begin = p->spp_begin; a.spp_count = p->spp_count;
+    a.k0 = (uint32_t)p->seed; a.k1 = (uint32_t)(p->seed >> 32);
+    a.tiles_x = (p->width + rtx::kTileW - 1) / rtx::kTileW;
+    a.albedo = reinterpret_cast<float4*>(d_albedo);
+    a.normal = reinterpret_cast<float4*>(d_normal);
+    a.depth = reinterpret_cast<float2*>(d_depth);
+    const int64_t n_tiles = (int64_t)a.tiles_x * ((p->height + rtx::kTileH - 1) / rtx::kTileH);
+    const int64_t grid = (n_tiles * 32 + rtx::kAovBlock - 1) / rtx::kAovBlock;
+    rtx::aov_kernel<<<(unsigned)grid, rtx::kAovBlock, 0, c->stream>>>(a);
+    c->launches += 1;
+    CU(cudaGetLastError());
+    return RTX_OK;
+}
+
 int rtx_tonemap_rgba8(rtx_ctx* c, const float* d_accum, int32_t width, int32_t height, uint8_t* out, int out_on_device) {
     if (!c || !d_accum || !out || width <= 0 || height <= 0) return fail(RTX_ERR_INVALID, "bad argument");
     JOIN(c);
@@ -1592,6 +1623,13 @@ int rtx_png_write_rgba8(const char* path, int32_t width, int32_t height, const u
     if (!path || !rgba) return fail(RTX_ERR_INVALID, "NULL argument");
     std::string err;
     if (!rttnw::png_write_rgba8(path, width, height, rgba, err)) return fail(RTX_ERR_IO, err);
+    return RTX_OK;
+}
+int rtx_pfm_write(const char* path, int32_t width, int32_t height, int32_t channels, const float* data) {
+    if (!path || !data) return fail(RTX_ERR_INVALID, "NULL argument");
+    if (width <= 0 || height <= 0 || (channels != 1 && channels != 3)) return fail(RTX_ERR_INVALID, "bad PFM size or channel count (1 or 3)");
+    std::string err;
+    if (!rttnw::pfm_write(path, width, height, channels, data, err)) return fail(RTX_ERR_IO, err);
     return RTX_OK;
 }
 int rtx_buffer_free(void* p) {

@@ -3,11 +3,16 @@
 // CWD and reads assets/earth.png relative to it. Optional flags default to the reference values:
 //   --spp N  --width W  --height H  --seed S  --scene-seed S  --gpus N  --out PATH  --chunk N
 //   --checkpoint PATH [--checkpoint-every K]  --resume PATH  --stop-after-chunks N
-//   --adaptive THRESHOLD [--min-spp N] [--step N]
+//   --adaptive THRESHOLD [--min-spp N] [--step N]  --aov PREFIX [--aov-spp N]
 // --adaptive (one GPU; rtx_render_adaptive): every 8x4 tile stops sampling once its noise estimate is below THRESHOLD,
 // with --spp as the most samples a pixel gets; --min-spp defaults to spp / 64 (at least 2, even), --step to --min-spp.
 // It prints the samples spent and the tiles that converged. Not with --gpus > 1, --checkpoint or --resume: several GPUs
 // would have to decide on their combined buffer every round.
+// --aov PREFIX (rtx_render_aov): after the frame, the feature pass renders samples [0, N) (--aov-spp, default
+// min(16, spp)) on the device that writes image.png and, exactly when image.png is written, writes four PFMs: PREFIX.beauty.pfm,
+// the linear mean radiance accum.rgb / accum.w of the accumulator image.png is tonemapped from (after the multi-GPU
+// combine), PREFIX.albedo.pfm and PREFIX.normal.pfm, the means over the N samples (normals not renormalised), and
+// PREFIX.depth.pfm (one channel), the mean distance over the samples that hit, 0 where none did.
 // Checkpoint / resume (the reference keeps pixels in RAM until the final save_buffer, main.rs:202-231, so a
 // killed 10k-spp render loses everything): after every K chunks each GPU writes its fp32 accumulator and the
 // next sample index it would render to PATH.<gpu>; --resume reloads them (same scene, size, spp, seed, gpus)
@@ -64,6 +69,42 @@ static void usage(const char* argv0) {  // main.rs:239-249
             return 1;                                                        \
         }                                                                    \
     } while (0)
+
+// The feature pass and the four PFMs of --aov (see the top of this file). d_accum holds the frame's samples.
+static int write_aov(rtx_ctx* ctx, rtx_scene* sc, const float* d_accum, int width, int height, int aov_spp, int max_depth,
+                     unsigned long long seed, const std::string& prefix) {
+    const size_t n = (size_t)width * height;
+    float *d_albedo = nullptr, *d_normal = nullptr, *d_depth = nullptr;
+    RTX(rtx_malloc(ctx, n * 40, (void**)&d_albedo));
+    d_normal = d_albedo + 4 * n;
+    d_depth = d_normal + 4 * n;
+    RTX(rtx_memset_zero(ctx, d_albedo, n * 40));
+    rtx_render_params p;
+    std::memset(&p, 0, sizeof(p));
+    p.width = width; p.height = height; p.spp_begin = 0; p.spp_count = aov_spp; p.max_depth = max_depth; p.seed = seed;
+    RTX(rtx_render_aov(ctx, sc, &p, d_albedo, d_normal, d_depth));
+    std::vector<float> acc(n * 4), aov(n * 10);
+    RTX(rtx_memcpy_d2h(ctx, acc.data(), d_accum, acc.size() * sizeof(float)));
+    RTX(rtx_memcpy_d2h(ctx, aov.data(), d_albedo, aov.size() * sizeof(float)));
+    rtx_free(ctx, d_albedo);
+    const float* al = aov.data();
+    const float* nm = al + 4 * n;
+    const float* dp = nm + 4 * n;
+    std::vector<float> beauty(n * 3), albedo(n * 3), normal(n * 3), depth(n);
+    for (size_t i = 0; i < n; ++i) {
+        for (int c = 0; c < 3; ++c) {
+            beauty[3 * i + c] = acc[4 * i + c] / acc[4 * i + 3];
+            albedo[3 * i + c] = al[4 * i + c] / al[4 * i + 3];
+            normal[3 * i + c] = nm[4 * i + c] / nm[4 * i + 3];
+        }
+        depth[i] = dp[2 * i + 1] > 0.f ? dp[2 * i] / dp[2 * i + 1] : 0.f;
+    }
+    RTX(rtx_pfm_write((prefix + ".beauty.pfm").c_str(), width, height, 3, beauty.data()));
+    RTX(rtx_pfm_write((prefix + ".albedo.pfm").c_str(), width, height, 3, albedo.data()));
+    RTX(rtx_pfm_write((prefix + ".normal.pfm").c_str(), width, height, 3, normal.data()));
+    RTX(rtx_pfm_write((prefix + ".depth.pfm").c_str(), width, height, 1, depth.data()));
+    return 0;
+}
 
 struct Rank {
     rtx_ctx* ctx = nullptr;
@@ -135,6 +176,8 @@ int main(int argc, char** argv) {
     std::string out = "image.png";
     double adaptive = -1.0;  // --adaptive THRESHOLD (< 0: uniform sampling)
     int min_spp = -1, step_spp = -1;
+    std::string aov_prefix;  // --aov PREFIX: the feature pass and the PFMs
+    long long aov_spp = -1;
     int worker_rank = -1, shm_fd = -1;  // --worker R --shm-fd FD --device-list L: a worker process of a multi-GPU render (internal)
     std::string device_list = std::getenv("CUDA_VISIBLE_DEVICES") ? std::getenv("CUDA_VISIBLE_DEVICES") : "";
     for (int i = 1; i < argc; ++i) {
@@ -163,6 +206,13 @@ int main(int argc, char** argv) {
         }
         else if (a == "--min-spp") min_spp = std::atoi(next("--min-spp"));
         else if (a == "--step") step_spp = std::atoi(next("--step"));
+        else if (a == "--aov") aov_prefix = next("--aov");
+        else if (a == "--aov-spp") {
+            const char* v = next("--aov-spp");
+            char* end = nullptr;
+            aov_spp = std::strtoll(v, &end, 10);
+            if (*end != 0 || aov_spp < 1 || aov_spp > (1 << 24)) { std::fprintf(stderr, "--aov-spp needs a sample count in [1, 2^24]\n"); return 1; }
+        }
         else if (a == "--worker") worker_rank = std::atoi(next("--worker"));
         else if (a == "--shm-fd") shm_fd = std::atoi(next("--shm-fd"));
         else if (a == "--device-list") device_list = next("--device-list");
@@ -179,6 +229,7 @@ int main(int argc, char** argv) {
                              "--checkpoint or --resume\n");
         return 1;
     }
+    if (aov_spp > 0 && aov_prefix.empty()) { std::fprintf(stderr, "--aov-spp needs --aov PREFIX\n"); return 1; }
     if (worker_rank < 0) std::printf("Scene number: %d\n", scene);
     auto t0 = std::chrono::steady_clock::now();
     rtx_scene_defaults def;
@@ -193,6 +244,7 @@ int main(int argc, char** argv) {
     if (gpus < 1) gpus = 1;
     if (chunk < 1) chunk = 1;
     if (!have_scene_seed) scene_seed = 0x5254544E57ull + (unsigned long long)scene;
+    if (aov_spp < 0) aov_spp = std::max(1, std::min(16, spp));
     rtx_scene_desc* desc = nullptr;
     RTX(rtx_builtin_scene(scene, scene_seed, nullptr, &desc));
 
@@ -214,6 +266,7 @@ int main(int argc, char** argv) {
         std::vector<uint8_t> rgba((size_t)width * height * 4);
         RTX(rtx_tonemap_rgba8(ctx, accum, width, height, rgba.data(), 0));
         RTX(rtx_png_write_rgba8(out.c_str(), width, height, rgba.data()));
+        if (!aov_prefix.empty() && write_aov(ctx, sc, accum, width, height, (int)aov_spp, def.max_depth, seed, aov_prefix) != 0) return 1;
         std::printf("Adaptive sampling: %lld path samples (%.1f per pixel, at most %d), %d rounds, %d of %d tiles converged, %d at %d spp\n",
                     (long long)st.path_samples, (double)st.path_samples / ((double)width * height), spp, st.rounds,
                     st.tiles_converged, st.tiles, st.tiles_at_max, spp);
@@ -426,6 +479,13 @@ int main(int argc, char** argv) {
         lap("frame on the host");
         RTX(rtx_png_write_rgba8(out.c_str(), width, height, rgba_mp.data()));
         lap("png written");
+        if (!aov_prefix.empty()) {
+            if (write_aov(k.ctx, k.scene, k.accum, width, height, (int)aov_spp, def.max_depth, seed, aov_prefix) != 0) {
+                for (int r = 1; r < gpus; ++r) if (pids[(size_t)r] > 0) waitpid(pids[(size_t)r], nullptr, 0);
+                return 1;
+            }
+            lap("feature buffers written");
+        }
         double secs_mp = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
         std::printf("%.6fs\n", secs_mp);  // println!("{:?}", instant.elapsed())
         std::fflush(stdout);
@@ -447,6 +507,10 @@ int main(int argc, char** argv) {
     lap("frame on the host");
     RTX(rtx_png_write_rgba8(out.c_str(), width, height, rgba.data()));  // image::save_buffer("image.png", ..), main.rs:231
     lap("png written");
+    if (!aov_prefix.empty()) {
+        if (write_aov(ranks[0].ctx, ranks[0].scene, ranks[0].accum, width, height, (int)aov_spp, def.max_depth, seed, aov_prefix) != 0) return 1;
+        lap("feature buffers written");
+    }
     rtx_free(ranks[0].ctx, d_rgba);
     for (auto& k : ranks) {
         rtx_free(k.ctx, k.accum);

@@ -2,6 +2,7 @@
 // Reader: what ImageTexture::new needs (src/math/texture.rs:69-75 decodes via the `image`
 // crate and converts to RGBA8): 8/16-bit gray, gray+alpha, RGB, RGBA and 8-bit palette,
 // non-interlaced. Writer: image::save_buffer(.., ColorType::Rgba8) of src/main.rs:231.
+// Also the PFM writer of the linear beauty and the feature buffers (rtx_pfm_write).
 #include <zlib.h>
 
 #include <cstdio>
@@ -165,6 +166,32 @@ bool png_write_rgba8(const char* path, int width, int height, const uint8_t* rgb
     size_t wr = std::fwrite(out.data(), 1, out.size(), f);
     std::fclose(f);
     if (wr != out.size()) { err = "short write"; return false; }
+    return true;
+}
+
+// Portable float map: "PF" (RGB) or "Pf" (grey), then "width height", then the scale, negative for little-endian
+// samples; the rows follow bottom-up. `data` has row 0 = top, like the accumulators.
+bool pfm_write(const char* path, int width, int height, int channels, const float* data, std::string& err) {
+    if (width <= 0 || height <= 0 || (channels != 1 && channels != 3) || !data) { err = "bad float map"; return false; }
+    const size_t row = (size_t)width * channels;
+    char hdr[64];
+    int n = std::snprintf(hdr, sizeof(hdr), "%s\n%d %d\n-1.0\n", channels == 3 ? "PF" : "Pf", width, height);
+    std::vector<uint8_t> out(hdr, hdr + n);
+    out.reserve((size_t)n + row * 4 * (size_t)height);
+    for (int y = height - 1; y >= 0; --y) {
+        const float* src = data + row * (size_t)y;
+        for (size_t i = 0; i < row; ++i) {
+            uint32_t u;
+            std::memcpy(&u, src + i, 4);
+            const uint8_t b[4] = {(uint8_t)u, (uint8_t)(u >> 8), (uint8_t)(u >> 16), (uint8_t)(u >> 24)};
+            out.insert(out.end(), b, b + 4);
+        }
+    }
+    FILE* f = std::fopen(path, "wb");
+    if (!f) { err = std::string("cannot open for writing: ") + path; return false; }
+    size_t wr = std::fwrite(out.data(), 1, out.size(), f);
+    bool ok = std::fclose(f) == 0 && wr == out.size();
+    if (!ok) { err = "short write"; return false; }
     return true;
 }
 

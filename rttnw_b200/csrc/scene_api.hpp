@@ -123,5 +123,7 @@ bool builtin_scene(int scene_number, uint64_t seed, const char* earth_png_path, 
 // PNG (zlib): returns false on failure.
 bool png_read_rgba8(const char* path, int& width, int& height, std::vector<uint8_t>& rgba, std::string& err);
 bool png_write_rgba8(const char* path, int width, int height, const uint8_t* rgba, std::string& err);
+// PFM, 1 or 3 little-endian float channels (rtx_pfm_write)
+bool pfm_write(const char* path, int width, int height, int channels, const float* data, std::string& err);
 
 }  // namespace rttnw

@@ -36,6 +36,18 @@ def png_write_rgba8(path: str, rgba: np.ndarray) -> None:
     abi.check(abi.load().rtx_png_write_rgba8(path.encode(), rgba.shape[1], rgba.shape[0], rgba.ctypes.data))
 
 
+def pfm_write(path: str, image: np.ndarray) -> None:
+    """Writes a linear float image (H, W, 3) or (H, W), row 0 = top, as a PFM (rtx_pfm_write)."""
+    image = np.ascontiguousarray(image, dtype=np.float32)
+    if image.ndim == 2:
+        channels = 1
+    elif image.ndim == 3 and image.shape[2] == 3:
+        channels = 3
+    else:
+        raise ValueError(f"pfm_write takes (H, W, 3) or (H, W), got {image.shape}")
+    abi.check(abi.load().rtx_pfm_write(path.encode(), image.shape[1], image.shape[0], channels, image.ctypes.data))
+
+
 def scene_defaults(number: int) -> dict:
     """Resolution / spp / depth of the scene table, src/main.rs:66-183,255."""
     d = abi.SceneDefaults()
@@ -224,11 +236,49 @@ class DeviceScene:
         abi.check(self.lib.rtx_adaptive_error(self.ctx.h, accum.data_ptr(), aux.data_ptr(), w, h, out.data_ptr()))
         return out
 
+    def new_aov(self, width: int, height: int) -> dict:
+        """Zeroed feature buffers for render_aov: albedo and normal (H, W, 4) {sum x, sum y, sum z, samples}, depth
+        (H, W, 2) {sum distance, samples with a vertex}, fp32 on this context's device."""
+        t = self.ctx.torch
+        dev = f"cuda:{self.ctx.device}"
+        return {"albedo": t.zeros((height, width, 4), dtype=t.float32, device=dev),
+                "normal": t.zeros((height, width, 4), dtype=t.float32, device=dev),
+                "depth": t.zeros((height, width, 2), dtype=t.float32, device=dev)}
+
+    def render_aov(self, aov: dict, spp_begin: int, spp_count: int, seed: int = 1, max_depth: int = 50) -> None:
+        """Adds the first-vertex albedo, normal and distance of the paths (pixel, s), s in [spp_begin, spp_begin +
+        spp_count), into the buffers of `aov` (rtx_render_aov; see new_aov). A key that is missing or None is not
+        computed. Asynchronous on the context's stream."""
+        bufs = [aov.get(k) for k in ("albedo", "normal", "depth")]
+        given = [b for b in bufs if b is not None]
+        if not given:
+            raise ValueError("render_aov needs at least one of albedo, normal, depth")
+        h, w = given[0].shape[:2]
+        for b, c in zip(bufs, (4, 4, 2)):
+            if b is not None:
+                assert b.is_contiguous() and b.dtype == self.ctx.torch.float32 and tuple(b.shape) == (h, w, c)
+        p = abi.RenderParams(w, h, spp_begin, spp_count, max_depth, 0, seed)
+        ptrs = [b.data_ptr() if b is not None else None for b in bufs]
+        abi.check(self.lib.rtx_render_aov(self.ctx.h, self.h, C.byref(p), *ptrs))
+
     def tonemap(self, accum) -> np.ndarray:
         h, w, _ = accum.shape
         out = np.zeros((h, w, 4), dtype=np.uint8)
         abi.check(self.lib.rtx_tonemap_rgba8(self.ctx.h, accum.data_ptr(), w, h, out.ctypes.data, 0))
         return out
+
+
+def write_aov_files(prefix: str, accum, aov: dict) -> None:
+    """PREFIX.beauty.pfm (the linear mean radiance accum.rgb / accum.w the PNG is tonemapped from), PREFIX.albedo.pfm
+    and PREFIX.normal.pfm (means over the feature samples; the normals are not renormalised) and PREFIX.depth.pfm (one
+    channel: the mean distance over the samples that hit, 0 where none did) — the files the CLI's --aov writes."""
+    acc = accum.cpu().numpy().astype(np.float64)
+    al, nm, dp = (aov[k].cpu().numpy().astype(np.float64) for k in ("albedo", "normal", "depth"))
+    with np.errstate(divide="ignore", invalid="ignore"):
+        pfm_write(prefix + ".beauty.pfm", acc[..., :3] / acc[..., 3:4])
+        pfm_write(prefix + ".albedo.pfm", al[..., :3] / al[..., 3:4])
+        pfm_write(prefix + ".normal.pfm", nm[..., :3] / nm[..., 3:4])
+        pfm_write(prefix + ".depth.pfm", np.where(dp[..., 1] > 0, dp[..., 0] / np.maximum(dp[..., 1], 1.0), 0.0))
 
 
 def shard_spp(total_spp: int, rank: int, world_size: int) -> tuple:
@@ -242,11 +292,13 @@ def shard_spp(total_spp: int, rank: int, world_size: int) -> tuple:
 def render(scene_number: int, width: Optional[int] = None, height: Optional[int] = None,
            samples: Optional[int] = None, seed: int = 1, device: int = 0, out_path: Optional[str] = None,
            scene_seed: Optional[int] = None, noise_threshold: Optional[float] = None,
-           min_samples: Optional[int] = None) -> np.ndarray:
+           min_samples: Optional[int] = None, aov_prefix: Optional[str] = None, aov_samples: int = 16) -> np.ndarray:
     """`render(width, aspect, samples, scene)` of src/main.rs:58 on one GPU; returns RGBA8 (H, W, 4)
     and, like the reference, writes it as a PNG when `out_path` is given ("image.png" there).
     With `noise_threshold`, adaptive sampling (DeviceScene.render_adaptive): `samples` is the most a pixel gets,
-    `min_samples` the least (default samples / 64, at least 2, even), each later round adds min_samples."""
+    `min_samples` the least (default samples / 64, at least 2, even), each later round adds min_samples.
+    With `aov_prefix`, also writes the linear frame and the feature buffers of samples [0, aov_samples) as PFMs (see
+    write_aov_files): the input of a denoiser such as OIDN or the OptiX denoiser."""
     d = scene_defaults(scene_number)
     width, height = width or d["width"], height or d["height"]
     samples = samples or d["samples"]
@@ -264,6 +316,10 @@ def render(scene_number: int, width: Optional[int] = None, height: Optional[int]
     rgba = scene.tonemap(accum)
     if out_path:
         png_write_rgba8(out_path, rgba)
+    if aov_prefix:
+        aov = scene.new_aov(width, height)
+        scene.render_aov(aov, 0, aov_samples, seed=seed, max_depth=d["max_depth"])
+        write_aov_files(aov_prefix, accum, aov)
     scene.close()
     ctx.close()
     return rgba

@@ -4,6 +4,7 @@
 use std::os::raw::{c_char, c_int, c_void};
 
 pub const RTX_OK: c_int = 0;
+pub const RTX_ERR_INVALID: c_int = -1;
 pub const RTX_MISS: i32 = -1;
 
 // rtx_node_kind
@@ -208,6 +209,7 @@ extern "C" {
     pub fn rtx_render_counted(ctx: *mut rtx_ctx, scene: *const rtx_scene, params: *const rtx_render_params, d_accum: *mut f32, out: *mut rtx_trace_stats) -> c_int;
     pub fn rtx_render_adaptive(ctx: *mut rtx_ctx, scene: *const rtx_scene, params: *const rtx_render_params, adaptive: *const rtx_adaptive_params, d_accum: *mut f32, d_aux: *mut f32, stats: *mut rtx_adaptive_stats) -> c_int;
     pub fn rtx_adaptive_error(ctx: *mut rtx_ctx, d_accum: *const f32, d_aux: *const f32, width: i32, height: i32, d_tile_error: *mut f32) -> c_int;
+    pub fn rtx_render_aov(ctx: *mut rtx_ctx, scene: *const rtx_scene, params: *const rtx_render_params, d_albedo: *mut f32, d_normal: *mut f32, d_depth: *mut f32) -> c_int;
     pub fn rtx_tonemap_rgba8(ctx: *mut rtx_ctx, d_accum: *const f32, width: i32, height: i32, out: *mut u8, out_on_device: c_int) -> c_int;
     pub fn rtx_reduce_tonemap_peers(ctx: *mut rtx_ctx, d_accum: *mut f32, d_peer_accums: *const *const f32, n_peers: i32, width: i32, height: i32, d_rgba8: *mut u8) -> c_int;
     pub fn rtx_reduce_tonemap_slice(ctx: *mut rtx_ctx, d_accums: *const *const f32, n_ranks: i32, rank: i32, width: i32, height: i32, d_rgba8_root: *mut u8) -> c_int;
@@ -230,5 +232,6 @@ extern "C" {
     pub fn rtx_flatten_check(desc: *const rtx_scene_desc, n_bvh_nodes: *mut i32, n_records: *mut i32, n_prim_ids: *mut i32) -> c_int;
     pub fn rtx_png_read_rgba8(path: *const c_char, width: *mut i32, height: *mut i32, rgba_out: *mut *mut u8) -> c_int;
     pub fn rtx_png_write_rgba8(path: *const c_char, width: i32, height: i32, rgba: *const u8) -> c_int;
+    pub fn rtx_pfm_write(path: *const c_char, width: i32, height: i32, channels: i32, data: *const f32) -> c_int;
     pub fn rtx_buffer_free(p: *mut c_void) -> c_int;
 }

@@ -20,7 +20,7 @@ pub mod scenes;
 pub use render::{render, render_world, scene_setup, shard_spp};
 
 use std::collections::HashMap;
-use std::ffi::CStr;
+use std::ffi::{CStr, CString};
 use std::os::raw::c_void;
 use std::ptr;
 
@@ -214,6 +214,53 @@ impl Gpu {
         }
         Ok((pixels, stats))
     }
+
+    /// The feature buffers of samples [0, samples) (`rtx_render_aov`): the albedo, normal and distance of every
+    /// path's first vertex, for a denoiser or a compositor. Host copies, row 0 = top: albedo and normal
+    /// `{sum x, sum y, sum z, samples}` per pixel, depth `{sum distance, samples with a vertex}`.
+    pub fn render_aov(&self, desc: *const ffi::rtx_scene_desc, width: u32, height: u32, samples: usize,
+                      seed: u64) -> Result<Aov, RtxError> {
+        let n = width as usize * height as usize;
+        let mut out = Aov { albedo: vec![0.0; 4 * n], normal: vec![0.0; 4 * n], depth: vec![0.0; 2 * n] };
+        unsafe {
+            let mut scene = ptr::null_mut();
+            check(ffi::rtx_scene_create(self.ctx, desc, &mut scene))?;
+            let mut d: *mut c_void = ptr::null_mut();
+            let result = (|| {
+                check(ffi::rtx_malloc(self.ctx, 40 * n, &mut d))?;
+                check(ffi::rtx_memset_zero(self.ctx, d, 40 * n))?;
+                let (albedo, normal, depth) = (d as *mut f32, (d as *mut f32).add(4 * n), (d as *mut f32).add(8 * n));
+                let params = ffi::rtx_render_params { width: width as i32, height: height as i32, spp_begin: 0,
+                                                      spp_count: samples as i32, max_depth: 50, _pad: 0, seed };
+                check(ffi::rtx_render_aov(self.ctx, scene, &params, albedo, normal, depth))?;
+                check(ffi::rtx_memcpy_d2h(self.ctx, out.albedo.as_mut_ptr() as *mut c_void, albedo as *const c_void, 16 * n))?;
+                check(ffi::rtx_memcpy_d2h(self.ctx, out.normal.as_mut_ptr() as *mut c_void, normal as *const c_void, 16 * n))?;
+                check(ffi::rtx_memcpy_d2h(self.ctx, out.depth.as_mut_ptr() as *mut c_void, depth as *const c_void, 8 * n))
+            })();
+            if !d.is_null() {
+                ffi::rtx_free(self.ctx, d);
+            }
+            ffi::rtx_scene_destroy(scene);
+            result?;
+        }
+        Ok(out)
+    }
+}
+
+/// Sums of `Gpu::render_aov`, host side (see there).
+pub struct Aov {
+    pub albedo: Vec<f32>,
+    pub normal: Vec<f32>,
+    pub depth: Vec<f32>,
+}
+
+/// Writes a linear float image as a PFM (`rtx_pfm_write`): `channels` 3 or 1, `data` row 0 = top.
+pub fn pfm_write(path: &str, width: u32, height: u32, channels: u32, data: &[f32]) -> Result<(), RtxError> {
+    if data.len() != width as usize * height as usize * channels as usize {
+        return Err(RtxError { status: ffi::RTX_ERR_INVALID, message: "pfm_write: data does not match the size".into() });
+    }
+    let c = CString::new(path).map_err(|_| RtxError { status: ffi::RTX_ERR_INVALID, message: "path contains a NUL".into() })?;
+    check(unsafe { ffi::rtx_pfm_write(c.as_ptr(), width as i32, height as i32, channels as i32, data.as_ptr()) })
 }
 
 impl Drop for Gpu {
