@@ -369,6 +369,41 @@ int rtx_adaptive_error(rtx_ctx* ctx, const float* d_accum, const float* d_aux, i
  * paths as the first k samples of a render. */
 int rtx_render_aov(rtx_ctx* ctx, const rtx_scene* scene, const rtx_render_params* params, float* d_albedo,
                    float* d_normal, float* d_depth);
+/* Denoiser: an edge-avoiding à-trous wavelet filter (Dammertz et al., HPG 2010) steered by a per-pixel variance
+ * estimate (as in SVGF, Schied et al., HPG 2017), over the beauty and the feature buffers. All buffers are device
+ * memory, width*height float4, row 0 = top: d_accum as rtx_render fills it; d_half a subset of the same samples chosen
+ * without looking at their values (the d_aux of rtx_render_adaptive, or the accumulator copied with rtx_memcpy_d2d
+ * between the renders of [0, n/2) and [n/2, n)); d_albedo and d_normal as rtx_render_aov fills them. d_out receives
+ * {r, g, b, 1}, which rtx_tonemap_rgba8 and rtx_pfm_write (after dropping .w) take unchanged.
+ * Per pixel p, with L(x) = 0.2126 x.r + 0.7152 x.g + 0.0722 x.b:
+ *   n = accum.w, m = half.w; a pixel with n == 0 has no samples: it contributes nothing and outputs {0, 0, 0, 1}.
+ *   c = accum.rgb / n;  a = albedo.rgb / albedo.w (0 if albedo.w == 0);  a' = max(a, 1e-3) per channel;
+ *   N = normal.xyz / normal.w (0 if normal.w == 0), not renormalised (0 at medium vertices and misses);
+ *   e = c / a' (demodulated irradiance);
+ *   v = L((H - R) / a')^2 * m (n - m) / n^2 if 0 < m < n, else 0, where H = half.rgb / m, R = (accum.rgb - half.rgb) /
+ *       (n - m): since E[(H - R)^2] = sigma^2 n / (m (n - m)), v estimates the variance of the mean, sigma^2 / n.
+ * Pass i = 0 .. iterations-1, step s = 2^i, over the pixels with samples:
+ *   g_p = sum k v_q / sum k over the 3x3 neighbours q (step 1) in the frame with samples, k = [1/4, 1/2, 1/4] per axis;
+ *   for the taps q = p + s (dx, dy), dx, dy in -2..2, in the frame and with samples, with h = [1, 4, 6, 4, 1] / 16:
+ *     w = h(dx) h(dy) exp(-|N_p - N_q|^2 / sigma_normal^2 - |a_p - a_q|^2 / sigma_albedo^2
+ *                         - |L(e_p) - L(e_q)| / (sigma_luminance sqrt(g_p) + 1e-10));
+ *   e_p <- sum w e_q / sum w,  v_p <- sum w^2 v_q / (sum w)^2  (all pixels update from the previous pass's values).
+ * Output: out_p = {e_p a'_p, 1}. Depth is deliberately not a weight: at a medium vertex it is a free-flight draw.
+ * The output is BIASED, unlike every other output of the library: a filtered estimate, not a sample mean.
+ * Asynchronous on the ctx stream; joins any queued asynchronous job first. Deterministic (one thread per pixel, no
+ * atomics): bit-identical from run to run. The inputs are not modified. RTX_ERR_INVALID: a NULL or not 16-byte
+ * aligned buffer (the kernels load and store float4), a d_out that overlaps an input, a size <= 0 or of 2^31 pixels or
+ * more, iterations outside [1, 10], a sigma <= 0 or not finite, and a sigma_normal or sigma_albedo below about 5.4e-20
+ * (the kernels multiply by 1 / sigma^2 in fp32, which must be finite). Any width and height within 2^31 pixels are
+ * accepted. The context keeps 56 bytes a pixel of scratch, grown as needed. params == NULL takes the defaults below. */
+typedef struct rtx_denoise_params {
+    int32_t iterations;    /* à-trous passes, in [1, 10]; pass i takes taps 2^i pixels apart (default 5) */
+    float sigma_normal;    /* > 0, finite (default 0.25) */
+    float sigma_albedo;    /* > 0, finite (default 0.1) */
+    float sigma_luminance; /* > 0, finite (default 8) */
+} rtx_denoise_params;      /* 16 bytes */
+int rtx_denoise(rtx_ctx* ctx, const float* d_accum, const float* d_half, const float* d_albedo, const float* d_normal,
+                int32_t width, int32_t height, const rtx_denoise_params* params, float* d_out);
 /* Rank-0 side of the multi-GPU combine: sums n_peers device accumulators
  * (peer-mapped pointers, read over NVLink) into d_accum and tonemaps in the
  * same kernel. d_rgba8 is a device buffer. Asynchronous. DESTRUCTIVE: d_accum
@@ -405,6 +440,8 @@ int rtx_free(rtx_ctx* ctx, void* ptr);
 int rtx_memset_zero(rtx_ctx* ctx, void* ptr, size_t bytes);
 int rtx_memcpy_h2d(rtx_ctx* ctx, void* dst, const void* src, size_t bytes);
 int rtx_memcpy_d2h(rtx_ctx* ctx, void* dst, const void* src, size_t bytes);
+/* device to device, asynchronous on the ctx stream (e.g. the d_half of rtx_denoise) */
+int rtx_memcpy_d2d(rtx_ctx* ctx, void* dst, const void* src, size_t bytes);
 int rtx_ipc_export(rtx_ctx* ctx, void* d_ptr, uint8_t handle_out[64]);
 int rtx_ipc_open(rtx_ctx* ctx, const uint8_t handle[64], void** d_ptr_out);
 int rtx_ipc_close(rtx_ctx* ctx, void* d_ptr);

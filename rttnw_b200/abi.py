@@ -100,9 +100,14 @@ class AdaptiveStats(C.Structure):
                 ("tiles_converged", C.c_int32), ("tiles_at_max", C.c_int32)]
 
 
+class DenoiseParams(C.Structure):
+    _fields_ = [("iterations", C.c_int32), ("sigma_normal", C.c_float), ("sigma_albedo", C.c_float),
+                ("sigma_luminance", C.c_float)]
+
+
 assert C.sizeof(Node) == 96 and C.sizeof(Material) == 40 and C.sizeof(Texture) == 48
 assert C.sizeof(Ray) == 80 and C.sizeof(Hit) == 88 and C.sizeof(RenderParams) == 32
-assert C.sizeof(AdaptiveParams) == 16 and C.sizeof(AdaptiveStats) == 24
+assert C.sizeof(AdaptiveParams) == 16 and C.sizeof(AdaptiveStats) == 24 and C.sizeof(DenoiseParams) == 16
 
 # numpy views of the two bulk records (same memory layout as the C structs)
 RAY_DTYPE = [("origin", "<f8", 3), ("direction", "<f8", 3), ("time", "<f8"), ("t_min", "<f8"),
@@ -140,6 +145,7 @@ SIGNATURES = {
                                       C.POINTER(AdaptiveStats)]),
     "rtx_adaptive_error": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, _P]),
     "rtx_render_aov": (C.c_int, [_P, _P, C.POINTER(RenderParams), _P, _P, _P]),
+    "rtx_denoise": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, C.c_int32, C.POINTER(DenoiseParams), _P]),
     "rtx_tonemap_rgba8": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P, C.c_int]),
     "rtx_reduce_tonemap_peers": (C.c_int, [_P, _P, C.POINTER(_P), C.c_int32, C.c_int32, C.c_int32, _P]),
     "rtx_reduce_tonemap_slice": (C.c_int, [_P, C.POINTER(_P), C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P]),
@@ -153,6 +159,7 @@ SIGNATURES = {
     "rtx_memset_zero": (C.c_int, [_P, _P, C.c_size_t]),
     "rtx_memcpy_h2d": (C.c_int, [_P, _P, _P, C.c_size_t]),
     "rtx_memcpy_d2h": (C.c_int, [_P, _P, _P, C.c_size_t]),
+    "rtx_memcpy_d2d": (C.c_int, [_P, _P, _P, C.c_size_t]),
     "rtx_ipc_export": (C.c_int, [_P, _P, C.POINTER(C.c_uint8 * 64)]),
     "rtx_ipc_open": (C.c_int, [_P, C.POINTER(C.c_uint8 * 64), C.POINTER(_P)]),
     "rtx_ipc_close": (C.c_int, [_P, _P]),

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <dlfcn.h>
 
+#include <cfloat>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -22,6 +23,7 @@
 #include "flatten.hpp"
 #include "adaptive.cuh"
 #include "aov.cuh"
+#include "denoise.cuh"
 #include "kernels.cuh"
 #include "lbvh.cuh"
 #include "sah_build.cuh"
@@ -123,6 +125,8 @@ struct rtx_ctx {
     int last_build_passes = 0;        // passes the last PLOC build took (RTX_DEBUG_BUILD=1 prints it)
     uint8_t* h_stage = nullptr;       // pinned staging buffer of rtx_scene_create (every H2D copy leaves from here)
     size_t stage_bytes = 0;
+    void* d_denoise = nullptr;        // rtx_denoise's per-pixel scratch (56 B a pixel), grown on demand
+    size_t denoise_bytes = 0;
     // optional per-kernel timing of the wavefront driver (rtx_ctx_set_profiling): CUDA events around every launch
     bool profiling = false;
     std::vector<cudaEvent_t> prof_events;  // grows on demand; [4 * iteration + {0,1,2,3}] = shade begin/end, trace begin/end
@@ -284,6 +288,7 @@ int rtx_ctx_destroy(rtx_ctx* c) {
     cudaFree(c->d_order);
     cudaFree(c->d_next_item);
     cudaFree(c->d_active);
+    cudaFree(c->d_denoise);
     if (c->h_status) cudaFreeHost(c->h_status);
     if (c->h_stage) cudaFreeHost(c->h_stage);
     for (auto& e : c->batch_done)
@@ -1308,6 +1313,71 @@ int rtx_render_aov(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, f
     return RTX_OK;
 }
 
+// ---- denoiser (denoise.cuh) ----------------------------------------------------
+int rtx_denoise(rtx_ctx* c, const float* d_accum, const float* d_half, const float* d_albedo, const float* d_normal,
+                int32_t width, int32_t height, const rtx_denoise_params* params, float* d_out) {
+    if (!c || !d_accum || !d_half || !d_albedo || !d_normal || !d_out) return fail(RTX_ERR_INVALID, "NULL argument");
+    for (const float* b : {d_accum, d_half, d_albedo, d_normal, (const float*)d_out})
+        if ((uintptr_t)b % 16 != 0) return fail(RTX_ERR_INVALID, "every buffer must be 16-byte aligned (float4)");
+    if (width <= 0 || height <= 0) return fail(RTX_ERR_INVALID, "bad image size");
+    if ((int64_t)width * height > 0x7fffffff) return fail(RTX_ERR_INVALID, "image too large");
+    const rtx_denoise_params p = params ? *params : rtx_denoise_params{5, 0.25f, 0.1f, 8.f};
+    if (p.iterations < 1 || p.iterations > 10) return fail(RTX_ERR_INVALID, "iterations must lie in [1, 10]");
+    for (float sg : {p.sigma_normal, p.sigma_albedo, p.sigma_luminance})
+        if (!(sg > 0.f) || !std::isfinite(sg)) return fail(RTX_ERR_INVALID, "every sigma must be > 0 and finite");
+    // the kernels multiply by 1 / sigma^2 in fp32: an infinite factor would turn the centre tap's 0 difference into NaN
+    const double inv_sn2 = 1.0 / ((double)p.sigma_normal * p.sigma_normal), inv_sa2 = 1.0 / ((double)p.sigma_albedo * p.sigma_albedo);
+    if (!(inv_sn2 <= FLT_MAX) || !(inv_sa2 <= FLT_MAX))
+        return fail(RTX_ERR_INVALID, "sigma_normal and sigma_albedo must be at least about 5.4e-20 (1 / sigma^2 finite in fp32)");
+    const size_t n = (size_t)width * height, bytes = n * sizeof(float4);
+    const uintptr_t o0 = (uintptr_t)d_out, o1 = o0 + bytes;
+    for (const float* in : {d_accum, d_half, d_albedo, d_normal}) {
+        const uintptr_t i0 = (uintptr_t)in;
+        if (o0 < i0 + bytes && i0 < o1) return fail(RTX_ERR_INVALID, "d_out overlaps an input buffer");
+    }
+    JOIN(c);
+    CU(cudaSetDevice(c->device));
+    const size_t need = n * (sizeof(float4) + sizeof(float2) + 2 * sizeof(float4));
+    if (c->denoise_bytes < need) {
+        cudaFree(c->d_denoise);  // (waits for the passes of an earlier call that still read it)
+        c->d_denoise = nullptr;
+        c->denoise_bytes = 0;
+        CU(cudaMalloc(&c->d_denoise, need));
+        c->denoise_bytes = need;
+    }
+    float4* feat0 = reinterpret_cast<float4*>(c->d_denoise);
+    float4* ev0 = feat0 + n;
+    float4* ev1 = ev0 + n;
+    float2* feat1 = reinterpret_cast<float2*>(ev1 + n);
+    const dim3 block(rtx::kDenoiseBX, rtx::kDenoiseBY);
+    const int tiles_x = (int)(((int64_t)width + rtx::kDenoiseBX - 1) / rtx::kDenoiseBX);
+    const unsigned grid = (unsigned)(tiles_x * (((int64_t)height + rtx::kDenoiseBY - 1) / rtx::kDenoiseBY));  // < 2^29 tiles for < 2^31 pixels
+    rtx::denoise_prepass_kernel<<<grid, block, 0, c->stream>>>(
+        reinterpret_cast<const float4*>(d_accum), reinterpret_cast<const float4*>(d_half),
+        reinterpret_cast<const float4*>(d_albedo), reinterpret_cast<const float4*>(d_normal), width, height, tiles_x, feat0,
+        feat1, ev0);
+    CU(cudaGetLastError());
+    rtx::DenoisePass a;
+    a.feat0 = feat0;
+    a.feat1 = feat1;
+    a.width = width;
+    a.height = height;
+    a.tiles_x = tiles_x;
+    a.inv_sn2 = (float)inv_sn2;
+    a.inv_sa2 = (float)inv_sa2;
+    a.sigma_l = p.sigma_luminance;
+    for (int i = 0; i < p.iterations; ++i) {
+        a.step = 1 << i;
+        a.ev_in = (i & 1) ? ev1 : ev0;
+        a.ev_out = (i & 1) ? ev0 : ev1;
+        a.out = i == p.iterations - 1 ? reinterpret_cast<float4*>(d_out) : nullptr;
+        rtx::denoise_atrous_kernel<<<grid, block, 0, c->stream>>>(a);
+        CU(cudaGetLastError());
+    }
+    c->launches += 1 + p.iterations;
+    return RTX_OK;
+}
+
 int rtx_tonemap_rgba8(rtx_ctx* c, const float* d_accum, int32_t width, int32_t height, uint8_t* out, int out_on_device) {
     if (!c || !d_accum || !out || width <= 0 || height <= 0) return fail(RTX_ERR_INVALID, "bad argument");
     JOIN(c);
@@ -1537,6 +1607,13 @@ int rtx_memcpy_d2h(rtx_ctx* c, void* dst, const void* src, size_t bytes) {
     CU(cudaSetDevice(c->device));
     CU(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
+    return RTX_OK;
+}
+int rtx_memcpy_d2d(rtx_ctx* c, void* dst, const void* src, size_t bytes) {
+    if (!c || !dst || !src) return fail(RTX_ERR_INVALID, "NULL argument");
+    JOIN(c);
+    CU(cudaSetDevice(c->device));
+    CU(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, c->stream));
     return RTX_OK;
 }
 int rtx_ipc_export(rtx_ctx* c, void* d_ptr, uint8_t handle_out[64]) {

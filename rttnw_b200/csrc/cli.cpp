@@ -3,7 +3,7 @@
 // CWD and reads assets/earth.png relative to it. Optional flags default to the reference values:
 //   --spp N  --width W  --height H  --seed S  --scene-seed S  --gpus N  --out PATH  --chunk N
 //   --checkpoint PATH [--checkpoint-every K]  --resume PATH  --stop-after-chunks N
-//   --adaptive THRESHOLD [--min-spp N] [--step N]  --aov PREFIX [--aov-spp N]
+//   --adaptive THRESHOLD [--min-spp N] [--step N]  --aov PREFIX [--aov-spp N]  --denoise
 // --adaptive (one GPU; rtx_render_adaptive): every 8x4 tile stops sampling once its noise estimate is below THRESHOLD,
 // with --spp as the most samples a pixel gets; --min-spp defaults to spp / 64 (at least 2, even), --step to --min-spp.
 // It prints the samples spent and the tiles that converged. Not with --gpus > 1, --checkpoint or --resume: several GPUs
@@ -13,6 +13,10 @@
 // the linear mean radiance accum.rgb / accum.w of the accumulator image.png is tonemapped from (after the multi-GPU
 // combine), PREFIX.albedo.pfm and PREFIX.normal.pfm, the means over the N samples (normals not renormalised), and
 // PREFIX.depth.pfm (one channel), the mean distance over the samples that hit, 0 where none did.
+// --denoise (rtx_denoise; one GPU): image.png is the denoised frame. The filter needs a half of the samples chosen
+// without looking at them: the uniform path splits its chunk loop at spp / 2 and copies the accumulator there, the
+// --adaptive path has its odd samples. The feature pass renders [0, N) as for --aov (--aov-spp); with --aov the
+// denoised frame is also written as PREFIX.denoised.pfm. Not with --gpus > 1, --checkpoint or --resume.
 // Checkpoint / resume (the reference keeps pixels in RAM until the final save_buffer, main.rs:202-231, so a
 // killed 10k-spp render loses everything): after every K chunks each GPU writes its fp32 accumulator and the
 // next sample index it would render to PATH.<gpu>; --resume reloads them (same scene, size, spp, seed, gpus)
@@ -70,12 +74,14 @@ static void usage(const char* argv0) {  // main.rs:239-249
         }                                                                    \
     } while (0)
 
-// The feature pass and the four PFMs of --aov (see the top of this file). d_accum holds the frame's samples.
-static int write_aov(rtx_ctx* ctx, rtx_scene* sc, const float* d_accum, int width, int height, int aov_spp, int max_depth,
-                     unsigned long long seed, const std::string& prefix) {
+// The feature pass of --aov and --denoise (see the top of this file), the four PFMs of --aov and the denoised frame.
+// d_accum holds the frame's samples. d_half is NULL without --denoise; with it, the denoised frame is tonemapped into
+// `rgba` (host, the pixels of image.png) and, with --aov (prefix not empty), written as PREFIX.denoised.pfm.
+static int write_aov(rtx_ctx* ctx, rtx_scene* sc, const float* d_accum, const float* d_half, int width, int height,
+                     int aov_spp, int max_depth, unsigned long long seed, const std::string& prefix, uint8_t* rgba) {
     const size_t n = (size_t)width * height;
     float *d_albedo = nullptr, *d_normal = nullptr, *d_depth = nullptr;
-    RTX(rtx_malloc(ctx, n * 40, (void**)&d_albedo));
+    RTX(rtx_malloc(ctx, n * 40, (void**)&d_albedo));  // albedo, normal, depth
     d_normal = d_albedo + 4 * n;
     d_depth = d_normal + 4 * n;
     RTX(rtx_memset_zero(ctx, d_albedo, n * 40));
@@ -83,6 +89,23 @@ static int write_aov(rtx_ctx* ctx, rtx_scene* sc, const float* d_accum, int widt
     std::memset(&p, 0, sizeof(p));
     p.width = width; p.height = height; p.spp_begin = 0; p.spp_count = aov_spp; p.max_depth = max_depth; p.seed = seed;
     RTX(rtx_render_aov(ctx, sc, &p, d_albedo, d_normal, d_depth));
+    std::vector<float> denoised;
+    if (d_half) {
+        float* d_out = nullptr;  // its own allocation: rtx_denoise wants float4-aligned buffers, and 40 n bytes is not
+                                 // a multiple of 16 when n is odd
+        RTX(rtx_malloc(ctx, n * 16, (void**)&d_out));
+        RTX(rtx_denoise(ctx, d_accum, d_half, d_albedo, d_normal, width, height, nullptr, d_out));
+        RTX(rtx_tonemap_rgba8(ctx, d_out, width, height, rgba, 0));
+        if (!prefix.empty()) {
+            denoised.resize(n * 4);
+            RTX(rtx_memcpy_d2h(ctx, denoised.data(), d_out, denoised.size() * sizeof(float)));
+        }
+        rtx_free(ctx, d_out);
+    }
+    if (prefix.empty()) {
+        rtx_free(ctx, d_albedo);
+        return 0;
+    }
     std::vector<float> acc(n * 4), aov(n * 10);
     RTX(rtx_memcpy_d2h(ctx, acc.data(), d_accum, acc.size() * sizeof(float)));
     RTX(rtx_memcpy_d2h(ctx, aov.data(), d_albedo, aov.size() * sizeof(float)));
@@ -103,6 +126,11 @@ static int write_aov(rtx_ctx* ctx, rtx_scene* sc, const float* d_accum, int widt
     RTX(rtx_pfm_write((prefix + ".albedo.pfm").c_str(), width, height, 3, albedo.data()));
     RTX(rtx_pfm_write((prefix + ".normal.pfm").c_str(), width, height, 3, normal.data()));
     RTX(rtx_pfm_write((prefix + ".depth.pfm").c_str(), width, height, 1, depth.data()));
+    if (d_half) {
+        for (size_t i = 0; i < n; ++i)
+            for (int c = 0; c < 3; ++c) beauty[3 * i + c] = denoised[4 * i + c];
+        RTX(rtx_pfm_write((prefix + ".denoised.pfm").c_str(), width, height, 3, beauty.data()));
+    }
     return 0;
 }
 
@@ -110,6 +138,7 @@ struct Rank {
     rtx_ctx* ctx = nullptr;
     rtx_scene* scene = nullptr;
     float* accum = nullptr;
+    float* half = nullptr;  // --denoise: the accumulator after samples [0, spp / 2)
     int rc = 0;
 };
 
@@ -178,6 +207,7 @@ int main(int argc, char** argv) {
     int min_spp = -1, step_spp = -1;
     std::string aov_prefix;  // --aov PREFIX: the feature pass and the PFMs
     long long aov_spp = -1;
+    bool denoise = false;
     int worker_rank = -1, shm_fd = -1;  // --worker R --shm-fd FD --device-list L: a worker process of a multi-GPU render (internal)
     std::string device_list = std::getenv("CUDA_VISIBLE_DEVICES") ? std::getenv("CUDA_VISIBLE_DEVICES") : "";
     for (int i = 1; i < argc; ++i) {
@@ -207,6 +237,7 @@ int main(int argc, char** argv) {
         else if (a == "--min-spp") min_spp = std::atoi(next("--min-spp"));
         else if (a == "--step") step_spp = std::atoi(next("--step"));
         else if (a == "--aov") aov_prefix = next("--aov");
+        else if (a == "--denoise") denoise = true;
         else if (a == "--aov-spp") {
             const char* v = next("--aov-spp");
             char* end = nullptr;
@@ -229,7 +260,12 @@ int main(int argc, char** argv) {
                              "--checkpoint or --resume\n");
         return 1;
     }
-    if (aov_spp > 0 && aov_prefix.empty()) { std::fprintf(stderr, "--aov-spp needs --aov PREFIX\n"); return 1; }
+    if (denoise && (gpus > 1 || !ckpt_path.empty() || !resume_path.empty())) {
+        std::fprintf(stderr, "--denoise renders on one GPU without checkpoints: it cannot be combined with --gpus > 1, "
+                             "--checkpoint or --resume\n");
+        return 1;
+    }
+    if (aov_spp > 0 && aov_prefix.empty() && !denoise) { std::fprintf(stderr, "--aov-spp needs --aov PREFIX or --denoise\n"); return 1; }
     if (worker_rank < 0) std::printf("Scene number: %d\n", scene);
     auto t0 = std::chrono::steady_clock::now();
     rtx_scene_defaults def;
@@ -265,8 +301,10 @@ int main(int argc, char** argv) {
         RTX(rtx_render_adaptive(ctx, sc, &p, &ap, accum, aux, &st));
         std::vector<uint8_t> rgba((size_t)width * height * 4);
         RTX(rtx_tonemap_rgba8(ctx, accum, width, height, rgba.data(), 0));
+        if ((denoise || !aov_prefix.empty()) &&
+            write_aov(ctx, sc, accum, denoise ? aux : nullptr, width, height, (int)aov_spp, def.max_depth, seed, aov_prefix, rgba.data()) != 0)
+            return 1;
         RTX(rtx_png_write_rgba8(out.c_str(), width, height, rgba.data()));
-        if (!aov_prefix.empty() && write_aov(ctx, sc, accum, width, height, (int)aov_spp, def.max_depth, seed, aov_prefix) != 0) return 1;
         std::printf("Adaptive sampling: %lld path samples (%.1f per pixel, at most %d), %d rounds, %d of %d tiles converged, %d at %d spp\n",
                     (long long)st.path_samples, (double)st.path_samples / ((double)width * height), spp, st.rounds,
                     st.tiles_converged, st.tiles, st.tiles_at_max, spp);
@@ -297,6 +335,11 @@ int main(int argc, char** argv) {
         size_t bytes = (size_t)width * height * 4 * sizeof(float);
         if (!chk(rtx_malloc(k.ctx, bytes, (void**)&k.accum))) return;
         if (!chk(rtx_memset_zero(k.ctx, k.accum, bytes))) return;
+        if (denoise) {  // (one rank, no checkpoints)
+            if (!chk(rtx_malloc(k.ctx, bytes, (void**)&k.half))) return;
+            if (!chk(rtx_memset_zero(k.ctx, k.half, bytes))) return;
+        }
+        const int split = denoise ? spp / 2 : -1;  // --denoise: no chunk crosses spp / 2, where the accumulator is copied
         int begin = (int)((long long)r * spp / gpus), end = (int)((long long)(r + 1) * spp / gpus);
         CheckpointHeader hdr;
         std::memset(&hdr, 0, sizeof(hdr));
@@ -318,12 +361,15 @@ int main(int argc, char** argv) {
             begin = got.next_sample;
         }
         int chunks_done = 0;
-        for (int b = begin; b < end; b += chunk) {
+        for (int b = begin, count = 0; b < end; b += count) {
+            count = (end - b < chunk) ? end - b : chunk;
+            if (b < split) count = std::min(count, split - b);
             rtx_render_params p;
             std::memset(&p, 0, sizeof(p));
-            p.width = width; p.height = height; p.spp_begin = b; p.spp_count = (end - b < chunk) ? end - b : chunk;
+            p.width = width; p.height = height; p.spp_begin = b; p.spp_count = count;
             p.max_depth = def.max_depth; p.seed = seed;
             if (!chk(rtx_render(k.ctx, k.scene, &p, k.accum, nullptr))) return;
+            if (b + count == split && !chk(rtx_memcpy_d2d(k.ctx, k.half, k.accum, bytes))) return;
             ++chunks_done;
             if (!ckpt_path.empty() && (chunks_done % (ckpt_every < 1 ? 1 : ckpt_every) == 0 || b + chunk >= end)) {
                 host_acc.resize(bytes / sizeof(float));
@@ -480,7 +526,7 @@ int main(int argc, char** argv) {
         RTX(rtx_png_write_rgba8(out.c_str(), width, height, rgba_mp.data()));
         lap("png written");
         if (!aov_prefix.empty()) {
-            if (write_aov(k.ctx, k.scene, k.accum, width, height, (int)aov_spp, def.max_depth, seed, aov_prefix) != 0) {
+            if (write_aov(k.ctx, k.scene, k.accum, nullptr, width, height, (int)aov_spp, def.max_depth, seed, aov_prefix, nullptr) != 0) {
                 for (int r = 1; r < gpus; ++r) if (pids[(size_t)r] > 0) waitpid(pids[(size_t)r], nullptr, 0);
                 return 1;
             }
@@ -505,15 +551,18 @@ int main(int argc, char** argv) {
     RTX(rtx_reduce_tonemap_peers(ranks[0].ctx, ranks[0].accum, peers.empty() ? nullptr : peers.data(), (int)peers.size(), width, height, d_rgba));
     RTX(rtx_memcpy_d2h(ranks[0].ctx, rgba.data(), d_rgba, rgba.size()));
     lap("frame on the host");
-    RTX(rtx_png_write_rgba8(out.c_str(), width, height, rgba.data()));  // image::save_buffer("image.png", ..), main.rs:231
-    lap("png written");
-    if (!aov_prefix.empty()) {
-        if (write_aov(ranks[0].ctx, ranks[0].scene, ranks[0].accum, width, height, (int)aov_spp, def.max_depth, seed, aov_prefix) != 0) return 1;
+    if (denoise || !aov_prefix.empty()) {
+        if (write_aov(ranks[0].ctx, ranks[0].scene, ranks[0].accum, ranks[0].half, width, height, (int)aov_spp, def.max_depth, seed,
+                      aov_prefix, rgba.data()) != 0)
+            return 1;
         lap("feature buffers written");
     }
+    RTX(rtx_png_write_rgba8(out.c_str(), width, height, rgba.data()));  // image::save_buffer("image.png", ..), main.rs:231
+    lap("png written");
     rtx_free(ranks[0].ctx, d_rgba);
     for (auto& k : ranks) {
         rtx_free(k.ctx, k.accum);
+        if (k.half) rtx_free(k.ctx, k.half);
         rtx_scene_destroy(k.scene);
         rtx_ctx_destroy(k.ctx);
     }

@@ -17,6 +17,8 @@ from . import abi
 SCENE_SEED_BASE = 0x5254544E57  # "RTTNW"; builtin scene seed = base + scene number (SURVEY.md §8d)
 _ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DEFAULT_EARTH = os.path.join(_ROOT, "assets", "earth.png")
+# rtx_denoise's defaults (params == NULL); DESIGN.md §4 gives the reason for each value
+DENOISE_DEFAULTS = {"iterations": 5, "sigma_normal": 0.25, "sigma_albedo": 0.1, "sigma_luminance": 8.0}
 
 
 def png_read_rgba8(path: str) -> np.ndarray:
@@ -132,6 +134,25 @@ class Context:
         n = C.c_uint64()
         abi.check(self.lib.rtx_ctx_kernel_launches(self.h, C.byref(n)))
         return n.value
+
+    def denoise(self, accum, half, aov: dict, iterations: int = DENOISE_DEFAULTS["iterations"],
+                sigma_normal: float = DENOISE_DEFAULTS["sigma_normal"],
+                sigma_albedo: float = DENOISE_DEFAULTS["sigma_albedo"],
+                sigma_luminance: float = DENOISE_DEFAULTS["sigma_luminance"]):
+        """The feature-guided à-trous filter (rtx_denoise; the exact filter is in include/rttnw_b200.h): accum (H, W, 4)
+        as render_into fills it, half (H, W, 4) a value-blind subset of its samples (the aux of render_adaptive, or
+        accum cloned after the first half of a uniform render), aov the albedo and normal of DeviceScene.new_aov.
+        Returns a new (H, W, 4) fp32 tensor {r, g, b, 1}: a biased, filtered estimate that tonemap() takes as it is.
+        Asynchronous on the context's stream; the inputs are not modified."""
+        t = self.torch
+        h, w, _ = accum.shape
+        bufs = (accum, half, aov["albedo"], aov["normal"])
+        for b in bufs:
+            assert b.is_contiguous() and b.dtype == t.float32 and tuple(b.shape) == (h, w, 4)
+        out = t.empty((h, w, 4), dtype=t.float32, device=accum.device)
+        p = abi.DenoiseParams(iterations, sigma_normal, sigma_albedo, sigma_luminance)
+        abi.check(self.lib.rtx_denoise(self.h, *(b.data_ptr() for b in bufs), w, h, C.byref(p), out.data_ptr()))
+        return out
 
     def close(self) -> None:
         if self.h:
@@ -292,13 +313,18 @@ def shard_spp(total_spp: int, rank: int, world_size: int) -> tuple:
 def render(scene_number: int, width: Optional[int] = None, height: Optional[int] = None,
            samples: Optional[int] = None, seed: int = 1, device: int = 0, out_path: Optional[str] = None,
            scene_seed: Optional[int] = None, noise_threshold: Optional[float] = None,
-           min_samples: Optional[int] = None, aov_prefix: Optional[str] = None, aov_samples: int = 16) -> np.ndarray:
+           min_samples: Optional[int] = None, aov_prefix: Optional[str] = None, aov_samples: int = 16,
+           denoise: bool = False) -> np.ndarray:
     """`render(width, aspect, samples, scene)` of src/main.rs:58 on one GPU; returns RGBA8 (H, W, 4)
     and, like the reference, writes it as a PNG when `out_path` is given ("image.png" there).
     With `noise_threshold`, adaptive sampling (DeviceScene.render_adaptive): `samples` is the most a pixel gets,
     `min_samples` the least (default samples / 64, at least 2, even), each later round adds min_samples.
     With `aov_prefix`, also writes the linear frame and the feature buffers of samples [0, aov_samples) as PFMs (see
-    write_aov_files): the input of a denoiser such as OIDN or the OptiX denoiser."""
+    write_aov_files): the input of a denoiser such as OIDN or the OptiX denoiser.
+    With `denoise`, the returned RGBA (and the PNG) is the tonemap of Context.denoise over the frame, the feature pass
+    of samples [0, aov_samples) and a value-blind half of the samples: the adaptive render's odd samples, or a copy of
+    the accumulator between the renders of [0, samples / 2) and [samples / 2, samples). With `aov_prefix` as well,
+    the denoised frame is also written as PREFIX.denoised.pfm."""
     d = scene_defaults(scene_number)
     width, height = width or d["width"], height or d["height"]
     samples = samples or d["samples"]
@@ -306,20 +332,32 @@ def render(scene_number: int, width: Optional[int] = None, height: Optional[int]
     desc = BuiltinDesc(scene_number, scene_seed)
     scene = DeviceScene(ctx, desc)
     accum = scene.new_accum(width, height)
+    half = None
     if noise_threshold is None:
-        scene.render_into(accum, 0, samples, seed=seed, max_depth=d["max_depth"])
+        if denoise:
+            scene.render_into(accum, 0, samples // 2, seed=seed, max_depth=d["max_depth"])
+            half = accum.clone()  # (torch's current stream is the context's: ordered between the two renders)
+            scene.render_into(accum, samples // 2, samples - samples // 2, seed=seed, max_depth=d["max_depth"])
+        else:
+            scene.render_into(accum, 0, samples, seed=seed, max_depth=d["max_depth"])
     else:
         if min_samples is None:
             min_samples = max(2, (samples // 64 + 1) // 2 * 2)
-        scene.render_adaptive(accum, scene.new_accum(width, height), noise_threshold, min_samples, min_samples, samples,
+        half = scene.new_accum(width, height)
+        scene.render_adaptive(accum, half, noise_threshold, min_samples, min_samples, samples,
                               seed=seed, max_depth=d["max_depth"])
-    rgba = scene.tonemap(accum)
+    aov = None
+    if aov_prefix or denoise:
+        aov = scene.new_aov(width, height)
+        scene.render_aov(aov, 0, aov_samples, seed=seed, max_depth=d["max_depth"])
+    denoised = ctx.denoise(accum, half, aov) if denoise else None
+    rgba = scene.tonemap(denoised if denoise else accum)
     if out_path:
         png_write_rgba8(out_path, rgba)
     if aov_prefix:
-        aov = scene.new_aov(width, height)
-        scene.render_aov(aov, 0, aov_samples, seed=seed, max_depth=d["max_depth"])
         write_aov_files(aov_prefix, accum, aov)
+        if denoise:
+            pfm_write(aov_prefix + ".denoised.pfm", denoised.cpu().numpy()[..., :3])
     scene.close()
     ctx.close()
     return rgba

@@ -169,6 +169,20 @@ pub struct rtx_adaptive_stats {
     pub tiles_converged: i32,
     pub tiles_at_max: i32,
 }
+/// Settings of the denoiser (`rtx_denoise`; the exact filter is written out in rttnw_b200.h).
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct rtx_denoise_params {
+    pub iterations: i32,
+    pub sigma_normal: f32,
+    pub sigma_albedo: f32,
+    pub sigma_luminance: f32,
+}
+impl Default for rtx_denoise_params {
+    fn default() -> Self {
+        rtx_denoise_params { iterations: 5, sigma_normal: 0.25, sigma_albedo: 0.1, sigma_luminance: 8.0 }
+    }
+}
 /// The scene table of src/main.rs:66-183 and the defaults of :255.
 #[repr(C)]
 #[derive(Clone, Copy)]
@@ -210,6 +224,7 @@ extern "C" {
     pub fn rtx_render_adaptive(ctx: *mut rtx_ctx, scene: *const rtx_scene, params: *const rtx_render_params, adaptive: *const rtx_adaptive_params, d_accum: *mut f32, d_aux: *mut f32, stats: *mut rtx_adaptive_stats) -> c_int;
     pub fn rtx_adaptive_error(ctx: *mut rtx_ctx, d_accum: *const f32, d_aux: *const f32, width: i32, height: i32, d_tile_error: *mut f32) -> c_int;
     pub fn rtx_render_aov(ctx: *mut rtx_ctx, scene: *const rtx_scene, params: *const rtx_render_params, d_albedo: *mut f32, d_normal: *mut f32, d_depth: *mut f32) -> c_int;
+    pub fn rtx_denoise(ctx: *mut rtx_ctx, d_accum: *const f32, d_half: *const f32, d_albedo: *const f32, d_normal: *const f32, width: i32, height: i32, params: *const rtx_denoise_params, d_out: *mut f32) -> c_int;
     pub fn rtx_tonemap_rgba8(ctx: *mut rtx_ctx, d_accum: *const f32, width: i32, height: i32, out: *mut u8, out_on_device: c_int) -> c_int;
     pub fn rtx_reduce_tonemap_peers(ctx: *mut rtx_ctx, d_accum: *mut f32, d_peer_accums: *const *const f32, n_peers: i32, width: i32, height: i32, d_rgba8: *mut u8) -> c_int;
     pub fn rtx_reduce_tonemap_slice(ctx: *mut rtx_ctx, d_accums: *const *const f32, n_ranks: i32, rank: i32, width: i32, height: i32, d_rgba8_root: *mut u8) -> c_int;
@@ -223,6 +238,7 @@ extern "C" {
     pub fn rtx_memset_zero(ctx: *mut rtx_ctx, ptr: *mut c_void, bytes: usize) -> c_int;
     pub fn rtx_memcpy_h2d(ctx: *mut rtx_ctx, dst: *mut c_void, src: *const c_void, bytes: usize) -> c_int;
     pub fn rtx_memcpy_d2h(ctx: *mut rtx_ctx, dst: *mut c_void, src: *const c_void, bytes: usize) -> c_int;
+    pub fn rtx_memcpy_d2d(ctx: *mut rtx_ctx, dst: *mut c_void, src: *const c_void, bytes: usize) -> c_int;
     pub fn rtx_ipc_export(ctx: *mut rtx_ctx, d_ptr: *mut c_void, handle_out: *mut u8) -> c_int;
     pub fn rtx_ipc_open(ctx: *mut rtx_ctx, handle: *const u8, d_ptr_out: *mut *mut c_void) -> c_int;
     pub fn rtx_ipc_close(ctx: *mut rtx_ctx, d_ptr: *mut c_void) -> c_int;

@@ -245,6 +245,56 @@ impl Gpu {
         }
         Ok(out)
     }
+
+    /// A denoised frame (`rtx_denoise`): `samples` uniform samples per pixel with the accumulator copied after the
+    /// first `samples / 2` (the value-blind half the filter's variance estimate needs), the feature pass of samples
+    /// [0, aov_samples), then the filter with `params` (None: the library's defaults). Returns the tonemapped RGBA8
+    /// pixels and the linear frame `{r, g, b, 1}` per pixel, row 0 = top. Unlike `render_desc`, a biased estimate.
+    #[allow(clippy::too_many_arguments)]
+    pub fn denoise(&self, desc: *const ffi::rtx_scene_desc, width: u32, height: u32, samples: usize, aov_samples: usize,
+                   params: Option<ffi::rtx_denoise_params>, seed: u64) -> Result<(Vec<u8>, Vec<f32>), RtxError> {
+        let n = width as usize * height as usize;
+        let mut pixels = vec![0u8; 4 * n];
+        let mut linear = vec![0f32; 4 * n];
+        unsafe {
+            let mut scene = ptr::null_mut();
+            check(ffi::rtx_scene_create(self.ctx, desc, &mut scene))?;
+            let mut d: *mut c_void = ptr::null_mut();
+            let result = (|| {
+                // accum, half, albedo, normal, out: float4 each; depth: float2
+                check(ffi::rtx_malloc(self.ctx, 88 * n, &mut d))?;
+                check(ffi::rtx_memset_zero(self.ctx, d, 88 * n))?;
+                let f = d as *mut f32;
+                let (accum, half, albedo, normal, out, depth) = (f, f.add(4 * n), f.add(8 * n), f.add(12 * n), f.add(16 * n), f.add(20 * n));
+                let mut begin = 0usize;
+                for end in [samples / 2, samples] {
+                    while begin < end {
+                        let count = (end - begin).min(1 << 20);
+                        let params = ffi::rtx_render_params { width: width as i32, height: height as i32, spp_begin: begin as i32,
+                                                              spp_count: count as i32, max_depth: 50, _pad: 0, seed };
+                        check(ffi::rtx_render(self.ctx, scene, &params, accum, ptr::null_mut()))?;
+                        begin += count;
+                    }
+                    if end == samples / 2 {
+                        check(ffi::rtx_memcpy_d2d(self.ctx, half as *mut c_void, accum as *const c_void, 16 * n))?;
+                    }
+                }
+                let feature_params = ffi::rtx_render_params { width: width as i32, height: height as i32, spp_begin: 0,
+                                                              spp_count: aov_samples as i32, max_depth: 50, _pad: 0, seed };
+                check(ffi::rtx_render_aov(self.ctx, scene, &feature_params, albedo, normal, depth))?;
+                let filter = params.as_ref().map_or(ptr::null(), |p| p as *const ffi::rtx_denoise_params);
+                check(ffi::rtx_denoise(self.ctx, accum, half, albedo, normal, width as i32, height as i32, filter, out))?;
+                check(ffi::rtx_tonemap_rgba8(self.ctx, out, width as i32, height as i32, pixels.as_mut_ptr(), 0))?;
+                check(ffi::rtx_memcpy_d2h(self.ctx, linear.as_mut_ptr() as *mut c_void, out as *const c_void, 16 * n))
+            })();
+            if !d.is_null() {
+                ffi::rtx_free(self.ctx, d);
+            }
+            ffi::rtx_scene_destroy(scene);
+            result?;
+        }
+        Ok((pixels, linear))
+    }
 }
 
 /// Sums of `Gpu::render_aov`, host side (see there).
