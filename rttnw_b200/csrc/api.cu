@@ -15,6 +15,7 @@
 #include <deque>
 #include <functional>
 #include <thread>
+#include <type_traits>
 #include <new>
 #include <string>
 #include <vector>
@@ -117,7 +118,6 @@ struct rtx_ctx {
     std::vector<cudaStream_t> aux_streams;
     std::vector<cudaEvent_t> join_events;
     cudaEvent_t fork_event = nullptr;
-    unsigned long long wf_iterations = 0;  // (shade, trace) iterations launched on partition 0
     unsigned long long launches = 0;  // kernels launched by this context (rtx_ctx_kernel_launches)
     int bvh_builder = 0;              // 0: host binned SAH (default), 1: device LBVH, 2: device PLOC, 3: device binned SAH
                                       // (rtx_ctx_set_bvh_builder, RTX_BVH=lbvh|ploc|sah_device)
@@ -680,6 +680,18 @@ int rtx_trace_rays(rtx_ctx* c, const rtx_scene* s, int64_t n, const rtx_ray* ray
     return RTX_OK;
 }
 
+// The device tallies as means per ray (the sums themselves when no ray was traced).
+static void trace_stats(const rtx::Counters& h, unsigned long long rays, rtx_trace_stats* out) {
+    const double dn = rays ? (double)rays : 1.0;
+    out->rays = (double)rays;
+    out->box_tests = (double)h.box_tests / dn;
+    out->node_visits = (double)h.node_visits / dn;
+    out->sphere_tests = (double)h.sphere_tests / dn;
+    out->rect_tests = (double)h.rect_tests / dn;
+    out->instance_enters = (double)h.instance_enters / dn;
+    out->medium_tests = (double)h.medium_tests / dn;
+}
+
 int rtx_trace_rays_stats(rtx_ctx* c, const rtx_scene* s, int64_t n, const rtx_ray* d_rays, rtx_trace_stats* out) {
     if (!c || !s || n <= 0 || !d_rays || !out) return fail(RTX_ERR_INVALID, "bad argument");
     JOIN(c);
@@ -694,22 +706,102 @@ int rtx_trace_rays_stats(rtx_ctx* c, const rtx_scene* s, int64_t n, const rtx_ra
     rtx::Counters h;
     CU(cudaMemcpyAsync(&h, c->d_counters, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
-    double dn = (double)n;
-    out->rays = dn;
-    out->box_tests = (double)h.box_tests / dn;
-    out->node_visits = (double)h.node_visits / dn;
-    out->sphere_tests = (double)h.sphere_tests / dn;
-    out->rect_tests = (double)h.rect_tests / dn;
-    out->instance_enters = (double)h.instance_enters / dn;
-    out->medium_tests = (double)h.medium_tests / dn;
+    trace_stats(h, (unsigned long long)n, out);
     return RTX_OK;
 }
 
-// ---- render: wavefront driver ---------------------------------------------------
-static size_t order_bins_padded(int groups) {
-    const size_t unit = 4 * (size_t)rtx::kShadeBlock;
-    return ((size_t)8 * (size_t)groups + 1 + unit - 1) / unit * unit;
+}  // extern "C"
+
+// ---- render: frame setup shared by the render entry points ------------------------
+// The refusals the render entry points share, in this order: a bad size, first sample or depth, or the entry point's own
+// condition `bad`, worded `bad_text`; 2^31 pixels or more; unless count_of is null, more than 2^24 samples per pixel
+// into the fp32 sample count of the buffer it names.
+static int check_frame(const rtx_render_params* p, int min_depth, bool bad, const char* bad_text, const char* count_of) {
+    if (p->width <= 0 || p->height <= 0 || p->spp_begin < 0 || p->max_depth < min_depth || bad) return fail(RTX_ERR_INVALID, bad_text);
+    if ((int64_t)p->width * p->height > 0x7fffffff) return fail(RTX_ERR_INVALID, "image too large");
+    if (count_of && p->spp_count > (1 << 24))
+        return fail(RTX_ERR_INVALID, std::string("more than 2^24 samples per pixel in one call (the fp32 sample count of the ") + count_of + ")");
+    return RTX_OK;
 }
+
+struct Tiles {  // a frame's 8x4-pixel tiles; inv_per_block_row = 1 / (x * kBlockH), see tile_of_order
+    int32_t x, y;
+    float inv_per_block_row;
+};
+static Tiles frame_tiles(int32_t width, int32_t height) {
+    const int32_t x = (width + rtx::kTileW - 1) / rtx::kTileW;
+    return {x, (height + rtx::kTileH - 1) / rtx::kTileH, 1.0f / (float)(x * rtx::kBlockH)};
+}
+
+// Fills the frame fields of WfArgs, RenderArgs and AovArgs and returns the frame's tiles. The feature pass stops at the
+// first vertex and numbers its tiles in raster order, so AovArgs has no max_depth, tiles_y or inv_per_block_row.
+template <class Args>
+static Tiles set_frame(Args& a, const rtx_scene* s, const rtx_render_params* p) {
+    const Tiles t = frame_tiles(p->width, p->height);
+    a.sc = s->view;
+    a.cam = s->camera;
+    a.width = p->width; a.height = p->height;
+    a.spp_begin = p->spp_begin; a.spp_count = p->spp_count;
+    a.k0 = (uint32_t)p->seed; a.k1 = (uint32_t)(p->seed >> 32);
+    a.tiles_x = t.x;
+    if constexpr (!std::is_same<Args, rtx::AovArgs>::value) {
+        a.max_depth = p->max_depth;
+        a.tiles_y = t.y;
+        a.inv_per_block_row = t.inv_per_block_row;
+    }
+    return t;
+}
+
+// ---- render: wavefront driver ---------------------------------------------------
+// The path pool's SoA arrays, carved out of one allocation of `slots` slots (kPoolBytesPerSlot each, 8-byte arrays
+// first), and the pool of a partition, the slots from `begin` on.
+template <class F>
+static void for_each_array(rtx::PathPool& pool, F f) {
+    f(pool.ox); f(pool.oy); f(pool.oz); f(pool.dx); f(pool.dy); f(pool.dz); f(pool.time); f(pool.best_t);
+    f(pool.best_rec); f(pool.best_chain); f(pool.bounce); f(pool.pixel); f(pool.sample);
+    f(pool.thr_r); f(pool.thr_g); f(pool.thr_b);
+}
+static rtx::PathPool pool_carve(void* base, int64_t slots) {
+    rtx::PathPool pool;
+    uint8_t* next = (uint8_t*)base;
+    for_each_array(pool, [&](auto*& arr) {
+        arr = reinterpret_cast<std::remove_reference_t<decltype(arr)>>(next);
+        next += (size_t)slots * sizeof(*arr);
+    });
+    return pool;
+}
+static rtx::PathPool pool_part(rtx::PathPool pool, int64_t begin) {
+    for_each_array(pool, [&](auto*& arr) { arr += begin; });
+    return pool;
+}
+
+// Slots of the pool for a job of `total` path samples: the configured maximum, but a small job (few pool refills) is
+// all ramp-up and drain with a pool that large: keep at least ~24 refills, down to 256 Ki slots. Whole CTAs.
+static int64_t pool_slots_for(const rtx_ctx* c, unsigned long long total) {
+    int64_t slots = c->pool_slots_wanted;
+    if ((unsigned long long)slots > total / 24) slots = (int64_t)(total / 24);
+    if (slots < (256 << 10)) slots = 256 << 10;
+    if (slots > c->pool_slots_wanted) slots = c->pool_slots_wanted;
+    if ((unsigned long long)slots > total) slots = (int64_t)total;
+    return (slots + rtx::kWfBlock - 1) / rtx::kWfBlock * rtx::kWfBlock;
+}
+
+// The scratch of ray ordering (order.cuh) for `parts` partitions of `slots` slots: per partition, hist [bins],
+// offsets [bins + 1] and done in a stride of part_words; behind them, 256-byte aligned at slots_at, key_rank (8 B)
+// and order (4 B) of every slot. bins (n_bins_padded) is 8 * groups + 1, rounded up to whole uint4 per shade thread.
+struct OrderLayout {
+    size_t bins, part_words, slots_at, bytes;
+};
+static OrderLayout order_layout(int groups, int parts, int64_t slots) {
+    const size_t unit = 4 * (size_t)rtx::kShadeBlock;
+    OrderLayout l;
+    l.bins = ((size_t)8 * (size_t)groups + 1 + unit - 1) / unit * unit;
+    l.part_words = 2 * l.bins + 64;
+    l.slots_at = ((size_t)parts * l.part_words * 4 + 255) & ~(size_t)255;
+    l.bytes = l.slots_at + (size_t)slots * 12;
+    return l;
+}
+
 static int wf_prepare(rtx_ctx* c, int64_t slots) {
     if (slots > c->pool_slots) {
         if (c->d_pool) { CU(cudaStreamSynchronize(c->stream)); CU(cudaFree(c->d_pool)); c->d_pool = nullptr; c->pool_slots = 0; }
@@ -717,9 +809,7 @@ static int wf_prepare(rtx_ctx* c, int64_t slots) {
         c->pool_slots = (int)slots;
     }
     if (c->order_form != 0) {
-        // per partition: hist [bins], offsets [bins + 1], done, then per slot key_rank (8 B) and order (4 B)
-        const size_t bins = order_bins_padded(c->order_groups);
-        const size_t need = (size_t)c->wf_streams * ((2 * bins + 64) * 4) + (size_t)slots * 12 + 4096;
+        const size_t need = order_layout(c->order_groups, c->wf_streams, slots).bytes;
         if (need > c->order_bytes) {
             if (c->d_order) { CU(cudaStreamSynchronize(c->stream)); CU(cudaFree(c->d_order)); c->d_order = nullptr; c->order_bytes = 0; }
             CU(cudaMalloc(&c->d_order, need));
@@ -744,206 +834,217 @@ static int wf_prepare(rtx_ctx* c, int64_t slots) {
     return RTX_OK;
 }
 
+// The signatures of the kernels a render call chooses among: every shade kernel; the trace kernels that take the slots
+// in slot order (form 1, wide or not, and 1c); the ordered trace kernel; forms 2 and 3.
+using ShadeKernel = void (*)(rtx::WfArgs, float4*, unsigned int*, rtx::Counters*);
+using SlotTraceKernel = void (*)(rtx::SceneView, rtx::PathPool, int, unsigned long long*, rtx::Counters*);
+using OrderedTraceKernel = void (*)(rtx::SceneView, rtx::PathPool, rtx::OrderArgs, unsigned long long*, rtx::Counters*);
+using Trace2Kernel = void (*)(rtx::SceneView, rtx::PathPool, int, rtx::TraceCfg, unsigned long long*, rtx::Counters*);
+using Trace3Kernel = void (*)(rtx::SceneView, rtx::PathPool, int, rtx::Trace3Cfg, unsigned long long*, rtx::Counters*);
+
+// The instantiations of the shared-memory forms 2 and 3 for a CTA size wf_plan has snapped, counted or not, with the
+// whole world BVH staged or not.
+template <bool kCount, bool kAll>
+static Trace2Kernel trace2_of(int threads) {
+    switch (threads) {
+        case 1024: return rtx::wf_trace2_kernel<kCount, 1024, kAll>;
+        case 896: return rtx::wf_trace2_kernel<kCount, 896, kAll>;
+        case 640: return rtx::wf_trace2_kernel<kCount, 640, kAll>;
+        case 512: return rtx::wf_trace2_kernel<kCount, 512, kAll>;
+        default: return rtx::wf_trace2_kernel<kCount, 448, kAll>;
+    }
+}
+static Trace2Kernel trace2_kernel(bool counted, int threads, bool all) {
+    if (counted) return all ? trace2_of<true, true>(threads) : trace2_of<true, false>(threads);
+    return all ? trace2_of<false, true>(threads) : trace2_of<false, false>(threads);
+}
+template <bool kCount, bool kAll>
+static Trace3Kernel trace3_of(int threads) {
+    switch (threads) {
+        case 896: return rtx::wf_trace3_kernel<kCount, 896, kAll>;
+        case 768: return rtx::wf_trace3_kernel<kCount, 768, kAll>;
+        case 640: return rtx::wf_trace3_kernel<kCount, 640, kAll>;
+        default: return rtx::wf_trace3_kernel<kCount, 512, kAll>;
+    }
+}
+static Trace3Kernel trace3_kernel(bool counted, int threads, bool all) {
+    if (counted) return all ? trace3_of<true, true>(threads) : trace3_of<true, false>(threads);
+    return all ? trace3_of<false, true>(threads) : trace3_of<false, false>(threads);
+}
+
+// A partition of the pool, driven on its own stream.
+struct WfPart {
+    rtx::WfArgs a;
+    cudaStream_t stream;
+    unsigned sgrid, tgrid;  // CTAs of its shade and trace launches
+    bool done;
+};
+
+// The kernels of one render call, chosen once before its first iteration. The trace step is exactly one of the four
+// trace kernels. The shared-memory forms 2 and 3 (threads > 0) run CTAs of `threads` threads with `smem` bytes of
+// dynamic shared memory, one per SM at most; the others run one thread per slot in kTraceBlock-thread CTAs.
+struct WfPlan {
+    ShadeKernel shade = nullptr;
+    bool order_pass = false;            // RTX_ORDER=1: wf_order_kernel sorts the slots between shade and trace
+    rtx::Counters* counters = nullptr;  // the tallies of a counted render (rtx_render_counted)
+    SlotTraceKernel trace_slots = nullptr;
+    OrderedTraceKernel trace_ordered = nullptr;
+    Trace2Kernel trace2 = nullptr;
+    Trace3Kernel trace3 = nullptr;
+    rtx::TraceCfg cfg2{};
+    rtx::Trace3Cfg cfg3{};
+    int threads = 0;
+    size_t smem = 0;
+
+    unsigned long long launches() const { return order_pass ? 3 : 2; }  // per iteration
+    unsigned trace_grid(int64_t slots, int sm_count) const {
+        if (threads == 0) return (unsigned)(slots / rtx::kTraceBlock);
+        // one CTA per SM (fewer when the partition is small): each stages the BVH once and walks its share of the slots
+        return (unsigned)std::max<int64_t>(1, std::min<int64_t>(sm_count, (slots + threads - 1) / threads));
+    }
+    void launch_shade(const WfPart& pt, float4* acc, unsigned int* active) const {
+        shade<<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, counters);
+        if (order_pass) rtx::wf_order_kernel<<<(unsigned)((pt.a.n_slots + 255) / 256), 256, 0, pt.stream>>>(pt.a.order, pt.a.n_slots);
+    }
+    void launch_trace(const WfPart& pt, unsigned long long* rays) const {
+        const rtx::WfArgs& a = pt.a;
+        if (trace_ordered) trace_ordered<<<pt.tgrid, rtx::kTraceBlock, 0, pt.stream>>>(a.sc, a.pool, a.order, rays, counters);
+        else if (trace2) trace2<<<pt.tgrid, threads, smem, pt.stream>>>(a.sc, a.pool, a.n_slots, cfg2, rays, counters);
+        else if (trace3) trace3<<<pt.tgrid, threads, smem, pt.stream>>>(a.sc, a.pool, a.n_slots, cfg3, rays, counters);
+        else trace_slots<<<pt.tgrid, rtx::kTraceBlock, 0, pt.stream>>>(a.sc, a.pool, a.n_slots, rays, counters);
+    }
+};
+
+// Forms 2 and 3 stage as much of the world BVH in shared memory as fits next to `fixed` bytes of their own (stacks,
+// ray state): the nodes staged, 0 when not even one fits.
+static int stage_cap(const rtx_ctx* c, const rtx_scene* s, size_t fixed) {
+    const size_t room = (size_t)c->smem_optin > fixed ? (size_t)c->smem_optin - fixed : 0;
+    return (int)std::min<size_t>(room / rtx::kNodeStride, (size_t)s->world_node_count);
+}
+
+static WfPlan wf_plan(const rtx_ctx* c, const rtx_scene* s, bool counted, bool adaptive) {
+    WfPlan pl;
+    pl.counters = counted ? c->d_counters : nullptr;
+    const bool wide = c->wf_wide != 0 && s->view.wide_root >= 0;
+    pl.order_pass = c->order_form != 0 && c->shade_form >= 2 && c->trace_form == 1 && !wide;
+    // the shade kernel stages the Perlin table in shared memory when the scene has exactly one (not when counting)
+    const bool perlin = c->perlin_smem && s->n_perlins == 1;
+    if (adaptive)  // (rtx_render_adaptive refuses the first shade form and ray ordering)
+        pl.shade = perlin ? rtx::wf_shade2_kernel<false, true, false, true> : rtx::wf_shade2_kernel<false, false, false, true>;
+    else if (c->shade_form < 2)
+        pl.shade = counted ? rtx::wf_shade_kernel<true> : rtx::wf_shade_kernel<false>;
+    else if (counted)
+        pl.shade = pl.order_pass ? rtx::wf_shade2_kernel<true, false, true> : rtx::wf_shade2_kernel<true>;
+    else if (pl.order_pass)
+        pl.shade = perlin ? rtx::wf_shade2_kernel<false, true, true> : rtx::wf_shade2_kernel<false, false, true>;
+    else
+        pl.shade = perlin ? rtx::wf_shade2_kernel<false, true> : rtx::wf_shade2_kernel<false>;
+    // forms 2-4 keep their stacks in shared memory: deeper world BVHs, and the wide one, fall back to form 1
+    const bool short_stack = !wide && s->world_depth <= rtx::kShortStack;
+    const bool staged = c->trace_form >= 2 && short_stack && s->world_node_count > 0;
+    if (pl.order_pass) {
+        pl.trace_ordered = counted ? rtx::wf_trace_ordered_kernel<true> : rtx::wf_trace_ordered_kernel<false>;
+        return pl;
+    }
+    if (c->trace_form == 4 && short_stack) {  // "1c": form 1's launch shape, shared-memory stack, 32-byte node loads
+        pl.trace_slots = counted ? rtx::wf_trace1c_kernel<true> : rtx::wf_trace1c_kernel<false>;
+        return pl;
+    }
+    // form 3 (trace3.cuh: rays regrouped by the kind of work they need next) where it fits, else form 2 (trace2.cuh:
+    // persistent warps with voted refill) for any form >= 2 where it fits, else form 1
+    const int t3 = c->trace_threads >= 896 ? 896 : (c->trace_threads >= 768 ? 768 : (c->trace_threads >= 640 ? 640 : 512));
+    const int t2 = c->trace_threads >= 1024 ? 1024 : c->trace_threads >= 896 ? 896 : (c->trace_threads >= 640 ? 640 : (c->trace_threads >= 512 ? 512 : 448));
+    const size_t fixed3 = rtx::trace3_smem_bytes(t3, 0), fixed2 = (size_t)(1 + rtx::kShortStack) * (size_t)t2 * 4 + 16;
+    const int cap3 = staged && c->trace_form == 3 ? stage_cap(c, s, fixed3) : 0;
+    const int cap2 = staged ? stage_cap(c, s, fixed2) : 0;
+    if (cap3 >= 1) {
+        pl.trace3 = trace3_kernel(counted, t3, cap3 == s->world_node_count);
+        pl.cfg3 = {s->world_first_node, cap3, cap3, c->t_burst};
+        pl.threads = t3;
+        pl.smem = rtx::trace3_smem_bytes(t3, cap3);
+    } else if (cap2 >= 1) {
+        pl.trace2 = trace2_kernel(counted, t2, cap2 == s->world_node_count);
+        pl.cfg2 = {s->world_first_node, cap2, cap2, c->t_leaf, c->t_refill, c->t_burst};
+        pl.threads = t2;
+        pl.smem = (size_t)cap2 * rtx::kNodeStride + fixed2;
+    } else {
+        pl.trace_slots = wide ? (counted ? rtx::wf_trace_kernel<true, true> : rtx::wf_trace_kernel<false, true>)
+                              : (counted ? rtx::wf_trace_kernel<true> : rtx::wf_trace_kernel<false>);
+    }
+    return pl;
+}
+
+// Adaptive sampling's part of a render (rtx_render_adaptive): only the n_tiles tiles of the list of dispenser order
+// indices are rendered, and the samples with an odd global index also go to aux.
+struct AdaptivePass {
+    rtx::AdaptiveArgs args;  // tile_list, aux
+    int64_t n_tiles;
+};
+
 // Submits iterations (shade, trace) in batches; after each batch the number of rays the batch's
 // last shade kernel produced and the dispenser position are copied to pinned memory. The host looks
 // at batch k-1 while batch k is already queued, so the GPU never waits for the host; it stops
 // submitting once a batch ended with no ray in flight and no sample left (the batch queued behind it
 // then runs over empty slots). The call returns when everything has been submitted AND that check
 // has come back, i.e. it may block the calling thread for most of the render.
-// With tile_list (adaptive sampling), only the n_list tiles of that list of dispenser order indices are rendered, and
-// the samples with an odd global index also go to d_aux.
 static int render_wavefront(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, float* d_accum,
-                            unsigned long long* d_ray_count, bool counted, const uint32_t* tile_list = nullptr,
-                            int64_t n_list = 0, float* d_aux = nullptr) {
-    const bool adaptive = tile_list != nullptr;
-    const int64_t n_tiles = adaptive ? n_list : (int64_t)((p->width + rtx::kTileW - 1) / rtx::kTileW) * ((p->height + rtx::kTileH - 1) / rtx::kTileH);
+                            unsigned long long* d_ray_count, bool counted, const AdaptivePass* adaptive = nullptr) {
+    const WfPlan pl = wf_plan(c, s, counted, adaptive != nullptr);
+    rtx::WfArgs a;
+    const Tiles tiles = set_frame(a, s, p);
+    const int64_t n_tiles = adaptive ? adaptive->n_tiles : (int64_t)tiles.x * tiles.y;
     const unsigned long long total = (unsigned long long)n_tiles * 32ull * (unsigned long long)p->spp_count;
-    // pool size: the configured maximum, but a small job (few pool refills) is all ramp-up and drain with a pool
-    // that large: keep at least ~24 refills, down to 256 Ki slots
-    int64_t slots = c->pool_slots_wanted;
-    if ((unsigned long long)slots > total / 24) slots = (int64_t)(total / 24);
-    if (slots < (256 << 10)) slots = 256 << 10;
-    if (slots > c->pool_slots_wanted) slots = c->pool_slots_wanted;
-    if ((unsigned long long)slots > total) slots = (int64_t)total;
-    slots = (slots + rtx::kWfBlock - 1) / rtx::kWfBlock * rtx::kWfBlock;  // whole CTAs
+    const int64_t slots = pool_slots_for(c, total);
     int rc = wf_prepare(c, slots);
     if (rc != RTX_OK) return rc;
-    rtx::WfArgs a;
-    a.sc = s->view;
-    a.cam = s->camera;
-    a.width = p->width; a.height = p->height;
-    a.spp_begin = p->spp_begin; a.spp_count = p->spp_count; a.max_depth = p->max_depth;
-    a.k0 = (uint32_t)p->seed; a.k1 = (uint32_t)(p->seed >> 32);
-    a.tiles_x = (p->width + rtx::kTileW - 1) / rtx::kTileW;
-    a.tiles_y = (p->height + rtx::kTileH - 1) / rtx::kTileH;
-    a.inv_per_block_row = 1.0f / (float)(a.tiles_x * rtx::kBlockH);
+    if (pl.trace2) CU(cudaFuncSetAttribute(pl.trace2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
+    if (pl.trace3) CU(cudaFuncSetAttribute(pl.trace3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
+    a.pool = pool_carve(c->d_pool, slots);
     a.n_slots = (int32_t)slots;
     a.total_items = total;
     a.next_item = c->d_next_item;
-    a.adaptive.tile_list = tile_list;  // (ray ordering, the other user of this space, fills it per partition below)
-    a.adaptive.aux = reinterpret_cast<float4*>(d_aux);
-    {   // carve the SoA arrays out of the pool allocation (8-byte arrays first)
-        uint8_t* base = (uint8_t*)c->d_pool;
-        size_t n = (size_t)slots;
-        double** d8[8] = {&a.pool.ox, &a.pool.oy, &a.pool.oz, &a.pool.dx, &a.pool.dy, &a.pool.dz, &a.pool.time, &a.pool.best_t};
-        for (auto pp : d8) { *pp = (double*)base; base += n * 8; }
-        a.pool.best_rec = (int32_t*)base; base += n * 4;
-        a.pool.best_chain = (int32_t*)base; base += n * 4;
-        a.pool.bounce = (int32_t*)base; base += n * 4;
-        a.pool.pixel = (uint32_t*)base; base += n * 4;
-        a.pool.sample = (uint32_t*)base; base += n * 4;
-        float** f4[3] = {&a.pool.thr_r, &a.pool.thr_g, &a.pool.thr_b};
-        for (auto pp : f4) { *pp = (float*)base; base += n * 4; }
-    }
+    a.adaptive = adaptive ? adaptive->args : rtx::AdaptiveArgs{};  // (ray ordering, the other user of this space, fills it per partition below)
     CU(cudaMemsetAsync(a.pool.bounce, 0xFF, (size_t)slots * 4, c->stream));  // every slot empty (-1)
     CU(cudaMemsetAsync(c->d_next_item, 0, sizeof(unsigned long long), c->stream));
     float4* acc = reinterpret_cast<float4*>(d_accum);
     const int batch = c->wf_batch;
-    const bool wide = c->wf_wide != 0 && s->view.wide_root >= 0;
     // P partitions of the pool, each driven on its own stream: the shade kernel of one partition (latency bound,
     // streams the pool) can share the SMs with the trace kernel of another (issue bound). Partition 0 runs on the
     // ctx stream; the others fork from it here and join it at the end.
     const int P = (slots >= (int64_t)c->wf_streams * 4 * rtx::kWfBlock) ? c->wf_streams : 1;
-    const bool ordered = c->order_form != 0 && c->shade_form >= 2 && c->trace_form == 1 && !wide;
-    if (ordered) CU(cudaMemsetAsync(c->d_order, 0, (size_t)P * (2 * order_bins_padded(c->order_groups) + 64) * 4, c->stream));
-    struct Part {
-        rtx::WfArgs a;
-        cudaStream_t stream;
-        unsigned grid, sgrid;
-        bool done;
-    };
-    std::vector<Part> parts((size_t)P);
-    {
-        int64_t per = slots / P / rtx::kWfBlock * rtx::kWfBlock;
-        for (int q = 0; q < P; ++q) {
-            Part& pt = parts[(size_t)q];
-            int64_t begin = (int64_t)q * per, count = q == P - 1 ? slots - begin : per;
-            pt.a = a;
-            pt.a.n_slots = (int32_t)count;
-            double** d8[8] = {&pt.a.pool.ox, &pt.a.pool.oy, &pt.a.pool.oz, &pt.a.pool.dx, &pt.a.pool.dy, &pt.a.pool.dz, &pt.a.pool.time, &pt.a.pool.best_t};
-            for (auto pp : d8) *pp += begin;
-            pt.a.pool.best_rec += begin; pt.a.pool.best_chain += begin; pt.a.pool.bounce += begin;
-            pt.a.pool.pixel += begin; pt.a.pool.sample += begin;
-            float** f4[3] = {&pt.a.pool.thr_r, &pt.a.pool.thr_g, &pt.a.pool.thr_b};
-            for (auto pp : f4) *pp += begin;
-            if (ordered) {
-                const size_t bins = order_bins_padded(c->order_groups);
-                uint32_t* w = (uint32_t*)c->d_order + (size_t)q * (2 * bins + 64);
-                rtx::OrderArgs& o = pt.a.order;
-                o.hist = w;
-                o.offsets = w + bins;
-                o.done = w + 2 * bins + 1;
-                uint8_t* per_slot = (uint8_t*)c->d_order + (((size_t)P * (2 * bins + 64) * 4 + 255) & ~(size_t)255);
-                o.key_rank = (uint2*)per_slot + begin;
-                o.order = (uint32_t*)(per_slot + (size_t)slots * 8) + begin;
-                o.n_bins_padded = (int32_t)bins;
-                o.groups = c->order_groups;
-                o.shift = 0;
-                while (((s->n_records - 1) >> o.shift) >= o.groups) ++o.shift;
-            }
-            pt.grid = (unsigned)(count / rtx::kTraceBlock);
-            pt.sgrid = (unsigned)(count / rtx::kShadeBlock);
-            pt.done = false;
-            pt.stream = q == 0 ? c->stream : c->aux_streams[(size_t)q - 1];
+    const OrderLayout ol = order_layout(c->order_groups, P, slots);
+    if (pl.order_pass) CU(cudaMemsetAsync(c->d_order, 0, (size_t)P * ol.part_words * 4, c->stream));
+    std::vector<WfPart> parts((size_t)P);
+    const int64_t per = slots / P / rtx::kWfBlock * rtx::kWfBlock;
+    for (int q = 0; q < P; ++q) {
+        WfPart& pt = parts[(size_t)q];
+        const int64_t begin = (int64_t)q * per, count = q == P - 1 ? slots - begin : per;
+        pt.a = a;
+        pt.a.pool = pool_part(a.pool, begin);
+        pt.a.n_slots = (int32_t)count;
+        if (pl.order_pass) {
+            uint32_t* w = (uint32_t*)c->d_order + (size_t)q * ol.part_words;
+            uint8_t* per_slot = (uint8_t*)c->d_order + ol.slots_at;
+            rtx::OrderArgs& o = pt.a.order;
+            o.hist = w;
+            o.offsets = w + ol.bins;
+            o.done = w + 2 * ol.bins + 1;
+            o.key_rank = (uint2*)per_slot + begin;
+            o.order = (uint32_t*)(per_slot + (size_t)slots * 8) + begin;
+            o.n_bins_padded = (int32_t)ol.bins;
+            o.groups = c->order_groups;
+            o.shift = 0;
+            while (((s->n_records - 1) >> o.shift) >= o.groups) ++o.shift;
         }
-        if (P > 1) {
-            CU(cudaEventRecord(c->fork_event, c->stream));
-            for (int q = 1; q < P; ++q) CU(cudaStreamWaitEvent(parts[(size_t)q].stream, c->fork_event, 0));
-        }
+        pt.sgrid = (unsigned)(count / rtx::kShadeBlock);
+        pt.tgrid = pl.trace_grid(count, c->sm_count);
+        pt.done = false;
+        pt.stream = q == 0 ? c->stream : c->aux_streams[(size_t)q - 1];
     }
-    // ---- which trace kernel: the shared-memory form when the world BVH is shallow enough for its shared stack ----
-    rtx::TraceCfg tcfg{};
-    int t2_threads = 0;  // 0: first form
-    size_t t2_smem = 0;
-    unsigned t2_grid_cap = (unsigned)c->sm_count;
-    if (c->trace_form >= 2 && !wide && s->world_node_count > 0 && s->world_depth <= rtx::kShortStack) {
-        t2_threads = c->trace_threads >= 1024 ? 1024 : c->trace_threads >= 896 ? 896 : (c->trace_threads >= 640 ? 640 : (c->trace_threads >= 512 ? 512 : 448));
-        const size_t stack_bytes = (size_t)(1 + rtx::kShortStack) * (size_t)t2_threads * 4 + 16;
-        const size_t room = (size_t)c->smem_optin > stack_bytes ? (size_t)c->smem_optin - stack_bytes : 0;
-        int cap = (int)std::min<size_t>(room / rtx::kNodeStride, (size_t)s->world_node_count);
-        if (cap < 1) {
-            t2_threads = 0;
-        } else {
-            tcfg.stage_first = s->world_first_node;
-            tcfg.n_stage = cap;
-            tcfg.cap = cap;
-            tcfg.t_leaf = c->t_leaf; tcfg.t_refill = c->t_refill; tcfg.burst = c->t_burst;
-            t2_smem = (size_t)cap * rtx::kNodeStride + stack_bytes;
-        }
+    if (P > 1) {
+        CU(cudaEventRecord(c->fork_event, c->stream));
+        for (int q = 1; q < P; ++q) CU(cudaStreamWaitEvent(parts[(size_t)q].stream, c->fork_event, 0));
     }
-    // sorted form (RTX_TRACE=3): rays regrouped by the kind of work they need next, through shared memory (trace3.cuh)
-    rtx::Trace3Cfg t3cfg{};
-    int t3_threads = 0;
-    size_t t3_smem = 0;
-    if (c->trace_form == 3 && !wide && s->world_node_count > 0 && s->world_depth <= rtx::kShortStack) {
-        t3_threads = c->trace_threads >= 896 ? 896 : (c->trace_threads >= 768 ? 768 : (c->trace_threads >= 640 ? 640 : 512));
-        const size_t fixed = rtx::trace3_smem_bytes(t3_threads, 0);
-        const size_t room = (size_t)c->smem_optin > fixed ? (size_t)c->smem_optin - fixed : 0;
-        const int cap = (int)std::min<size_t>(room / rtx::kNodeStride, (size_t)s->world_node_count);
-        if (cap < 1) {
-            t3_threads = 0;
-        } else {
-            t3cfg.stage_first = s->world_first_node;
-            t3cfg.n_stage = cap;
-            t3cfg.cap = cap;
-            t3cfg.burst = c->t_burst;
-            t3_smem = rtx::trace3_smem_bytes(t3_threads, cap);
-            t2_threads = 0;
-        }
-    }
-    // form "1c" (RTX_TRACE=4): the first form's launch shape with the stack in shared memory and 32-byte node loads
-    const bool t1c = c->trace_form == 4 && !wide && s->world_depth <= rtx::kShortStack;
-    if (t1c) t2_threads = 0;
-    const bool t3_all = t3_threads != 0 && t3cfg.n_stage == s->world_node_count;
-    auto launch_trace3 = [&](const Part& pt) -> cudaError_t {
-        unsigned grid = std::min<unsigned>((unsigned)c->sm_count, (unsigned)((pt.a.n_slots + t3_threads - 1) / t3_threads));
-        if (grid < 1) grid = 1;
-#define RTX_T3_LAUNCH(CNT, THR, ALL)                                                                                               \
-    do {                                                                                                                           \
-        auto k = rtx::wf_trace3_kernel<CNT, THR, ALL>;                                                                             \
-        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t3_smem);                         \
-        if (e != cudaSuccess) return e;                                                                                            \
-        k<<<grid, THR, t3_smem, pt.stream>>>(pt.a.sc, pt.a.pool, pt.a.n_slots, t3cfg, d_ray_count, CNT ? c->d_counters : nullptr); \
-    } while (0)
-#define RTX_T3_THREADS(CNT, ALL)                                  \
-    do {                                                          \
-        if (t3_threads == 896) RTX_T3_LAUNCH(CNT, 896, ALL);      \
-        else if (t3_threads == 768) RTX_T3_LAUNCH(CNT, 768, ALL); \
-        else if (t3_threads == 640) RTX_T3_LAUNCH(CNT, 640, ALL); \
-        else RTX_T3_LAUNCH(CNT, 512, ALL);                        \
-    } while (0)
-        if (counted) { if (t3_all) RTX_T3_THREADS(true, true); else RTX_T3_THREADS(true, false); }
-        else { if (t3_all) RTX_T3_THREADS(false, true); else RTX_T3_THREADS(false, false); }
-#undef RTX_T3_THREADS
-#undef RTX_T3_LAUNCH
-        return cudaSuccess;
-    };
-    const bool t2_all = t2_threads != 0 && tcfg.n_stage == s->world_node_count;
-    auto launch_trace2 = [&](const Part& pt) -> cudaError_t {
-        // one CTA per SM (fewer when the partition is small): each stages the BVH once and walks its share of the slots
-        unsigned grid = std::min<unsigned>(t2_grid_cap, (unsigned)((pt.a.n_slots + t2_threads - 1) / t2_threads));
-        if (grid < 1) grid = 1;
-#define RTX_T2_LAUNCH(CNT, THR, ALL)                                                                                              \
-    do {                                                                                                                          \
-        auto k = rtx::wf_trace2_kernel<CNT, THR, ALL>;                                                                            \
-        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t2_smem);                        \
-        if (e != cudaSuccess) return e;                                                                                           \
-        k<<<grid, THR, t2_smem, pt.stream>>>(pt.a.sc, pt.a.pool, pt.a.n_slots, tcfg, d_ray_count, CNT ? c->d_counters : nullptr); \
-    } while (0)
-#define RTX_T2_THREADS(CNT, ALL)                                  \
-    do {                                                          \
-        if (t2_threads == 1024) RTX_T2_LAUNCH(CNT, 1024, ALL);    \
-        else if (t2_threads == 896) RTX_T2_LAUNCH(CNT, 896, ALL); \
-        else if (t2_threads == 640) RTX_T2_LAUNCH(CNT, 640, ALL); \
-        else if (t2_threads == 512) RTX_T2_LAUNCH(CNT, 512, ALL); \
-        else RTX_T2_LAUNCH(CNT, 448, ALL);                        \
-    } while (0)
-        if (counted) { if (t2_all) RTX_T2_THREADS(true, true); else RTX_T2_THREADS(true, false); }
-        else { if (t2_all) RTX_T2_THREADS(false, true); else RTX_T2_THREADS(false, false); }
-#undef RTX_T2_THREADS
-#undef RTX_T2_LAUNCH
-        return cudaSuccess;
-    };
     size_t prof_used = 0;
     // every kProfStride-th iteration of partition 0 is bracketed (events between back-to-back launches cost ~10 %
     // when every launch has them); the accumulated times are scaled back up by the stride
@@ -964,7 +1065,7 @@ static int render_wavefront(rtx_ctx* c, const rtx_scene* s, const rtx_render_par
     for (int k = 0; remaining > 0; ++k) {
         const int par = k & 1;
         for (int q = 0; q < P; ++q) {
-            Part& pt = parts[(size_t)q];
+            WfPart& pt = parts[(size_t)q];
             if (pt.done) continue;
             unsigned int* d_act = c->d_active + 2 * q + par;
             for (int it = 0; it < batch; ++it) {
@@ -975,51 +1076,14 @@ static int render_wavefront(rtx_ctx* c, const rtx_scene* s, const rtx_render_par
                 }
                 prof_now = q == 0 && c->profiling && (iteration++ % kProfStride) == 0;
                 CU(prof_mark());
-                if (adaptive) {  // (rtx_render_adaptive refuses the first shade form and ray ordering)
-                    if (c->perlin_smem && s->n_perlins == 1) rtx::wf_shade2_kernel<false, true, false, true><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, nullptr);
-                    else rtx::wf_shade2_kernel<false, false, false, true><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, nullptr);
-                } else if (c->shade_form >= 2) {
-                    if (counted && !ordered) rtx::wf_shade2_kernel<true><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, c->d_counters);
-                    else if (ordered) {
-                        if (counted) rtx::wf_shade2_kernel<true, false, true><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, c->d_counters);
-                        else if (c->perlin_smem && s->n_perlins == 1) rtx::wf_shade2_kernel<false, true, true><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, nullptr);
-                        else rtx::wf_shade2_kernel<false, false, true><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, nullptr);
-                        rtx::wf_order_kernel<<<(unsigned)((pt.a.n_slots + 255) / 256), 256, 0, pt.stream>>>(pt.a.order, pt.a.n_slots);
-                    }
-                    else if (c->perlin_smem && s->n_perlins == 1) rtx::wf_shade2_kernel<false, true><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, nullptr);
-                    else rtx::wf_shade2_kernel<false><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, nullptr);
-                } else {
-                    if (counted) rtx::wf_shade_kernel<true><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, c->d_counters);
-                    else rtx::wf_shade_kernel<false><<<pt.sgrid, rtx::kShadeBlock, 0, pt.stream>>>(pt.a, acc, active, nullptr);
-                }
+                pl.launch_shade(pt, acc, active);
                 CU(prof_mark());
                 CU(prof_mark());
-                if (ordered) {
-                    if (counted) rtx::wf_trace_ordered_kernel<true><<<pt.grid, rtx::kTraceBlock, 0, pt.stream>>>(pt.a.sc, pt.a.pool, pt.a.order, d_ray_count, c->d_counters);
-                    else rtx::wf_trace_ordered_kernel<false><<<pt.grid, rtx::kTraceBlock, 0, pt.stream>>>(pt.a.sc, pt.a.pool, pt.a.order, d_ray_count, nullptr);
-                } else if (t1c) {
-                    if (counted) rtx::wf_trace1c_kernel<true><<<pt.grid, rtx::kTraceBlock, 0, pt.stream>>>(pt.a.sc, pt.a.pool, pt.a.n_slots, d_ray_count, c->d_counters);
-                    else rtx::wf_trace1c_kernel<false><<<pt.grid, rtx::kTraceBlock, 0, pt.stream>>>(pt.a.sc, pt.a.pool, pt.a.n_slots, d_ray_count, nullptr);
-                } else if (t3_threads != 0) {
-                    CU(launch_trace3(pt));
-                } else if (t2_threads != 0) {
-                    CU(launch_trace2(pt));
-                } else if (counted) {
-                    if (wide)
-                        rtx::wf_trace_kernel<true, true><<<pt.grid, rtx::kTraceBlock, 0, pt.stream>>>(pt.a.sc, pt.a.pool, pt.a.n_slots, d_ray_count, c->d_counters);
-                    else
-                        rtx::wf_trace_kernel<true><<<pt.grid, rtx::kTraceBlock, 0, pt.stream>>>(pt.a.sc, pt.a.pool, pt.a.n_slots, d_ray_count, c->d_counters);
-                } else {
-                    if (wide)
-                        rtx::wf_trace_kernel<false, true><<<pt.grid, rtx::kTraceBlock, 0, pt.stream>>>(pt.a.sc, pt.a.pool, pt.a.n_slots, d_ray_count, nullptr);
-                    else
-                        rtx::wf_trace_kernel<false><<<pt.grid, rtx::kTraceBlock, 0, pt.stream>>>(pt.a.sc, pt.a.pool, pt.a.n_slots, d_ray_count, nullptr);
-                }
+                pl.launch_trace(pt, d_ray_count);
                 CU(prof_mark());
             }
             CU(cudaGetLastError());
-            c->launches += (ordered ? 3ull : 2ull) * (unsigned long long)batch;
-            if (q == 0) c->wf_iterations += (unsigned long long)batch;
+            c->launches += pl.launches() * (unsigned long long)batch;
             // status of this batch -> pinned memory (active is 32-bit: widen on the host side)
             unsigned long long* hs = c->h_status + 4 * q + 2 * par;
             hs[0] = 0;
@@ -1030,7 +1094,7 @@ static int render_wavefront(rtx_ctx* c, const rtx_scene* s, const rtx_render_par
         if (k >= 1) {  // look at the previous batches while these run
             const int prev = par ^ 1;
             for (int q = 0; q < P; ++q) {
-                Part& pt = parts[(size_t)q];
+                WfPart& pt = parts[(size_t)q];
                 if (pt.done) continue;
                 CU(cudaEventSynchronize(c->batch_done[2 * q + prev]));
                 const unsigned long long* hs = c->h_status + 4 * q + 2 * prev;
@@ -1061,13 +1125,36 @@ static int render_wavefront(rtx_ctx* c, const rtx_scene* s, const rtx_render_par
 }
 
 // ---- render -----------------------------------------------------------------
+// The megakernel (RTX_MODE=mega): one persistent render_kernel launch over the frame.
+static int render_mega(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, float* d_accum,
+                       unsigned long long* d_ray_count, bool counted) {
+    rtx::RenderArgs a;
+    const Tiles tiles = set_frame(a, s, p);
+    a.w_node = c->w_node; a.w_leaf = c->w_leaf; a.w_shade = c->w_shade;
+    a.node_burst = c->node_burst;
+    CU(cudaMemsetAsync(c->d_work_counter, 0, sizeof(unsigned int), c->stream));
+    const auto kernel = counted ? rtx::render_kernel<true> : rtx::render_kernel<false>;
+    // persistent grid: as many CTAs as fit, a whole number per SM
+    int per_sm = 0;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, rtx::kRenderBlock, 0));
+    if (per_sm < 1) per_sm = 1;
+    int64_t n_tiles = (int64_t)tiles.x * tiles.y;
+    int64_t grid = (int64_t)c->sm_count * per_sm;
+    const int warps = rtx::kRenderBlock / 32;
+    int64_t needed = (n_tiles + warps - 1) / warps;
+    if (grid > needed) grid = needed;
+    if (grid < 1) grid = 1;
+    kernel<<<(unsigned)grid, rtx::kRenderBlock, 0, c->stream>>>(a, reinterpret_cast<float4*>(d_accum), d_ray_count, c->d_work_counter,
+                                                               counted ? c->d_counters : nullptr);
+    CU(cudaGetLastError());
+    c->launches += 1;
+    return RTX_OK;
+}
+
 static int render_launch(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, float* d_accum,
                          unsigned long long* d_ray_count, bool counted) {
     if (!c || !s || !p || !d_accum) return fail(RTX_ERR_INVALID, "NULL argument");
-    if (p->width <= 0 || p->height <= 0 || p->spp_count < 0 || p->spp_begin < 0 || p->max_depth < 0)
-        return fail(RTX_ERR_INVALID, "bad render parameters");
-    if ((int64_t)p->width * p->height > 0x7fffffff) return fail(RTX_ERR_INVALID, "image too large");
-    if (p->spp_count > (1 << 24)) return fail(RTX_ERR_INVALID, "more than 2^24 samples per pixel in one call (the fp32 sample count of the accumulator)");
+    if (const int rc = check_frame(p, 0, p->spp_count < 0, "bad render parameters", "accumulator"); rc != RTX_OK) return rc;
     if (p->spp_count == 0) return RTX_OK;
     CU(cudaSetDevice(c->device));
     if (p->max_depth == 0) {  // color(.., depth = 0) is black (main.rs:27-29): only the sample counts move
@@ -1078,38 +1165,10 @@ static int render_launch(rtx_ctx* c, const rtx_scene* s, const rtx_render_params
         return RTX_OK;
     }
     if (c->mode == 1) return render_wavefront(c, s, p, d_accum, d_ray_count, counted);
-    rtx::RenderArgs a;
-    a.sc = s->view;
-    a.cam = s->camera;
-    a.width = p->width; a.height = p->height;
-    a.spp_begin = p->spp_begin; a.spp_count = p->spp_count; a.max_depth = p->max_depth;
-    a.k0 = (uint32_t)p->seed; a.k1 = (uint32_t)(p->seed >> 32);
-    a.tiles_x = (p->width + rtx::kTileW - 1) / rtx::kTileW;
-    a.tiles_y = (p->height + rtx::kTileH - 1) / rtx::kTileH;
-    a.inv_per_block_row = 1.0f / (float)(a.tiles_x * rtx::kBlockH);
-    a.w_node = c->w_node; a.w_leaf = c->w_leaf; a.w_shade = c->w_shade;
-    a.node_burst = c->node_burst;
-    CU(cudaMemsetAsync(c->d_work_counter, 0, sizeof(unsigned int), c->stream));
-    // persistent grid: as many CTAs as fit, a whole number per SM
-    int per_sm = 0;
-    if (counted) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rtx::render_kernel<true>, rtx::kRenderBlock, 0));
-    else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rtx::render_kernel<false>, rtx::kRenderBlock, 0));
-    if (per_sm < 1) per_sm = 1;
-    int64_t n_tiles = (int64_t)a.tiles_x * a.tiles_y;
-    int64_t grid = (int64_t)c->sm_count * per_sm;
-    const int warps = rtx::kRenderBlock / 32;
-    int64_t needed = (n_tiles + warps - 1) / warps;
-    if (grid > needed) grid = needed;
-    if (grid < 1) grid = 1;
-    float4* acc = reinterpret_cast<float4*>(d_accum);
-    if (counted)
-        rtx::render_kernel<true><<<(unsigned)grid, rtx::kRenderBlock, 0, c->stream>>>(a, acc, d_ray_count, c->d_work_counter, c->d_counters);
-    else
-        rtx::render_kernel<false><<<(unsigned)grid, rtx::kRenderBlock, 0, c->stream>>>(a, acc, d_ray_count, c->d_work_counter, nullptr);
-    CU(cudaGetLastError());
-    c->launches += 1;
-    return RTX_OK;
+    return render_mega(c, s, p, d_accum, d_ray_count, counted);
 }
+
+extern "C" {
 
 int rtx_render(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, float* d_accum, unsigned long long* d_ray_count) {
     if (c && c->async && s && p && d_accum) {
@@ -1144,14 +1203,7 @@ int rtx_render_counted(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* 
     }
     cudaFree(d_rays);
     if (rc != RTX_OK) return rc;
-    double dn = rays ? (double)rays : 1.0;
-    out->rays = (double)rays;
-    out->box_tests = (double)h.box_tests / dn;
-    out->node_visits = (double)h.node_visits / dn;
-    out->sphere_tests = (double)h.sphere_tests / dn;
-    out->rect_tests = (double)h.rect_tests / dn;
-    out->instance_enters = (double)h.instance_enters / dn;
-    out->medium_tests = (double)h.medium_tests / dn;
+    trace_stats(h, rays, out);
     return RTX_OK;
 }
 
@@ -1159,9 +1211,8 @@ int rtx_render_counted(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* 
 int rtx_render_adaptive(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, const rtx_adaptive_params* ap,
                         float* d_accum, float* d_aux, rtx_adaptive_stats* stats) {
     if (!c || !s || !p || !ap || !d_accum || !d_aux) return fail(RTX_ERR_INVALID, "NULL argument");
-    if (p->width <= 0 || p->height <= 0 || p->max_depth < 0 || p->spp_begin < 0 || (p->spp_begin & 1))
-        return fail(RTX_ERR_INVALID, "bad render parameters (spp_begin must be even)");
-    if ((int64_t)p->width * p->height > 0x7fffffff) return fail(RTX_ERR_INVALID, "image too large");
+    if (const int rc = check_frame(p, 0, (p->spp_begin & 1) != 0, "bad render parameters (spp_begin must be even)", nullptr); rc != RTX_OK)
+        return rc;
     const int max_spp = p->spp_count;
     if (max_spp < 2 || (max_spp & 1) || max_spp > (1 << 24)) return fail(RTX_ERR_INVALID, "spp_count (max_spp) must be even, in [2, 2^24]");
     if (ap->min_spp < 2 || (ap->min_spp & 1) || ap->min_spp > max_spp) return fail(RTX_ERR_INVALID, "min_spp must be even, in [2, max_spp]");
@@ -1172,9 +1223,8 @@ int rtx_render_adaptive(rtx_ctx* c, const rtx_scene* s, const rtx_render_params*
     JOIN(c);
     CU(cudaSetDevice(c->device));
     const int w = p->width, h = p->height;
-    const int tiles_x = (w + rtx::kTileW - 1) / rtx::kTileW, tiles_y = (h + rtx::kTileH - 1) / rtx::kTileH;
-    const int n_tiles = tiles_x * tiles_y;
-    const float inv_per_block_row = 1.0f / (float)(tiles_x * rtx::kBlockH);
+    const Tiles tiles = frame_tiles(w, h);
+    const int n_tiles = tiles.x * tiles.y;
     // scratch: tile errors, flags, their scan, the list, the round's read-back, cub's temporary storage
     size_t scan_bytes = 0;
     CU(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, n_tiles, c->stream));
@@ -1196,10 +1246,10 @@ int rtx_render_adaptive(rtx_ctx* c, const rtx_scene* s, const rtx_render_params*
     auto select_tiles = [&](const float* err) -> int {
         const unsigned grid = (unsigned)((n_tiles + 255) / 256);
         CU(cudaMemsetAsync(d_round, 0, sizeof(rtx::AdaptiveRound), c->stream));
-        rtx::adaptive_flag_kernel<<<grid, 256, 0, c->stream>>>(err, ap->threshold, tiles_x, tiles_y, inv_per_block_row, d_flag);
+        rtx::adaptive_flag_kernel<<<grid, 256, 0, c->stream>>>(err, ap->threshold, tiles.x, tiles.y, tiles.inv_per_block_row, d_flag);
         size_t cb = scan_bytes;
         CU(cub::DeviceScan::ExclusiveSum(block + o_cub, cb, d_flag, d_pos, n_tiles, c->stream));
-        rtx::adaptive_scatter_kernel<<<grid, 256, 0, c->stream>>>(d_flag, d_pos, w, h, tiles_x, tiles_y, inv_per_block_row, d_list, d_round);
+        rtx::adaptive_scatter_kernel<<<grid, 256, 0, c->stream>>>(d_flag, d_pos, w, h, tiles.x, tiles.y, tiles.inv_per_block_row, d_list, d_round);
         c->launches += 4;  // (cub's scan counts as two)
         CU(cudaGetLastError());
         CU(cudaMemcpyAsync(&cur, d_round, sizeof(cur), cudaMemcpyDeviceToHost, c->stream));
@@ -1222,14 +1272,15 @@ int rtx_render_adaptive(rtx_ctx* c, const rtx_scene* s, const rtx_render_params*
             double render_ms = 0.0;
             if (p->max_depth == 0) {  // color(.., depth = 0) is black (main.rs:27-29): only the sample counts move
                 rtx::adaptive_black_kernel<<<(unsigned)((cur.tiles * 32 + 127) / 128), 128, 0, c->stream>>>(
-                    d_list, (int)cur.tiles, w, h, tiles_x, tiles_y, inv_per_block_row, p->spp_begin + n, spp, acc, aux);
+                    d_list, (int)cur.tiles, w, h, tiles.x, tiles.y, tiles.inv_per_block_row, p->spp_begin + n, spp, acc, aux);
                 c->launches += 1;
                 CU(cudaGetLastError());
             } else {
                 rtx_render_params rp = *p;
                 rp.spp_begin = p->spp_begin + n;
                 rp.spp_count = spp;
-                rc = render_wavefront(c, s, &rp, d_accum, nullptr, false, d_list, (int64_t)cur.tiles, d_aux);
+                const AdaptivePass pass{{d_list, aux}, (int64_t)cur.tiles};
+                rc = render_wavefront(c, s, &rp, d_accum, nullptr, false, &pass);
                 if (rc != RTX_OK) return rc;
             }
             if (debug) {
@@ -1247,7 +1298,7 @@ int rtx_render_adaptive(rtx_ctx* c, const rtx_scene* s, const rtx_render_params*
                 break;
             }
             rtx::adaptive_error_kernel<<<(unsigned)(((int64_t)n_tiles * 32 + rtx::kAdaptiveBlock - 1) / rtx::kAdaptiveBlock),
-                                         rtx::kAdaptiveBlock, 0, c->stream>>>(acc, aux, w, h, tiles_x, n_tiles, d_err);
+                                         rtx::kAdaptiveBlock, 0, c->stream>>>(acc, aux, w, h, tiles.x, n_tiles, d_err);
             c->launches += 1;
             CU(cudaGetLastError());
             const unsigned long long pixels = cur.pixels;
@@ -1274,10 +1325,10 @@ int rtx_adaptive_error(rtx_ctx* c, const float* d_accum, const float* d_aux, int
     if ((int64_t)width * height > 0x7fffffff) return fail(RTX_ERR_INVALID, "image too large");
     JOIN(c);
     CU(cudaSetDevice(c->device));
-    const int tiles_x = (width + rtx::kTileW - 1) / rtx::kTileW, tiles_y = (height + rtx::kTileH - 1) / rtx::kTileH;
-    const int64_t n_tiles = (int64_t)tiles_x * tiles_y;
+    const Tiles tiles = frame_tiles(width, height);
+    const int64_t n_tiles = (int64_t)tiles.x * tiles.y;
     rtx::adaptive_error_kernel<<<(unsigned)((n_tiles * 32 + rtx::kAdaptiveBlock - 1) / rtx::kAdaptiveBlock), rtx::kAdaptiveBlock, 0, c->stream>>>(
-        reinterpret_cast<const float4*>(d_accum), reinterpret_cast<const float4*>(d_aux), width, height, tiles_x, (int)n_tiles, d_tile_error);
+        reinterpret_cast<const float4*>(d_accum), reinterpret_cast<const float4*>(d_aux), width, height, tiles.x, (int)n_tiles, d_tile_error);
     c->launches += 1;
     CU(cudaGetLastError());
     return RTX_OK;
@@ -1288,24 +1339,17 @@ int rtx_render_aov(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, f
                    float* d_depth) {
     if (!c || !s || !p) return fail(RTX_ERR_INVALID, "NULL argument");
     if (!d_albedo && !d_normal && !d_depth) return fail(RTX_ERR_INVALID, "no feature buffer given");
-    if (p->width <= 0 || p->height <= 0 || p->spp_count < 0 || p->spp_begin < 0 || p->max_depth < 1)
-        return fail(RTX_ERR_INVALID, "bad render parameters (the feature pass needs max_depth >= 1)");
-    if ((int64_t)p->width * p->height > 0x7fffffff) return fail(RTX_ERR_INVALID, "image too large");
-    if (p->spp_count > (1 << 24)) return fail(RTX_ERR_INVALID, "more than 2^24 samples per pixel in one call (the fp32 sample count of the buffers)");
+    if (const int rc = check_frame(p, 1, p->spp_count < 0, "bad render parameters (the feature pass needs max_depth >= 1)", "buffers"); rc != RTX_OK)
+        return rc;
     JOIN(c);
     if (p->spp_count == 0) return RTX_OK;
     CU(cudaSetDevice(c->device));
     rtx::AovArgs a;
-    a.sc = s->view;
-    a.cam = s->camera;
-    a.width = p->width; a.height = p->height;
-    a.spp_begin = p->spp_begin; a.spp_count = p->spp_count;
-    a.k0 = (uint32_t)p->seed; a.k1 = (uint32_t)(p->seed >> 32);
-    a.tiles_x = (p->width + rtx::kTileW - 1) / rtx::kTileW;
+    const Tiles tiles = set_frame(a, s, p);
     a.albedo = reinterpret_cast<float4*>(d_albedo);
     a.normal = reinterpret_cast<float4*>(d_normal);
     a.depth = reinterpret_cast<float2*>(d_depth);
-    const int64_t n_tiles = (int64_t)a.tiles_x * ((p->height + rtx::kTileH - 1) / rtx::kTileH);
+    const int64_t n_tiles = (int64_t)tiles.x * tiles.y;
     const int64_t grid = (n_tiles * 32 + rtx::kAovBlock - 1) / rtx::kAovBlock;
     rtx::aov_kernel<<<(unsigned)grid, rtx::kAovBlock, 0, c->stream>>>(a);
     c->launches += 1;
