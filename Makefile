@@ -5,7 +5,7 @@ NVFLAGS := $(ARCH) -std=c++17 -O3 -lineinfo -Xcompiler -fPIC,-Wall,-Wextra -Xptx
 SRC := rttnw_b200/csrc
 LIB := rttnw_b200/lib/librttnw_b200.so
 CLI := rttnw_b200/lib/rttnw
-HDRS := include/rttnw_b200.h $(SRC)/device_types.h $(SRC)/flatten.hpp $(SRC)/kernels.cuh $(SRC)/shade2.cuh $(SRC)/order.cuh $(SRC)/trace2.cuh $(SRC)/trace3.cuh $(SRC)/lbvh.cuh $(SRC)/sah_build.cuh $(SRC)/adaptive.cuh $(SRC)/aov.cuh $(SRC)/denoise.cuh $(SRC)/scene_api.hpp
+HDRS := include/rttnw_b200.h $(SRC)/device_types.h $(SRC)/flatten.hpp $(SRC)/kernels.cuh $(SRC)/shade2.cuh $(SRC)/shade2_body.cuh $(SRC)/aov_body.cuh $(SRC)/order.cuh $(SRC)/trace2.cuh $(SRC)/trace3.cuh $(SRC)/lbvh.cuh $(SRC)/sah_build.cuh $(SRC)/adaptive.cuh $(SRC)/aov.cuh $(SRC)/denoise.cuh $(SRC)/scene_api.hpp
 
 all: $(LIB) $(CLI) oracle
 

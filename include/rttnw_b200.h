@@ -414,6 +414,34 @@ int rtx_denoise(rtx_ctx* ctx, const float* d_accum, const float* d_half, const f
 int rtx_reduce_tonemap_peers(rtx_ctx* ctx, float* d_accum, const float* const* d_peer_accums,
                              int32_t n_peers, int32_t width, int32_t height, uint8_t* d_rgba8);
 
+/* Environment lighting: an HDR latitude-longitude map in place of the constant background. The reference's color()
+ * returns Scene.background when a ray leaves the scene (main.rs:26-45, Q8); with an environment it returns
+ * E(d), d the (f64, not normalised) direction of the ray that missed. The estimator is unchanged: the same paths, the
+ * same Philox draws, one contribution per path. Only the value of a miss changes. E(d) is:
+ *   rotation about +y by θ = rotation_y in radians:  x' = cos θ d.x − sin θ d.z,  z' = sin θ d.x + cos θ d.z,  y' = d.y;
+ *   map coordinates, in f64:  u = 0.5 + atan2(x', −z') / 2π,  v = atan2(hypot(x', z'), y') / π;
+ *   texel coordinates:  X = u W − 0.5,  Y = v H − 0.5;  x0 = floor(X), y0 = floor(Y), fx = (float)(X − x0),
+ *   fy = (float)(Y − y0); columns wrap (x0 mod W, (x0 + 1) mod W), rows clamp to [0, H − 1];
+ *   blend, in fp32, per channel, with t(i, j) the texel of column i, row j (row 0 = top, +y):
+ *     a = t(x0, y0) + fx (t(x0 + 1, y0) − t(x0, y0)),  b = t(x0, y0 + 1) + fx (t(x0 + 1, y0 + 1) − t(x0, y0 + 1)),
+ *     E = (a + fy (b − a)) × (float)scale.
+ * The lerp form gives back a constant map's value exactly, so a 1x1 map of float(background) renders bit for bit what
+ * the background does. Seen from inside, the map is not mirrored: looking along −z shows the centre column (u = 0.5),
+ * +x lies to its right (u > 0.5), +y is row 0. With rotation_y = 90 the centre column is seen looking along −x. */
+typedef struct rtx_environment {
+    int32_t width, height; /* texels, >= 1 each, width*height < 2^31 */
+    const float* rgb;      /* host, width*height*3 linear floats, row 0 = top (+y), finite and >= 0 */
+    double rotation_y;     /* degrees, finite */
+    double scale[3];       /* finite, >= 0; multiplies every texel */
+} rtx_environment;         /* 48 bytes */
+/* env == NULL restores desc.background. Copies the texels to the device (16 bytes a texel, counted in rtx_scene_info's
+ * device_bytes); joins any queued asynchronous job of ctx first and waits for the device before it frees the previous
+ * map, so renders queued before the call use the map they were queued with. Bad input is RTX_ERR_INVALID. rtx_render,
+ * rtx_render_adaptive and rtx_render_aov take the map; the fixed-ray calls never look at it. With a map, the megakernel
+ * (RTX_MODE=mega), the first shade form (RTX_SHADE=1), ray ordering (RTX_ORDER=1) and rtx_render_counted give
+ * RTX_ERR_UNSUPPORTED. Host input only; the device must be the scene's. */
+int rtx_scene_set_environment(rtx_ctx* ctx, rtx_scene* scene, const rtx_environment* env);
+
 /* The same combine with the work spread over the ranks: EVERY rank calls this with the accumulators of all n_ranks
  * ranks (its own and the peer-mapped / IPC-opened others, in rank order) and reduces + tonemaps pixels
  * [rank * n / n_ranks, (rank + 1) * n / n_ranks) only, writing them straight into rank 0's RGBA8 buffer
@@ -483,6 +511,13 @@ int rtx_png_write_rgba8(const char* path, int32_t width, int32_t height, const u
  * RTX_ERR_INVALID. `data` is host memory, width*height*channels floats, row 0 = top; the file stores the rows
  * bottom-up as little-endian floats (scale -1.0). */
 int rtx_pfm_write(const char* path, int32_t width, int32_t height, int32_t channels, const float* data);
+/* Readers for environment maps. Both return host memory, rows top-first, to free with rtx_buffer_free.
+ * rtx_pfm_read: "PF" (channels = 3) or "Pf" (channels = 1), either byte order (the sign of the scale).
+ * rtx_hdr_read: Radiance RGBE ("#?RADIANCE" / "#?RGBE"), FORMAT=32-bit_rle_rgbe, flat or new-style run-length
+ * scanlines, 3 channels; only the "-Y H +X W" orientation (RTX_ERR_UNSUPPORTED otherwise). A missing file is
+ * RTX_ERR_IO; a truncated or malformed one RTX_ERR_INVALID. Neither reads past the end of the file. */
+int rtx_pfm_read(const char* path, int32_t* width, int32_t* height, int32_t* channels, float** data);
+int rtx_hdr_read(const char* path, int32_t* width, int32_t* height, float** rgb);
 int rtx_buffer_free(void* p);
 
 #ifdef __cplusplus

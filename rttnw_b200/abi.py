@@ -105,9 +105,15 @@ class DenoiseParams(C.Structure):
                 ("sigma_luminance", C.c_float)]
 
 
+class Environment(C.Structure):
+    _fields_ = [("width", C.c_int32), ("height", C.c_int32), ("rgb", C.POINTER(C.c_float)), ("rotation_y", C.c_double),
+                ("scale", C.c_double * 3)]
+
+
 assert C.sizeof(Node) == 96 and C.sizeof(Material) == 40 and C.sizeof(Texture) == 48
 assert C.sizeof(Ray) == 80 and C.sizeof(Hit) == 88 and C.sizeof(RenderParams) == 32
 assert C.sizeof(AdaptiveParams) == 16 and C.sizeof(AdaptiveStats) == 24 and C.sizeof(DenoiseParams) == 16
+assert C.sizeof(Environment) == 48
 
 # numpy views of the two bulk records (same memory layout as the C structs)
 RAY_DTYPE = [("origin", "<f8", 3), ("direction", "<f8", 3), ("time", "<f8"), ("t_min", "<f8"),
@@ -172,6 +178,10 @@ SIGNATURES = {
                                      C.POINTER(C.POINTER(C.c_uint8))]),
     "rtx_png_write_rgba8": (C.c_int, [C.c_char_p, C.c_int32, C.c_int32, _P]),
     "rtx_pfm_write": (C.c_int, [C.c_char_p, C.c_int32, C.c_int32, C.c_int32, _P]),
+    "rtx_scene_set_environment": (C.c_int, [_P, _P, C.POINTER(Environment)]),
+    "rtx_pfm_read": (C.c_int, [C.c_char_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                               C.POINTER(C.POINTER(C.c_float))]),
+    "rtx_hdr_read": (C.c_int, [C.c_char_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.POINTER(C.c_float))]),
     "rtx_buffer_free": (C.c_int, [_P]),
 }
 

@@ -156,6 +156,9 @@ struct rtx_scene {
     int32_t n_nodes = 0, n_records = 0, n_xforms = 0;
     int32_t world_first_node = 0, world_node_count = 0, world_depth = 0;  // the world BVH's node range (root first) and depth
     int32_t n_perlins = 0;
+    // rtx_scene_set_environment: the map (env.texels == nullptr: none, the constant background) in its own allocation
+    rtx::EnvArgs env{};
+    size_t env_bytes = 0;
 };
 
 // Waits until the context's worker thread has nothing queued or running; returns (once) the failure of an asynchronous
@@ -614,6 +617,7 @@ int rtx_scene_destroy(rtx_scene* s) {
         }
         if (!kept) cudaFree(s->d_arena);
     }
+    if (s->env.texels) cudaFree((void*)s->env.texels);
     delete s;
     return RTX_OK;
 }
@@ -636,7 +640,53 @@ int rtx_scene_info(const rtx_scene* s, int32_t* n_bvh_nodes, int32_t* n_records,
     if (n_bvh_nodes) *n_bvh_nodes = s->n_nodes;
     if (n_records) *n_records = s->n_records;
     if (n_xform_ops) *n_xform_ops = s->n_xforms;
-    if (device_bytes) *device_bytes = (int64_t)s->arena_bytes;
+    if (device_bytes) *device_bytes = (int64_t)(s->arena_bytes + s->env_bytes);
+    return RTX_OK;
+}
+
+int rtx_scene_set_environment(rtx_ctx* c, rtx_scene* s, const rtx_environment* env) {
+    if (!c || !s) return fail(RTX_ERR_INVALID, "NULL argument");
+    if (c->device != s->device) return fail(RTX_ERR_INVALID, "the context and the scene are on different devices");
+    std::vector<float4> host;
+    rtx::EnvArgs e{};
+    if (env) {
+        if (env->width < 1 || env->height < 1 || (int64_t)env->width * env->height > 0x7fffffff)
+            return fail(RTX_ERR_INVALID, "environment size must be >= 1 x 1 and below 2^31 texels");
+        if (!env->rgb) return fail(RTX_ERR_INVALID, "environment texels are NULL");
+        if (!std::isfinite(env->rotation_y)) return fail(RTX_ERR_INVALID, "environment rotation must be finite");
+        for (double k : env->scale)
+            if (!(k >= 0.0) || !std::isfinite(k)) return fail(RTX_ERR_INVALID, "environment scale must be finite and >= 0");
+        const size_t n = (size_t)env->width * env->height;
+        host.resize(n + 1);
+        host[0] = make_float4((float)env->scale[0], (float)env->scale[1], (float)env->scale[2], 0.f);
+        for (size_t i = 0; i < n; ++i) {
+            const float* t = env->rgb + 3 * i;
+            for (int k = 0; k < 3; ++k)
+                if (!(t[k] >= 0.f) || !std::isfinite(t[k])) return fail(RTX_ERR_INVALID, "environment texels must be finite and >= 0");
+            host[i + 1] = make_float4(t[0], t[1], t[2], 0.f);
+        }
+        const double th = env->rotation_y * (3.14159265358979323846 / 180.0);
+        e.width = env->width;
+        e.height = env->height;
+        e.cos_t = std::cos(th);
+        e.sin_t = std::sin(th);
+    }
+    JOIN(c);
+    CU(cudaSetDevice(s->device));
+    void* d = nullptr;
+    if (env) {
+        CU(cudaMalloc(&d, host.size() * sizeof(float4)));
+        // on the ctx stream and waited for, like the scene upload: once the call returns the texels are on the device,
+        // whichever stream renders next
+        cudaError_t err = cudaMemcpyAsync(d, host.data(), host.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream);
+        if (err == cudaSuccess) err = cudaStreamSynchronize(c->stream);
+        if (err != cudaSuccess) { cudaFree(d); return cuda_fail(err, "cudaMemcpyAsync (environment)"); }
+        e.texels = (const float4*)d;
+    }
+    // renders queued on any stream may still read the old map
+    if (s->env.texels) { CU(cudaDeviceSynchronize()); CU(cudaFree((void*)s->env.texels)); }
+    s->env = e;
+    s->env_bytes = host.size() * sizeof(float4);
     return RTX_OK;
 }
 
@@ -924,12 +974,16 @@ static int stage_cap(const rtx_ctx* c, const rtx_scene* s, size_t fixed) {
 
 static WfPlan wf_plan(const rtx_ctx* c, const rtx_scene* s, bool counted, bool adaptive) {
     WfPlan pl;
+    const bool env = s->env.texels != nullptr;  // (env_refusal has ruled out counting, ray ordering and the first form)
     pl.counters = counted ? c->d_counters : nullptr;
     const bool wide = c->wf_wide != 0 && s->view.wide_root >= 0;
     pl.order_pass = c->order_form != 0 && c->shade_form >= 2 && c->trace_form == 1 && !wide;
     // the shade kernel stages the Perlin table in shared memory when the scene has exactly one (not when counting)
     const bool perlin = c->perlin_smem && s->n_perlins == 1;
-    if (adaptive)  // (rtx_render_adaptive refuses the first shade form and ray ordering)
+    if (env)
+        pl.shade = adaptive ? (perlin ? rtx::wf_shade2_env_kernel<true, true> : rtx::wf_shade2_env_kernel<false, true>)
+                            : (perlin ? rtx::wf_shade2_env_kernel<true, false> : rtx::wf_shade2_env_kernel<false, false>);
+    else if (adaptive)  // (rtx_render_adaptive refuses the first shade form and ray ordering)
         pl.shade = perlin ? rtx::wf_shade2_kernel<false, true, false, true> : rtx::wf_shade2_kernel<false, false, false, true>;
     else if (c->shade_form < 2)
         pl.shade = counted ? rtx::wf_shade_kernel<true> : rtx::wf_shade_kernel<false>;
@@ -1004,6 +1058,7 @@ static int render_wavefront(rtx_ctx* c, const rtx_scene* s, const rtx_render_par
     a.total_items = total;
     a.next_item = c->d_next_item;
     a.adaptive = adaptive ? adaptive->args : rtx::AdaptiveArgs{};  // (ray ordering, the other user of this space, fills it per partition below)
+    a.env = s->env;
     CU(cudaMemsetAsync(a.pool.bounce, 0xFF, (size_t)slots * 4, c->stream));  // every slot empty (-1)
     CU(cudaMemsetAsync(c->d_next_item, 0, sizeof(unsigned long long), c->stream));
     float4* acc = reinterpret_cast<float4*>(d_accum);
@@ -1151,9 +1206,19 @@ static int render_mega(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* 
     return RTX_OK;
 }
 
+// The render forms that have no environment-map variant refuse a scene that has a map.
+static int env_refusal(const rtx_ctx* c, const rtx_scene* s, bool counted) {
+    if (!s->env.texels) return RTX_OK;
+    if (counted) return fail(RTX_ERR_UNSUPPORTED, "rtx_render_counted does not render scenes with an environment map");
+    if (c->mode != 1 || c->shade_form < 2 || c->order_form != 0)
+        return fail(RTX_ERR_UNSUPPORTED, "an environment map needs the wavefront driver with the default shade form and no ray ordering");
+    return RTX_OK;
+}
+
 static int render_launch(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, float* d_accum,
                          unsigned long long* d_ray_count, bool counted) {
     if (!c || !s || !p || !d_accum) return fail(RTX_ERR_INVALID, "NULL argument");
+    if (const int rc = env_refusal(c, s, counted); rc != RTX_OK) return rc;
     if (const int rc = check_frame(p, 0, p->spp_count < 0, "bad render parameters", "accumulator"); rc != RTX_OK) return rc;
     if (p->spp_count == 0) return RTX_OK;
     CU(cudaSetDevice(c->device));
@@ -1172,6 +1237,7 @@ extern "C" {
 
 int rtx_render(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, float* d_accum, unsigned long long* d_ray_count) {
     if (c && c->async && s && p && d_accum) {
+        if (const int rc = env_refusal(c, s, false); rc != RTX_OK) return rc;  // refused now, not from the next join
         const rtx_render_params params = *p;  // the caller's struct need not outlive the call
         {
             std::lock_guard<std::mutex> lock(c->mu);
@@ -1351,7 +1417,8 @@ int rtx_render_aov(rtx_ctx* c, const rtx_scene* s, const rtx_render_params* p, f
     a.depth = reinterpret_cast<float2*>(d_depth);
     const int64_t n_tiles = (int64_t)tiles.x * tiles.y;
     const int64_t grid = (n_tiles * 32 + rtx::kAovBlock - 1) / rtx::kAovBlock;
-    rtx::aov_kernel<<<(unsigned)grid, rtx::kAovBlock, 0, c->stream>>>(a);
+    if (s->env.texels) rtx::aov_env_kernel<<<(unsigned)grid, rtx::kAovBlock, 0, c->stream>>>(a, s->env);
+    else rtx::aov_kernel<<<(unsigned)grid, rtx::kAovBlock, 0, c->stream>>>(a);
     c->launches += 1;
     CU(cudaGetLastError());
     return RTX_OK;
@@ -1751,6 +1818,34 @@ int rtx_pfm_write(const char* path, int32_t width, int32_t height, int32_t chann
     if (width <= 0 || height <= 0 || (channels != 1 && channels != 3)) return fail(RTX_ERR_INVALID, "bad PFM size or channel count (1 or 3)");
     std::string err;
     if (!rttnw::pfm_write(path, width, height, channels, data, err)) return fail(RTX_ERR_IO, err);
+    return RTX_OK;
+}
+// A reader's result as a malloc'd buffer the caller frees with rtx_buffer_free.
+static int hand_over(const std::vector<float>& px, float** out) {
+    float* buf = (float*)std::malloc(px.size() * sizeof(float));
+    if (!buf) return fail(RTX_ERR_NOMEM, "out of host memory");
+    std::memcpy(buf, px.data(), px.size() * sizeof(float));
+    *out = buf;
+    return RTX_OK;
+}
+int rtx_pfm_read(const char* path, int32_t* width, int32_t* height, int32_t* channels, float** data) {
+    if (!path || !width || !height || !channels || !data) return fail(RTX_ERR_INVALID, "NULL argument");
+    std::vector<float> px;
+    std::string err;
+    int w = 0, h = 0, ch = 0;
+    if (const int rc = rttnw::pfm_read(path, w, h, ch, px, err); rc != RTX_OK) return fail(rc, err);
+    if (const int rc = hand_over(px, data); rc != RTX_OK) return rc;
+    *width = w; *height = h; *channels = ch;
+    return RTX_OK;
+}
+int rtx_hdr_read(const char* path, int32_t* width, int32_t* height, float** rgb) {
+    if (!path || !width || !height || !rgb) return fail(RTX_ERR_INVALID, "NULL argument");
+    std::vector<float> px;
+    std::string err;
+    int w = 0, h = 0;
+    if (const int rc = rttnw::hdr_read(path, w, h, px, err); rc != RTX_OK) return fail(rc, err);
+    if (const int rc = hand_over(px, rgb); rc != RTX_OK) return rc;
+    *width = w; *height = h;
     return RTX_OK;
 }
 int rtx_buffer_free(void* p) {

@@ -4,6 +4,12 @@
 //   --spp N  --width W  --height H  --seed S  --scene-seed S  --gpus N  --out PATH  --chunk N
 //   --checkpoint PATH [--checkpoint-every K]  --resume PATH  --stop-after-chunks N
 //   --adaptive THRESHOLD [--min-spp N] [--step N]  --aov PREFIX [--aov-spp N]  --denoise
+//   --env FILE [--env-rotate DEG] [--env-scale K]
+// --env FILE (rtx_scene_set_environment): the scene is lit by an HDR latitude-longitude map (a .pfm, "PF" or "Pf", or a
+// Radiance .hdr, told apart by the first bytes) in place of its constant background, rotated by DEG degrees about +y
+// (default 0) and multiplied by K (default 1). Every path below takes it: uniform, multi-process and threaded rendering,
+// checkpoints, --adaptive, --aov and --denoise. A --resume must be given the same --env as the render it continues
+// (the checkpoint does not record the map and this is not checked).
 // --adaptive (one GPU; rtx_render_adaptive): every 8x4 tile stops sampling once its noise estimate is below THRESHOLD,
 // with --spp as the most samples a pixel gets; --min-spp defaults to spp / 64 (at least 2, even), --step to --min-spp.
 // It prints the samples spent and the tiles that converged. Not with --gpus > 1, --checkpoint or --resume: several GPUs
@@ -48,6 +54,7 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstdint>
@@ -208,6 +215,9 @@ int main(int argc, char** argv) {
     std::string aov_prefix;  // --aov PREFIX: the feature pass and the PFMs
     long long aov_spp = -1;
     bool denoise = false;
+    std::string env_path;  // --env FILE
+    const char* env_rotate = nullptr;
+    const char* env_scale = nullptr;
     int worker_rank = -1, shm_fd = -1;  // --worker R --shm-fd FD --device-list L: a worker process of a multi-GPU render (internal)
     std::string device_list = std::getenv("CUDA_VISIBLE_DEVICES") ? std::getenv("CUDA_VISIBLE_DEVICES") : "";
     for (int i = 1; i < argc; ++i) {
@@ -238,6 +248,9 @@ int main(int argc, char** argv) {
         else if (a == "--step") step_spp = std::atoi(next("--step"));
         else if (a == "--aov") aov_prefix = next("--aov");
         else if (a == "--denoise") denoise = true;
+        else if (a == "--env") env_path = next("--env");
+        else if (a == "--env-rotate") env_rotate = next("--env-rotate");
+        else if (a == "--env-scale") env_scale = next("--env-scale");
         else if (a == "--aov-spp") {
             const char* v = next("--aov-spp");
             char* end = nullptr;
@@ -266,6 +279,38 @@ int main(int argc, char** argv) {
         return 1;
     }
     if (aov_spp > 0 && aov_prefix.empty() && !denoise) { std::fprintf(stderr, "--aov-spp needs --aov PREFIX or --denoise\n"); return 1; }
+    // --env: the map is read and the numbers checked here, before CUDA starts
+    rtx_environment env{};
+    std::vector<float> env_rgb;
+    if (env_path.empty() && (env_rotate || env_scale)) { std::fprintf(stderr, "--env-rotate and --env-scale need --env FILE\n"); return 1; }
+    if (!env_path.empty()) {
+        auto number = [](const char* v, double& out) {
+            char* end = nullptr;
+            out = std::strtod(v, &end);
+            return end != v && *end == 0 && std::isfinite(out);
+        };
+        double rot = 0.0, k = 1.0;
+        if (env_rotate && !number(env_rotate, rot)) { std::fprintf(stderr, "--env-rotate needs a finite number of degrees\n"); return 1; }
+        if (env_scale && (!number(env_scale, k) || k < 0.0)) { std::fprintf(stderr, "--env-scale needs a finite number >= 0\n"); return 1; }
+        char magic[2] = {0, 0};
+        if (FILE* f = std::fopen(env_path.c_str(), "rb")) {
+            if (std::fread(magic, 1, 2, f) != 2) magic[0] = 0;
+            std::fclose(f);
+        }
+        int32_t w = 0, h = 0, ch = 3;
+        float* data = nullptr;
+        const bool pfm = magic[0] == 'P' && (magic[1] == 'F' || magic[1] == 'f'), hdr = magic[0] == '#' && magic[1] == '?';
+        if (!pfm && !hdr) { std::fprintf(stderr, "--env %s: not a readable PFM or Radiance HDR file\n", env_path.c_str()); return 1; }
+        const int rc = pfm ? rtx_pfm_read(env_path.c_str(), &w, &h, &ch, &data) : rtx_hdr_read(env_path.c_str(), &w, &h, &data);
+        if (rc != RTX_OK) { std::fprintf(stderr, "--env %s: %s\n", env_path.c_str(), rtx_last_error()); return 1; }
+        env_rgb.resize((size_t)w * h * 3);
+        for (size_t i = 0; i < (size_t)w * h; ++i)
+            for (int c = 0; c < 3; ++c) env_rgb[3 * i + c] = data[ch == 3 ? 3 * i + c : i];  // a grey map on every channel
+        rtx_buffer_free(data);
+        env = rtx_environment{w, h, env_rgb.data(), rot, {k, k, k}};
+    }
+    // every rank's scene gets the map right after it is created
+    auto set_env = [&](rtx_ctx* c, rtx_scene* sc) { return env_path.empty() ? RTX_OK : rtx_scene_set_environment(c, sc, &env); };
     if (worker_rank < 0) std::printf("Scene number: %d\n", scene);
     auto t0 = std::chrono::steady_clock::now();
     rtx_scene_defaults def;
@@ -293,6 +338,7 @@ int main(int argc, char** argv) {
         const size_t bytes = (size_t)width * height * 4 * sizeof(float);
         RTX(rtx_ctx_create(0, nullptr, &ctx));
         RTX(rtx_scene_create(ctx, desc, &sc));
+        RTX(set_env(ctx, sc));
         RTX(rtx_malloc(ctx, bytes, (void**)&accum));
         RTX(rtx_malloc(ctx, bytes, (void**)&aux));
         rtx_render_params p{width, height, 0, spp, def.max_depth, 0, seed};
@@ -331,6 +377,7 @@ int main(int argc, char** argv) {
         if (!chk(rtx_ctx_create(one_device_per_process ? 0 : r, nullptr, &k.ctx))) return;
         if (r == 0) lap("context created");
         if (!chk(rtx_scene_create(k.ctx, desc, &k.scene))) return;
+        if (!chk(set_env(k.ctx, k.scene))) return;
         if (r == 0) lap("scene uploaded");
         size_t bytes = (size_t)width * height * 4 * sizeof(float);
         if (!chk(rtx_malloc(k.ctx, bytes, (void**)&k.accum))) return;
@@ -409,6 +456,7 @@ int main(int argc, char** argv) {
             if (!chk(rtx_ctx_create(0, nullptr, &k.ctx))) return;
             if (me == 0) lap("context created");
             if (!chk(rtx_scene_create(k.ctx, desc, &k.scene))) return;
+            if (!chk(set_env(k.ctx, k.scene))) return;
             if (!chk(rtx_malloc(k.ctx, frame_bytes, (void**)&k.accum))) return;
             if (!chk(rtx_memset_zero(k.ctx, k.accum, frame_bytes))) return;
         };

@@ -1230,6 +1230,34 @@ struct AdaptiveArgs {
     float4* aux;                // receives the samples with an odd global index a second time
 };
 
+// The environment map of a scene (rtx_scene_set_environment): one float4 per texel, row 0 = top (+y), behind a header.
+struct EnvArgs {
+    const float4* texels;  // texels[0] = {scale r, g, b, 0}; texel (column i, row j) is texels[1 + j * width + i]
+    int32_t width, height;
+    double cos_t, sin_t;  // of rotation_y
+};
+
+// E(d) of include/rttnw_b200.h: the miss value of a ray with direction d. f64 map coordinates, fp32 bilinear blend.
+// The integer coordinates are clamped before use, so no direction reads outside the map.
+__device__ __forceinline__ float3 env_lookup(const EnvArgs& e, const d3& d) {
+    const double xr = e.cos_t * d.x - e.sin_t * d.z, zr = e.sin_t * d.x + e.cos_t * d.z;
+    const double u = 0.5 + atan2(xr, -zr) / (2.0 * 3.14159265358979323846);
+    const double v = atan2(hypot(xr, zr), d.y) / 3.14159265358979323846;
+    const double X = u * e.width - 0.5, Y = v * e.height - 0.5;
+    const double xf = floor(X), yf = floor(Y);
+    const float fx = (float)(X - xf), fy = (float)(Y - yf);
+    const int ix = (int)fmax(fmin(xf, (double)(e.width - 1)), -1.0), iy = (int)fmax(fmin(yf, (double)(e.height - 1)), -1.0);
+    const int i0 = ix < 0 ? e.width - 1 : ix, i1 = ix + 1 >= e.width ? 0 : ix + 1;  // columns wrap
+    const int j0 = iy < 0 ? 0 : iy, j1 = iy + 1 >= e.height ? e.height - 1 : iy + 1;  // rows clamp
+    const float4* row0 = e.texels + 1 + (size_t)j0 * e.width;
+    const float4* row1 = e.texels + 1 + (size_t)j1 * e.width;
+    const float4 t00 = __ldg(row0 + i0), t10 = __ldg(row0 + i1), t01 = __ldg(row1 + i0), t11 = __ldg(row1 + i1);
+    const float4 s = __ldg(e.texels);
+    const float ar = t00.x + fx * (t10.x - t00.x), ag = t00.y + fx * (t10.y - t00.y), ab = t00.z + fx * (t10.z - t00.z);
+    const float br = t01.x + fx * (t11.x - t01.x), bg = t01.y + fx * (t11.y - t01.y), bb = t01.z + fx * (t11.z - t01.z);
+    return make_float3((ar + fy * (br - ar)) * s.x, (ag + fy * (bg - ag)) * s.y, (ab + fy * (bb - ab)) * s.z);
+}
+
 struct WfArgs {
     SceneView sc;
     CameraView cam;
@@ -1241,14 +1269,19 @@ struct WfArgs {
     int32_t n_slots;
     unsigned long long total_items;   // tiles * 32 * spp_count
     unsigned long long* next_item;    // global dispenser of path samples
-    // Last, what one specialisation of the shade kernel needs, never both: ray ordering for the trace pass (order.cuh,
-    // kOrder) or adaptive sampling (adaptive.cuh, kAdaptive). Sharing the space keeps the size of WfArgs, so the kernel
-    // parameters behind it, and the code of every other shade kernel, stay where they were.
+    // Last, what one specialisation of the shade kernel needs: ray ordering for the trace pass (order.cuh, kOrder), or
+    // adaptive sampling (adaptive.cuh, kAdaptive) and the environment map (kEnv), which the kernels that order rays
+    // never take. Sharing the space keeps the size of WfArgs, so the kernel parameters behind it, and the code of every
+    // other shade kernel, stay where they were.
     union {
         OrderArgs order;
-        AdaptiveArgs adaptive;
+        struct {
+            AdaptiveArgs adaptive;
+            EnvArgs env;
+        };
     };
 };
+static_assert(sizeof(OrderArgs) >= sizeof(AdaptiveArgs) + sizeof(EnvArgs), "the union must keep the size of OrderArgs");
 
 constexpr int kWfBlock = 128;   // trace kernel CTA; the pool size is a multiple of it
 #ifndef WF_SHADE_BLOCK

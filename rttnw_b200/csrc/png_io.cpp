@@ -2,9 +2,12 @@
 // Reader: what ImageTexture::new needs (src/math/texture.rs:69-75 decodes via the `image`
 // crate and converts to RGBA8): 8/16-bit gray, gray+alpha, RGB, RGBA and 8-bit palette,
 // non-interlaced. Writer: image::save_buffer(.., ColorType::Rgba8) of src/main.rs:231.
-// Also the PFM writer of the linear beauty and the feature buffers (rtx_pfm_write).
+// Also the PFM writer of the linear beauty and the feature buffers (rtx_pfm_write), and the PFM and Radiance .hdr
+// readers of environment maps (rtx_pfm_read, rtx_hdr_read).
 #include <zlib.h>
 
+#include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -193,6 +196,146 @@ bool pfm_write(const char* path, int width, int height, int channels, const floa
     bool ok = std::fclose(f) == 0 && wr == out.size();
     if (!ok) { err = "short write"; return false; }
     return true;
+}
+
+// ---- readers of environment maps ----
+static bool slurp(const char* path, std::vector<uint8_t>& file, std::string& err) {
+    FILE* f = std::fopen(path, "rb");
+    if (!f) { err = std::string("cannot open ") + path; return false; }
+    uint8_t buf[1 << 16];
+    size_t n;
+    while ((n = std::fread(buf, 1, sizeof(buf), f)) > 0) file.insert(file.end(), buf, buf + n);
+    std::fclose(f);
+    return true;
+}
+static bool is_space(uint8_t c) { return c == ' ' || c == '\t' || c == '\n' || c == '\r'; }
+// The next whitespace-delimited token of at most 63 characters starting at or after pos; false at the end of the file.
+static bool next_token(const std::vector<uint8_t>& f, size_t& pos, std::string& tok) {
+    while (pos < f.size() && is_space(f[pos])) ++pos;
+    tok.clear();
+    while (pos < f.size() && !is_space(f[pos]) && tok.size() < 64) tok.push_back((char)f[pos++]);
+    return !tok.empty() && tok.size() < 64;
+}
+static bool parse_dim(const std::string& t, int& v) {
+    char* end = nullptr;
+    const long long x = std::strtoll(t.c_str(), &end, 10);
+    if (*end != 0 || t.empty() || x < 1 || x > 0x7fffffff) return false;
+    v = (int)x;
+    return true;
+}
+
+// "PF" (RGB) or "Pf" (grey), "width height", the scale (negative: little-endian samples, positive: big-endian), one
+// whitespace character, then the rows bottom-up.
+int pfm_read(const char* path, int& width, int& height, int& channels, std::vector<float>& data, std::string& err) {
+    std::vector<uint8_t> f;
+    if (!slurp(path, f, err)) return RTX_ERR_IO;
+    size_t pos = 0;
+    std::string magic, ws, hs, ss;
+    if (!next_token(f, pos, magic) || (magic != "PF" && magic != "Pf")) { err = "not a PFM file"; return RTX_ERR_INVALID; }
+    if (!next_token(f, pos, ws) || !next_token(f, pos, hs) || !parse_dim(ws, width) || !parse_dim(hs, height)) {
+        err = "bad PFM size";
+        return RTX_ERR_INVALID;
+    }
+    char* end = nullptr;
+    const double scale = next_token(f, pos, ss) ? std::strtod(ss.c_str(), &end) : 0.0;
+    if (!end || *end != 0 || !(scale != 0.0) || !std::isfinite(scale)) { err = "bad PFM scale"; return RTX_ERR_INVALID; }
+    if (pos >= f.size() || !is_space(f[pos])) { err = "truncated PFM header"; return RTX_ERR_INVALID; }
+    ++pos;
+    channels = magic == "PF" ? 3 : 1;
+    const uint64_t row = (uint64_t)width * (uint64_t)channels, count = row * (uint64_t)height;
+    if (count > (f.size() - pos) / 4) { err = "truncated PFM data"; return RTX_ERR_INVALID; }
+    data.resize((size_t)count);
+    const bool little = scale < 0.0;
+    for (int y = 0; y < height; ++y) {
+        const uint8_t* src = f.data() + pos + 4 * row * (uint64_t)(height - 1 - y);  // the file stores the bottom row first
+        float* dst = data.data() + row * (uint64_t)y;
+        for (uint64_t i = 0; i < row; ++i, src += 4) {
+            const uint32_t u = little ? (uint32_t)src[0] | ((uint32_t)src[1] << 8) | ((uint32_t)src[2] << 16) | ((uint32_t)src[3] << 24)
+                                      : be32(src);
+            std::memcpy(dst + i, &u, 4);
+        }
+    }
+    return RTX_OK;
+}
+
+// Radiance RGBE: "#?" header lines up to an empty line (FORMAT must be 32-bit_rle_rgbe when given), the resolution line
+// "-Y H +X W" (rows top-first, columns left to right; the other seven orientations are refused), then H scanlines, each
+// flat (W x RGBE) or new-style run-length encoded (2, 2, W >> 8, W & 255, then the four components one after the other,
+// each as runs: a count byte c > 128 repeats the next byte c - 128 times, 1 <= c <= 128 copies c bytes). A texel is
+// m * 2^(e - 136) per channel (m the mantissa byte), black when e = 0: exact in fp32.
+int hdr_read(const char* path, int& width, int& height, std::vector<float>& rgb, std::string& err) {
+    std::vector<uint8_t> f;
+    if (!slurp(path, f, err)) return RTX_ERR_IO;
+    if (f.size() < 2 || f[0] != '#' || f[1] != '?') { err = "not a Radiance HDR file"; return RTX_ERR_INVALID; }
+    size_t pos = 0;
+    auto line = [&](std::string& out) -> bool {  // the next line without its newline; false when the file ends first
+        out.clear();
+        while (pos < f.size() && f[pos] != '\n') {
+            if (out.size() < 256) out.push_back((char)f[pos]);
+            ++pos;
+        }
+        if (pos >= f.size()) return false;
+        ++pos;
+        return true;
+    };
+    std::string l;
+    for (;;) {
+        if (!line(l)) { err = "truncated HDR header"; return RTX_ERR_INVALID; }
+        if (l.empty()) break;
+        if (l.compare(0, 7, "FORMAT=") == 0 && l != "FORMAT=32-bit_rle_rgbe") { err = "unsupported HDR format " + l; return RTX_ERR_UNSUPPORTED; }
+    }
+    if (!line(l)) { err = "truncated HDR resolution line"; return RTX_ERR_INVALID; }
+    char a0 = 0, a1 = 0, b0 = 0, b1 = 0;
+    long long n0 = 0, n1 = 0;
+    int used = 0;
+    if (std::sscanf(l.c_str(), " %c%c %lld %c%c %lld %n", &a0, &a1, &n0, &b0, &b1, &n1, &used) != 6 || (size_t)used != l.size() ||
+        (a0 != '-' && a0 != '+') || (b0 != '-' && b0 != '+') || !((a1 == 'Y' && b1 == 'X') || (a1 == 'X' && b1 == 'Y')) ||
+        n0 < 1 || n1 < 1 || n0 > 0x7fffffff || n1 > 0x7fffffff) {
+        err = "bad HDR resolution line";
+        return RTX_ERR_INVALID;
+    }
+    if (a0 != '-' || a1 != 'Y' || b0 != '+' || b1 != 'X') { err = "unsupported HDR orientation " + l + " (only -Y H +X W)"; return RTX_ERR_UNSUPPORTED; }
+    height = (int)n0;
+    width = (int)n1;
+    // the fewest bytes a scanline can take (flat, or run-length: 4 + per component 2 bytes per run of at most 127)
+    const uint64_t min_scan = std::min<uint64_t>(4 * (uint64_t)width, 4 + 8 * (((uint64_t)width + 126) / 127));
+    if (min_scan * (uint64_t)height > f.size() - pos) { err = "truncated HDR data"; return RTX_ERR_INVALID; }
+    const size_t W = (size_t)width;
+    std::vector<uint8_t> scan(4 * W);
+    rgb.resize(3 * W * (size_t)height);
+    for (int y = 0; y < height; ++y) {
+        const bool rle = W >= 8 && W < 32768 && pos + 4 <= f.size() && f[pos] == 2 && f[pos + 1] == 2 && ((size_t)f[pos + 2] << 8 | f[pos + 3]) == W;
+        if (rle) {
+            pos += 4;
+            for (int c = 0; c < 4; ++c) {
+                for (size_t x = 0; x < W;) {
+                    if (pos >= f.size()) { err = "truncated HDR scanline"; return RTX_ERR_INVALID; }
+                    size_t n = f[pos++];
+                    if (n > 128) {
+                        n -= 128;
+                        if (pos >= f.size() || n > W - x) { err = "bad HDR run"; return RTX_ERR_INVALID; }
+                        for (size_t k = 0; k < n; ++k) scan[4 * (x + k) + (size_t)c] = f[pos];
+                        ++pos;
+                    } else {
+                        if (n == 0 || n > W - x || n > f.size() - pos) { err = "bad HDR run"; return RTX_ERR_INVALID; }
+                        for (size_t k = 0; k < n; ++k) scan[4 * (x + k) + (size_t)c] = f[pos + k];
+                        pos += n;
+                    }
+                    x += n;
+                }
+            }
+        } else {
+            if (4 * W > f.size() - pos) { err = "truncated HDR scanline"; return RTX_ERR_INVALID; }
+            std::memcpy(scan.data(), f.data() + pos, 4 * W);
+            pos += 4 * W;
+        }
+        float* out = rgb.data() + 3 * W * (size_t)y;
+        for (size_t x = 0; x < W; ++x) {
+            const uint8_t* p = &scan[4 * x];
+            for (int c = 0; c < 3; ++c) out[3 * x + (size_t)c] = p[3] == 0 ? 0.f : std::ldexp((float)p[c], (int)p[3] - 136);
+        }
+    }
+    return RTX_OK;
 }
 
 }  // namespace rttnw

@@ -125,5 +125,9 @@ bool png_read_rgba8(const char* path, int& width, int& height, std::vector<uint8
 bool png_write_rgba8(const char* path, int width, int height, const uint8_t* rgba, std::string& err);
 // PFM, 1 or 3 little-endian float channels (rtx_pfm_write)
 bool pfm_write(const char* path, int width, int height, int channels, const float* data, std::string& err);
+// PFM ("PF" / "Pf", either byte order) and Radiance .hdr readers for environment maps (rtx_pfm_read, rtx_hdr_read):
+// rows top-first; they return an rtx_status and never read past the end of the file
+int pfm_read(const char* path, int& width, int& height, int& channels, std::vector<float>& data, std::string& err);
+int hdr_read(const char* path, int& width, int& height, std::vector<float>& rgb, std::string& err);
 
 }  // namespace rttnw

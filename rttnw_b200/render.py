@@ -50,6 +50,42 @@ def pfm_write(path: str, image: np.ndarray) -> None:
     abi.check(abi.load().rtx_pfm_write(path.encode(), image.shape[1], image.shape[0], channels, image.ctypes.data))
 
 
+def pfm_read(path: str) -> np.ndarray:
+    """A PFM file ("PF" or "Pf", either byte order) as float32 (H, W, 3) or (H, W), row 0 = top (rtx_pfm_read)."""
+    lib = abi.load()
+    w, h, c, buf = C.c_int32(), C.c_int32(), C.c_int32(), C.POINTER(C.c_float)()
+    abi.check(lib.rtx_pfm_read(path.encode(), C.byref(w), C.byref(h), C.byref(c), C.byref(buf)))
+    try:
+        shape = (h.value, w.value, 3) if c.value == 3 else (h.value, w.value)
+        return np.ctypeslib.as_array(buf, shape=shape).copy()
+    finally:
+        lib.rtx_buffer_free(buf)
+
+
+def hdr_read(path: str) -> np.ndarray:
+    """A Radiance RGBE file ("-Y H +X W") as float32 (H, W, 3), row 0 = top (rtx_hdr_read)."""
+    lib = abi.load()
+    w, h, buf = C.c_int32(), C.c_int32(), C.POINTER(C.c_float)()
+    abi.check(lib.rtx_hdr_read(path.encode(), C.byref(w), C.byref(h), C.byref(buf)))
+    try:
+        return np.ctypeslib.as_array(buf, shape=(h.value, w.value, 3)).copy()
+    finally:
+        lib.rtx_buffer_free(buf)
+
+
+def env_read(path: str) -> np.ndarray:
+    """An environment map as float32 (H, W, 3), row 0 = top (+y): a PFM (a grey "Pf" map is repeated over the three
+    channels) or a Radiance .hdr, told apart by the file's first bytes."""
+    with open(path, "rb") as f:
+        magic = f.read(2)
+    if magic in (b"PF", b"Pf"):
+        m = pfm_read(path)
+        return np.ascontiguousarray(np.repeat(m[..., None], 3, axis=2)) if m.ndim == 2 else m
+    if magic == b"#?":
+        return hdr_read(path)
+    raise ValueError(f"{path}: not a PFM or Radiance HDR file")
+
+
 def scene_defaults(number: int) -> dict:
     """Resolution / spp / depth of the scene table, src/main.rs:66-183,255."""
     d = abi.SceneDefaults()
@@ -176,6 +212,22 @@ class DeviceScene:
         d = desc.desc if hasattr(desc, "desc") else desc
         self.h = C.c_void_p()
         abi.check(self.lib.rtx_scene_create(ctx.h, C.byref(d), C.byref(self.h)))
+
+    def set_environment(self, rgb: Optional[np.ndarray] = None, rotation_y: float = 0.0, scale=(1.0, 1.0, 1.0)) -> None:
+        """Lights the scene with an HDR latitude-longitude map (rtx_scene_set_environment; the lookup is written out in
+        include/rttnw_b200.h): rgb (H, W, 3) linear float32, row 0 = top (+y), rotated by rotation_y degrees about +y,
+        times scale (one number or three). A ray that leaves the scene then returns the map's value in its direction
+        instead of the constant background; rgb=None restores the background. Waits for the renders queued before it."""
+        if rgb is None:
+            abi.check(self.lib.rtx_scene_set_environment(self.ctx.h, self.h, None))
+            return
+        rgb = np.ascontiguousarray(rgb, dtype=np.float32)
+        if rgb.ndim != 3 or rgb.shape[2] != 3:
+            raise ValueError(f"set_environment takes an (H, W, 3) array, got {rgb.shape}")
+        k = (float(scale),) * 3 if np.isscalar(scale) else tuple(float(x) for x in scale)
+        env = abi.Environment(rgb.shape[1], rgb.shape[0], rgb.ctypes.data_as(C.POINTER(C.c_float)), float(rotation_y),
+                              (C.c_double * 3)(*k))
+        abi.check(self.lib.rtx_scene_set_environment(self.ctx.h, self.h, C.byref(env)))
 
     def info(self) -> dict:
         a, b, c, n = C.c_int32(), C.c_int32(), C.c_int32(), C.c_int64()
@@ -314,7 +366,7 @@ def render(scene_number: int, width: Optional[int] = None, height: Optional[int]
            samples: Optional[int] = None, seed: int = 1, device: int = 0, out_path: Optional[str] = None,
            scene_seed: Optional[int] = None, noise_threshold: Optional[float] = None,
            min_samples: Optional[int] = None, aov_prefix: Optional[str] = None, aov_samples: int = 16,
-           denoise: bool = False) -> np.ndarray:
+           denoise: bool = False, env=None, env_rotation: float = 0.0, env_scale=1.0) -> np.ndarray:
     """`render(width, aspect, samples, scene)` of src/main.rs:58 on one GPU; returns RGBA8 (H, W, 4)
     and, like the reference, writes it as a PNG when `out_path` is given ("image.png" there).
     With `noise_threshold`, adaptive sampling (DeviceScene.render_adaptive): `samples` is the most a pixel gets,
@@ -324,13 +376,18 @@ def render(scene_number: int, width: Optional[int] = None, height: Optional[int]
     With `denoise`, the returned RGBA (and the PNG) is the tonemap of Context.denoise over the frame, the feature pass
     of samples [0, aov_samples) and a value-blind half of the samples: the adaptive render's odd samples, or a copy of
     the accumulator between the renders of [0, samples / 2) and [samples / 2, samples). With `aov_prefix` as well,
-    the denoised frame is also written as PREFIX.denoised.pfm."""
+    the denoised frame is also written as PREFIX.denoised.pfm.
+    With `env` (a .pfm / .hdr path or an (H, W, 3) float32 array), the scene is lit by that environment map, rotated by
+    `env_rotation` degrees about +y and scaled by `env_scale` (DeviceScene.set_environment), in place of its constant
+    background."""
     d = scene_defaults(scene_number)
     width, height = width or d["width"], height or d["height"]
     samples = samples or d["samples"]
     ctx = Context(device)
     desc = BuiltinDesc(scene_number, scene_seed)
     scene = DeviceScene(ctx, desc)
+    if env is not None:
+        scene.set_environment(env_read(env) if isinstance(env, (str, os.PathLike)) else env, env_rotation, env_scale)
     accum = scene.new_accum(width, height)
     half = None
     if noise_threshold is None:

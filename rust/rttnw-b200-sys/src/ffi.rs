@@ -183,6 +183,16 @@ impl Default for rtx_denoise_params {
         rtx_denoise_params { iterations: 5, sigma_normal: 0.25, sigma_albedo: 0.1, sigma_luminance: 8.0 }
     }
 }
+/// An HDR latitude-longitude environment map (`rtx_scene_set_environment`; the lookup is written out in the header).
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct rtx_environment {
+    pub width: i32,
+    pub height: i32,
+    pub rgb: *const f32,
+    pub rotation_y: f64,
+    pub scale: [f64; 3],
+}
 /// The scene table of src/main.rs:66-183 and the defaults of :255.
 #[repr(C)]
 #[derive(Clone, Copy)]
@@ -249,5 +259,8 @@ extern "C" {
     pub fn rtx_png_read_rgba8(path: *const c_char, width: *mut i32, height: *mut i32, rgba_out: *mut *mut u8) -> c_int;
     pub fn rtx_png_write_rgba8(path: *const c_char, width: i32, height: i32, rgba: *const u8) -> c_int;
     pub fn rtx_pfm_write(path: *const c_char, width: i32, height: i32, channels: i32, data: *const f32) -> c_int;
+    pub fn rtx_scene_set_environment(ctx: *mut rtx_ctx, scene: *mut rtx_scene, env: *const rtx_environment) -> c_int;
+    pub fn rtx_pfm_read(path: *const c_char, width: *mut i32, height: *mut i32, channels: *mut i32, data: *mut *mut f32) -> c_int;
+    pub fn rtx_hdr_read(path: *const c_char, width: *mut i32, height: *mut i32, rgb: *mut *mut f32) -> c_int;
     pub fn rtx_buffer_free(p: *mut c_void) -> c_int;
 }

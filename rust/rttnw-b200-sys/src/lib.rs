@@ -155,35 +155,78 @@ impl Gpu {
 
     /// The same for a ready-made description (e.g. `rtx_builtin_scene`).
     pub fn render_desc(&self, desc: *const ffi::rtx_scene_desc, width: u32, height: u32, samples: usize, seed: u64) -> Result<Vec<u8>, RtxError> {
+        self.scene(desc)?.render(width, height, samples, seed)
+    }
+
+    /// The scene uploaded to this device, to light with an environment map (`Scene::set_environment`) before rendering.
+    pub fn scene(&self, desc: *const ffi::rtx_scene_desc) -> Result<Scene<'_>, RtxError> {
+        let mut scene = ptr::null_mut();
+        check(unsafe { ffi::rtx_scene_create(self.ctx, desc, &mut scene) })?;
+        Ok(Scene { gpu: self, scene })
+    }
+}
+
+/// A scene resident on one device (`rtx_scene`).
+pub struct Scene<'a> {
+    gpu: &'a Gpu,
+    scene: *mut ffi::rtx_scene,
+}
+
+impl Scene<'_> {
+    /// Lights the scene with an HDR latitude-longitude map in place of its constant background: `rgb` holds
+    /// width * height linear RGB texels, row 0 = top (+y), rotated by `rotation_y` degrees about +y and multiplied by
+    /// `scale`. `None` restores the background. The texels are copied.
+    pub fn set_environment(&mut self, env: Option<(&[f32], u32, u32, f64, [f64; 3])>) -> Result<(), RtxError> {
+        match env {
+            None => check(unsafe { ffi::rtx_scene_set_environment(self.gpu.ctx, self.scene, ptr::null()) }),
+            Some((rgb, width, height, rotation_y, scale)) => {
+                if rgb.len() != width as usize * height as usize * 3 {
+                    return Err(RtxError { status: -1, message: "environment: rgb must hold width * height * 3 floats".into() });
+                }
+                let e = ffi::rtx_environment { width: width as i32, height: height as i32, rgb: rgb.as_ptr(), rotation_y, scale };
+                check(unsafe { ffi::rtx_scene_set_environment(self.gpu.ctx, self.scene, &e) })
+            }
+        }
+    }
+
+    /// `samples` paths per pixel, sqrt gamma, RGBA8, top row first (`Gpu::render_desc`).
+    pub fn render(&self, width: u32, height: u32, samples: usize, seed: u64) -> Result<Vec<u8>, RtxError> {
+        let ctx = self.gpu.ctx;
+        let scene = self.scene;
         let bytes = width as usize * height as usize * 16;
         let mut pixels = vec![0u8; width as usize * height as usize * 4];
         unsafe {
-            let mut scene = ptr::null_mut();
-            check(ffi::rtx_scene_create(self.ctx, desc, &mut scene))?;
             let mut accum: *mut c_void = ptr::null_mut();
             let result = (|| {
-                check(ffi::rtx_malloc(self.ctx, bytes, &mut accum))?;
-                check(ffi::rtx_memset_zero(self.ctx, accum, bytes))?;
+                check(ffi::rtx_malloc(ctx, bytes, &mut accum))?;
+                check(ffi::rtx_memset_zero(ctx, accum, bytes))?;
                 // rtx_render takes at most 2^24 samples per pixel per call: a frame is rendered in chunks of sample indices
                 let mut begin = 0usize;
                 while begin < samples {
                     let count = (samples - begin).min(1 << 20);
                     let params = ffi::rtx_render_params { width: width as i32, height: height as i32, spp_begin: begin as i32,
                                                           spp_count: count as i32, max_depth: 50, _pad: 0, seed };
-                    check(ffi::rtx_render(self.ctx, scene, &params, accum as *mut f32, ptr::null_mut()))?;
+                    check(ffi::rtx_render(ctx, scene, &params, accum as *mut f32, ptr::null_mut()))?;
                     begin += count;
                 }
-                check(ffi::rtx_tonemap_rgba8(self.ctx, accum as *const f32, width as i32, height as i32, pixels.as_mut_ptr(), 0))
+                check(ffi::rtx_tonemap_rgba8(ctx, accum as *const f32, width as i32, height as i32, pixels.as_mut_ptr(), 0))
             })();
             if !accum.is_null() {
-                ffi::rtx_free(self.ctx, accum);
+                ffi::rtx_free(ctx, accum);
             }
-            ffi::rtx_scene_destroy(scene);
             result?;
         }
         Ok(pixels)
     }
+}
 
+impl Drop for Scene<'_> {
+    fn drop(&mut self) {
+        unsafe { ffi::rtx_scene_destroy(self.scene) };
+    }
+}
+
+impl Gpu {
     /// `render_desc` with adaptive sampling (`rtx_render_adaptive`): every 8x4 tile stops once its noise estimate is
     /// below `adaptive.threshold`, after at least `adaptive.min_spp` and at most `max_spp` samples per pixel.
     pub fn render_adaptive_desc(&self, desc: *const ffi::rtx_scene_desc, width: u32, height: u32, max_spp: usize,
